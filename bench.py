@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """Headline benchmark: sampled branch-site histories / second (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes the statistics row the last timed sweep returned (dwell times, then transition counts, float64)
+to DIR/rows.npy.  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 
 Workload (config.workload): BASELINE.json configs[3] — sumstatMCMC_bigtree on a 10 000-tip Yule tree, 4-state
 hidden-rate model make2sQ(.1,.1,.2,.2,10), 1 000 000 sites site-sharded over 8 GPUs = 125 000 sites per GPU, weak
@@ -246,18 +249,16 @@ def run_reference(a, rank, world):
     kind = "reference" if bridge.ref_lib() is not None else "port_faithful"
     for _ in range(min(a.warmup, 1)):   # a tiny run so that page-in / fork costs stay out of the measurement
         cpu_leg(kind, tree, Q, pid, 1, order, sites_per_core=1)
-    steps = max(1, min(a.steps, int(os.environ.get("PM_BENCH_CPU_STEPS", 6))))
-    cb, wall = cpu_leg(kind, tree, Q, pid, steps, order)
+    cb, wall = cpu_leg(kind, tree, Q, pid, a.steps, order)
     cfg = config(a.gpus, SITES_PER_GPU)
     cfg["precision"] = "f64"
     cfg["rng"] = "R Mersenne-Twister (sequential)"
-    line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": steps,
-            "warmup": min(a.warmup, 1), "ms_per_step": 1e3 * wall / steps, "higher_is_better": True, "scaling": "weak",
+    line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
+            "warmup": min(a.warmup, 1), "ms_per_step": 1e3 * wall / a.steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": cfg,
             "cpu_baseline": cb, "gpu_launches": 0,
             "e2e": {"value": cb["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-            "note": "each step is one sweep over a bounded site sample of the workload (%s); steps = sweeps actually run "
-                    "(requested %d)" % (cb["sample"], a.steps)}
+            "note": "each step is one sweep over a bounded site sample of the workload (%s)" % cb["sample"]}
     print(json.dumps(line))
 
 
@@ -326,6 +327,9 @@ def run_ours(a, rank, local_rank, world):
     expect = S * world * tree.edge_length.sum()
     if not np.allclose(tot, expect, rtol=1e-3):
         raise SystemExit("bench sanity check failed: dwell %r vs %r" % (tot[:3], expect))
+    if a.dump_outputs and rank == 0:   # the rows are already summed over ranks
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "rows.npy"), np.ascontiguousarray(rows[-1:], dtype=np.float64))
 
     # roofline of the pruning pass (K1, SURVEY.md 8(d)).  In the step it is the first pass of the fused launch
     # k_prune_nodes_clade (prune the block's 32 sites, then draw their node states): the launch is timed with CUDA events
@@ -459,12 +463,20 @@ def run_ours(a, rank, local_rank, world):
 def main():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=10)
+    p.add_argument("--steps", type=int, default=None,
+                   help="timed sweeps (default 10; for --impl reference PM_BENCH_CPU_STEPS, else 6)")
     p.add_argument("--warmup", type=int, default=3)
     p.add_argument("--impl", default="ours")
     p.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     p.add_argument("--no-rate", action="store_true", help="skip the rate_sampler block")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the last timed sweep's statistics row to DIR/rows.npy")
     a = p.parse_args()
+    if a.steps is None:
+        a.steps = int(os.environ.get("PM_BENCH_CPU_STEPS", 6)) if a.impl == "reference" else 10
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        sys.stderr.write("bench.py: --dump-outputs ignored: the reference arm runs on the CPU and returns no GPU outputs\n")
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))

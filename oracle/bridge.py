@@ -129,19 +129,15 @@ def shim_path():
 
 
 def shim_lib():
-    """oracle/_ref/libphylomap_shim.so: the reference's unmodified RcppExports.cpp + shim/phylomap_b200_shim.cpp (the
-    drop-in replacement of src/phylomap.cpp on the product's C ABI) + the same driver, against the stand-in headers
-    (oracle/Makefile, target `shim`).  The `.Call` symbols of the package, served by libphylomap_b200.so.  This is the one
-    place where test infrastructure loads the PRODUCT through the reference's boundary; nothing of the oracle restatement
-    is involved.  Returns None when it is not built."""
+    """oracle/_ref/libphylomap_shim.so: the package's `.Call` glue (oracle/shim_glue.cpp) + shim/phylomap_b200_shim.cpp
+    (the drop-in replacement of src/phylomap.cpp on the product's C ABI) + the same driver, against the stand-in headers
+    (oracle/Makefile, target `shim`; make relinks it when a source or libphylomap_b200.so is newer).  The `.Call`
+    symbols of the package, served by libphylomap_b200.so.  This is the one place where test infrastructure loads the
+    PRODUCT through the reference's boundary; nothing of the oracle restatement is involved."""
     global _SHIM
     if _SHIM is None:
-        if os.path.exists("/root/reference/src/RcppExports.cpp"):
-            subprocess.check_call(["make", "-C", _HERE, "-s", "shim"])
-        so = shim_path()
-        if not os.path.exists(so):
-            return None
-        L = C.CDLL(so)
+        subprocess.check_call(["make", "-C", _HERE, "-s", "shim"])
+        L = C.CDLL(shim_path())
         L.ref_run.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_char_p, C.c_int]
         L.ref_ncols.argtypes = [C.c_int, C.c_int]
         L.ref_rng_probe.argtypes = [C.c_uint32, C.c_int, C.c_int, C.c_double, C.c_double, C.c_void_p]
@@ -153,10 +149,7 @@ def shim_lib():
 def shim_run(variant, trees, Q, pid, Omega, N, prior=None, seed=1, B=None, eig=None):
     """The same call as ref_run, answered by the product through the shim (any number of sites: states become an
     ntips x nsites matrix).  Precision / mode / device come from the PHYLOMAP_B200_* environment like in an R session."""
-    L = shim_lib()
-    if L is None:
-        raise OracleError("oracle/_ref/libphylomap_shim.so is not built")
-    return _lib_run(L, variant, trees, Q, pid, Omega, N, prior, seed, B, eig)
+    return _lib_run(shim_lib(), variant, trees, Q, pid, Omega, N, prior, seed, B, eig)
 
 
 def shim_seed(seed):

@@ -7,8 +7,8 @@
 // Build inside the R package (src/Makevars, see INTEGRATION.md):  replace src/phylomap.cpp by this file and add
 //   PKG_CPPFLAGS += -I<repo>/include      PKG_LIBS += -L<repo>/phylomap_b200 -lphylomap_b200 -Wl,-rpath,<repo>/phylomap_b200
 // It uses plain Rcpp only (no Armadillo).  In this repository it is compiled against the stand-in headers of
-// oracle/standin/ together with the reference's own, unmodified RcppExports.cpp (oracle/Makefile, target `shim`) and
-// driven through the `.Call` symbols by tests/test_shim.py.
+// oracle/standin/ together with oracle/shim_glue.cpp, the package's `.Call` glue as Rcpp generates it into
+// src/RcppExports.cpp (oracle/Makefile, target `shim`), and driven through the `.Call` symbols by tests/test_shim.py.
 //
 // The site axis (new): x$states may be a matrix with one COLUMN per character (ntips x nsites); its column-major storage
 // is already the [site][tip] order pm_tree.states wants, so it is passed through untouched.  A plain vector is the

@@ -1,15 +1,18 @@
-"""The drop-in shim (shim/phylomap_b200_shim.cpp) driven through the reference's own `.Call` symbols.
+"""The drop-in shim (shim/phylomap_b200_shim.cpp) driven through the package's `.Call` symbols.
 
-oracle/_ref/libphylomap_shim.so = the reference's unmodified src/RcppExports.cpp + the shim (which replaces
-src/phylomap.cpp) compiled against the stand-in Rcpp headers and linked to libphylomap_b200.so.  The driver builds the R
-objects an R session would pass (tree list with maps / mapnames / edge / states, Q, pid, B, nen, nodelist, root, N, prior;
-lists of trees and nen / nodelist MATRICES for mt / ksmt, R/sumstatMCMCmt.R:27-33) and calls phylomap_<fn>.  The result
-must equal the library called directly with the seed the shim derives from R's stream: that pins the flattening
-(CSR maps, column-major edge, the ntips x nsites states matrix, one nen / nodelist row per tree) and the in-place
-rewrite of Q and B.
+oracle/_ref/libphylomap_shim.so = the package's `.Call` glue (oracle/shim_glue.cpp, written as Rcpp generates
+src/RcppExports.cpp) + the shim (which replaces src/phylomap.cpp) compiled against the stand-in Rcpp headers and linked
+to libphylomap_b200.so.  The driver builds the R objects an R session would pass (tree list with maps / mapnames / edge /
+states, Q, pid, B, nen, nodelist, root, N, prior; lists of trees and nen / nodelist MATRICES for mt / ksmt,
+R/sumstatMCMCmt.R:27-33) and calls phylomap_<fn>.  The result must equal the library called directly with the seed the
+shim derives from R's stream: that pins the flattening (CSR maps, column-major edge, the ntips x nsites states matrix, one
+nen / nodelist row per tree) and the in-place rewrite of Q and B.  The glue is bound to the shim's signatures by the link;
+tests/golden/shim/call_signatures.json binds those to the package's.
 """
 import ctypes
+import json
 import os
+import re
 
 import numpy as np
 import pytest
@@ -24,15 +27,22 @@ SYMBOLS = ["phylomap_SPARSEmaketreelistMCMC", "phylomap_maketreelistMCMC", "phyl
            "phylomap_maketreelistMCMCksDICt"]
 
 
-def _shim(oracle):
-    L = oracle.shim_lib()
-    if L is None:
-        pytest.skip("oracle/_ref/libphylomap_shim.so not built here")
-    return L
+def test_shim_signatures_are_the_packages():
+    """The shim defines the ten functions with the parameter types the package's generated glue passes."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    with open(os.path.join(root, "tests", "golden", "shim", "call_signatures.json")) as f:
+        want = {k: v for k, v in json.load(f).items() if not k.startswith("_")}
+    with open(os.path.join(root, "shim", "phylomap_b200_shim.cpp")) as f:
+        src = f.read()
+    assert len(want) == 10
+    for fn, types in want.items():
+        defs = re.findall(r"NumericMatrix %s\(([^)]*)\)\s*\{" % fn, src)
+        assert len(defs) == 1, fn
+        assert [" ".join(p.split()[:-1]) for p in defs[0].split(",")] == types, fn
 
 
 def test_shim_exports_the_ten_call_symbols(oracle):
-    _shim(oracle)
+    oracle.shim_lib()
     L = ctypes.CDLL(oracle.shim_path())
     for s in SYMBOLS:
         assert hasattr(L, s), s
@@ -40,7 +50,7 @@ def test_shim_exports_the_ten_call_symbols(oracle):
 
 def test_shim_tree_order_is_pm_tree_order(oracle):
     """phylomap_tree_order (the O(E) replacement of R/sumstatMCMC.R:1-18) through the shim: host code, no device."""
-    L = _shim(oracle)
+    L = oracle.shim_lib()
     z = cases.tree2(T=40, S=1, seed=3)
     E = z.E
     edge = np.asfortranarray(z.edge, dtype=np.int32)
@@ -69,7 +79,6 @@ def _trees_multi(base, k, seed):
 @pytest.mark.parametrize("name", ["PLAIN", "SPARSE", "BIGTREE", "BF", "KS", "MT", "KSMT", "DIC2S", "DICKS"])
 @pytest.mark.parametrize("S", [1, 5])
 def test_shim_call_equals_direct_call(oracle, det_env, name, S):
-    _shim(oracle)
     Q4, p4 = cases.q4(), np.full(4, 0.25)
     hidden = name in ("KS", "KSMT", "DICKS")
     two = name in ("BF", "MT", "DIC2S")
@@ -95,7 +104,6 @@ def test_shim_call_equals_direct_call(oracle, det_env, name, S):
 
 @pytest.mark.gpu
 def test_shim_direct_sampler_and_errors(oracle, monkeypatch):
-    _shim(oracle)
     monkeypatch.setenv("PHYLOMAP_B200_PRECISION", "f32")
     monkeypatch.delenv("PHYLOMAP_B200_MODE", raising=False)
     Q, pid = cases.jc(4, 0.1), np.full(4, 0.25)
