@@ -293,7 +293,7 @@ struct TreeDev {
   DevBuf cl_entries, cl_warp_off, cl_top_entries, cl_top_off, cd_top, cd_top_off, cd_entries, cd_warp_off, cd_tips;
   int n_cd_top_levels = 0, n_cd_tips = 0;  // clade schedule of the production pruning kernel
   int n_cl_top_levels = 0;
-  DevBuf up_entries8, up_entries, up_off, down_entries, down_off, e_parent, e_child, e_len, maps_off, maps_len, cap_off;
+  DevBuf up_entries, up_off, down_entries, down_off, e_parent, e_child, e_len, maps_off, maps_len, cap_off;
   DevBuf tipcode, node_state, meta, PL, rec_len[2], rec_st[2], dw_partial, hard_ballot, wk_off, wk_g, wk_hint, wk_item, rec_cursor, shape;
   long long wk_total = 0, dw_rows = 0;
   int hard_blocks = 0;
@@ -351,7 +351,6 @@ struct ChainT : pm_chain {
   size_t smem_prune = 0, smem_nodes = 0, smem_paths = 0;
   int rows_cap = 0;
   bool debug_sync = false; int debug_kernel = 0;
-  int k1_variant = 42;  // production pruning kernel variant (pm_launch_impl.cuh; PHYLOMAP_B200_K1_UNROLL overrides, for tuning)
   struct Timed { cudaEvent_t a, b; int k; };
   std::vector<Timed> timed;
   // CUDA-graph replay of one sweep (fixed-Q samplers on small problems: a sweep of a 100-tip tree is seven launches of a
@@ -451,7 +450,7 @@ struct ChainT : pm_chain {
         end_timed();
       } else {
         begin_timed(0);
-        pm::Sweep<Real, NSc, EX>::prune(P, gx, prune_smem(t), stream, k1_variant);
+        pm::Sweep<Real, NSc, EX>::prune(P, gx, prune_smem(t), stream);
         end_timed();
         begin_timed(1);
         pm::Sweep<Real, NSc, EX>::nodes(P, gx, smem_nodes, stream, iter);
@@ -540,7 +539,7 @@ struct ChainT : pm_chain {
       if (only_site >= 0) pm::Sweep<Real, NSc, EX>::prune_nodes(t.P, 1, smem_nodes, stream, 0u, only_site / 32, 1, nullptr, 0, nullptr);
       else pm::Sweep<Real, NSc, EX>::prune_nodes(t.P, (int)nb, smem_nodes, stream, 0u, 0, 1, t.slots_per_sm ? t.slot_busy.template as<int>() : nullptr,
                                                  t.slots_per_sm, nullptr);
-    } else pm::Sweep<Real, NSc, EX>::prune(t.P, (int)nb, prune_smem(t), stream, k1_variant);
+    } else pm::Sweep<Real, NSc, EX>::prune(t.P, (int)nb, prune_smem(t), stream);
     launches++;
   }
 
@@ -764,7 +763,6 @@ struct ChainT : pm_chain {
       // launch geometry of the path kernel: a thread owns one site x one chunk of consecutive branches
       const long long gx = (S + 127) / 128;
       long long ny = (148LL * 16 * 6 + gx - 1) / gx;
-      if (const char* v = getenv("PHYLOMAP_B200_PATH_CHUNKS")) ny = std::max(1, atoi(v));  // (experiments: wave quantisation of the streaming path kernel)
       ny = std::max(1LL, std::min<long long>(ny, (E + 15) / 16));
       ny = std::min<long long>(ny, 65535);
       ny = std::max<long long>(ny, (E + 2047) / 2048);  // the easy path kernel stages a chunk's topology in shared memory
@@ -900,19 +898,13 @@ struct ChainT : pm_chain {
         }
       }
       upload(t->up_entries, t->sch.up_entries, stream);
-      {
-        std::vector<int> e8((size_t)8 * (T - 1), 0);
-        for (int i = 0; i < T - 1; i++) for (int j = 0; j < 5; j++) e8[(size_t)8 * i + j] = t->sch.up_entries[(size_t)5 * i + j];
-        upload(t->up_entries8, e8, stream);
-      }
       upload(t->up_off, t->sch.up_off, stream);
       if (!exact && (NS == 2 || NS == 4)) {
         // clades of ~1/64 of the tree: ~8 per warp to balance, and only ~100 nodes left above them.  Small trees (where a
         // sweep is a matter of latency, not throughput): ~1/8 of the tree, so that almost every node is walked inside a
         // warp's prefetched sequence and only a few levels with block barriers are left above.  (A function of the tree
         // alone: the node draws are keyed by schedule position, and a site must not depend on how many others run.)
-        int clade_max = (T - 1 < 512) ? std::max(8, (T - 1) / 8) : std::max(8, std::min(512, (T - 1) / 64));
-        if (const char* v = getenv("PHYLOMAP_B200_CLADE")) clade_max = std::max(1, atoi(v));
+        const int clade_max = (T - 1 < 512) ? std::max(8, (T - 1) / 8) : std::max(8, std::min(512, (T - 1) / 64));
         pm::host::CladeSchedule cs;
         pm::host::build_clade_schedule(t->sch, 8, clade_max, cs);
         // phase-1 entries as byte offsets (PM_CLADE_ENTRY_INTS ints each): the kernel only adds them to per-lane bases
@@ -1104,7 +1096,6 @@ struct ChainT : pm_chain {
       if (opt.host_tab) replay.reset(new pm::host::ReplaySource(opt.host_tab, opt.host_tab_n));
     }
     mt.reseed((uint32_t)opt.seed);
-    if (const char* v = getenv("PHYLOMAP_B200_K1_UNROLL")) k1_variant = atoi(v);
     if (const char* v = getenv("PHYLOMAP_B200_DEBUG_SYNC")) debug_sync = v[0] == '1';
 
     mark("pinned buffers, replay table");
@@ -1124,12 +1115,10 @@ struct ChainT : pm_chain {
       P.hard_ballot = t.hard_ballot.template as<uint32_t>(); P.W = (int)((t.S + 31) / 32);
       P.wk_off = t.wk_off.template as<long long>(); P.wk_g = t.wk_g.template as<int>(); P.wk_total = t.wk_total;
       P.wk_hint = t.wk_hint.template as<int>(); P.wk_item = t.wk_item.template as<unsigned long long>();
-      P.tune = getenv("PHYLOMAP_B200_TUNE") ? atoi(getenv("PHYLOMAP_B200_TUNE")) : 0;
       P.rec_cursor = t.rec_cursor.template as<int>(); P.chunk = t.chunk; P.easy_blocks = t.nblocks;
       P.shape = t.shape.template as<uint16_t>();
       P.model = model.as<Real>(); P.ppow = model.as<Real>() + model_stride(); P.jcap = jcap;
       P.up_entries = t.up_entries.template as<int>(); P.up_off = t.up_off.template as<int>();
-      P.up_entries8 = t.up_entries8.template as<int>();
       P.n_up_levels = (int)t.sch.up_off.size() - 1;
       P.cl_entries = t.cl_entries.template as<int>(); P.cl_warp_off = t.cl_warp_off.template as<int>();
       P.cl_top_entries = t.cl_top_entries.template as<int>();

@@ -34,7 +34,9 @@ struct ChainParams {
   const Real* ppow;   // [jcap][n*n] P_j = Bs * P_{j-1}
   int jcap;
   const int* up_entries; const int* up_off; int n_up_levels;        // 5 ints per internal node: parent, a, ea, b, eb
-  const int* up_entries8;  // the same entries padded to 8 ints (two 16-byte loads)
+  // (rec_cursor sits here so that every field below keeps its offset modulo 16: the kernels' parameter loads are
+  // scheduled by it, and with the fields shifted by 8 bytes k_loglik<float, 2> takes 35 registers instead of 32)
+  int* rec_cursor;  // [n_chunks][rec_groups] records appended so far to the slice of (chunk, site group) in this sweep
   // clade schedule of k_prune_clade (pm_tree.hpp): 8 ints per node, per-warp sequences then the top levels
   const int* cl_entries; const int* cl_warp_off; const int* cl_top_entries; const int* cl_top_off; int n_cl_top_levels;
   // ... and of k_nodes_clade: top part by depth (4 ints per node: v, parent, edge, -), then per-warp pre-order sequences (16 ints)
@@ -68,8 +70,6 @@ struct ChainParams {
   // ... flattened (k_build_items): item i = branch (bits 32-63) | first ballot word (5-31) | words - 1 (0-4), so that a warp
   // finds its next item with ONE load, issued an item ahead, instead of a chain of four dependent ones
   const unsigned long long* wk_item;
-  int tune;            // PHYLOMAP_B200_TUNE (experiments)
-  int* rec_cursor;  // [n_chunks][rec_groups] records appended so far to the slice of (chunk, site group) in this sweep
   int chunk;        // branches per record chunk
   long long easy_blocks;  // blocks of k_paths_easy: k_paths_hard's dwell partials follow theirs in dw_partial
   // production: meta[e][s] = m | q << 16, q = 16-bit position (pos_dec) of the jump point of a path with one jump point
@@ -198,12 +198,17 @@ __device__ __forceinline__ void pow_times(const ChainParams<Real>& P, const Real
 }
 
 // ------------------------------------------------------------------------------------------------
-// K1, production arithmetic, software-pipelined.  Same tiling as k_prune.  A plain load-then-compute loop spends
-// about as long issuing the arithmetic of a round as it waits for the round's loads, one after the other, so neither
-// the issue slots nor HBM are busy more than ~45 % of the time (ncu, profiles/).  Here the loads of the NEXT round of the level are issued before the
-// arithmetic of the current one (two register buffers, ping-pong), and the arithmetic is shorter: a tip child
-// contributes a COLUMN of P_k, read as one vector from a transposed copy of the table, instead of a mat-vec with a
-// one-hot vector; schedule entries are two vector loads; the normalisation uses the hardware reciprocal.
+// K1, production arithmetic (2 or 4 states), clade order.  Same tiling as k_prune.  A walk level by level would read
+// every partial back from HBM a whole level after writing it (40 % of the 410 KB of traffic per site).  Here every warp
+// walks complete subtrees ("clades", pm_tree.hpp) alone, in post-order with the larger child first:
+//   * a parent follows its last child immediately -> that child's partial is taken from registers;
+//   * its other internal child was finished a few nodes earlier by the same lane -> an L2 hit (same thread, same
+//     address: program order makes the store visible to the load);
+//   * jump counts, tip codes and the schedule never depend on the kernel's own output, so they are fetched DEPTH nodes
+//     ahead with cp.async into a per-warp shared-memory ring;
+//   * no block-wide barrier until the clades are done; the few hundred nodes above them go level by level.
+// A tip child contributes a COLUMN of P_k, read as one vector from a transposed copy of the table, instead of a mat-vec
+// with a one-hot vector; the normalisation uses the hardware reciprocal.
 // ------------------------------------------------------------------------------------------------
 template <typename Real> __device__ __forceinline__ Real fast_rcp(Real x) { return (Real)1 / x; }
 template <> __device__ __forceinline__ float fast_rcp<float>(float x) {  // one MUFU: the result only rescales a partial
@@ -211,126 +216,12 @@ template <> __device__ __forceinline__ float fast_rcp<float>(float x) {  // one 
 }
 
 template <typename Real, int NS>
-struct PruneNode {  // one node of a round: what was loaded for it
+struct PruneNode {  // one node above the clades: what was loaded for it
   int pn; uint32_t ma, mb;
   int ca, cb;        // tip codes (or -1 for an internal child)
   Real va[NS], vb[NS];
 };
 
-template <typename Real, int NS, int U, int MINB>
-__global__ void __launch_bounds__(256, MINB) k_prune_pipe(ChainParams<Real> P) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Real* sPow = reinterpret_cast<Real*>(smem_raw);            // [PM_SMEM_POW][NS*NS]  P_k, row-major
-  Real* sPowT = sPow + PM_SMEM_POW * NS * NS;                // [PM_SMEM_POW][NS*NS]  P_k transposed
-  const int npow_s = min(PM_SMEM_POW, P.jcap);
-  for (int i = threadIdx.x; i < npow_s * NS * NS; i += blockDim.x) {
-    const Real v = P.ppow[i];
-    sPow[i] = v;
-    const int k = i / (NS * NS), r = (i / NS) % NS, c = i % NS;
-    sPowT[k * NS * NS + c * NS + r] = v;
-  }
-  __syncthreads();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  const long long S = P.S;
-  const long long site_raw = P.tile_base + (long long)blockIdx.x * 32 + lane;
-  const bool active = site_raw < S;
-  const long long site = active ? site_raw : S - 1;
-  const bool parity = P.parity_tips != 0;
-  const bool normalize = P.normalize != 0;
-  const int T = P.T;
-  const uint32_t* __restrict__ meta = P.meta + site;
-  const uint8_t* __restrict__ tip = P.tipcode + site;
-  Real* PLs = P.PL + (site - P.tile_base) * NS;
-  const long long rowPL = P.pl_S * NS;
-  const int4* __restrict__ ent = reinterpret_cast<const int4*>(P.up_entries8);  // (pn, a, ea, b) (eb, -, -, -)
-
-  auto load = [&](PruneNode<Real, NS>* nd, int idx, int end) {
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      const int id = min(idx + u * nw, end - 1);
-      const int4 e0 = __ldg(ent + 2 * id), e1 = __ldg(ent + 2 * id + 1);
-      nd[u].pn = e0.x;
-      nd[u].ma = meta[(long long)e0.z * S];
-      nd[u].mb = meta[(long long)e1.x * S];
-      nd[u].ca = -1; nd[u].cb = -1;
-      if (e0.y < T) nd[u].ca = tip[(long long)e0.y * P.TS];
-      else VecIO<Real, NS>::load(PLs + (long long)(e0.y - T) * rowPL, NS, nd[u].va);
-      if (e0.w < T) nd[u].cb = tip[(long long)e0.w * P.TS];
-      else VecIO<Real, NS>::load(PLs + (long long)(e0.w - T) * rowPL, NS, nd[u].vb);
-    }
-  };
-  // child contribution: P_k v for an internal child, column `code` of P_k for a tip
-  auto contribution = [&](int k, int code, Real* v) {
-    if (code >= 0 && !parity && k < npow_s) {
-      VecIO<Real, NS>::load(sPowT + k * NS * NS + code * NS, NS, v);
-    } else {
-      if (code >= 0) tip_partial<Real, NS>(code, NS, parity, v);
-      pow_times<Real, NS>(P, sPow, npow_s, k, v);
-    }
-  };
-  auto compute = [&](PruneNode<Real, NS>* nd, int idx, int end) {
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      if (idx + u * nw < end) {  // warp-uniform
-        contribution((int)(nd[u].mb & 0xffffu) - 1, nd[u].cb, nd[u].vb);
-        contribution((int)(nd[u].ma & 0xffffu) - 1, nd[u].ca, nd[u].va);
-        Real out[NS];
-        Real s = 0;
-#pragma unroll
-        for (int j = 0; j < NS; j++) { out[j] = nd[u].vb[j] * nd[u].va[j]; s += out[j]; }
-        if (normalize) {
-          // structural zeros must stay zeros (no floor); a product that underflowed altogether becomes the zero
-          // vector and surfaces in the draw as "Not enough positive probabilities", like a NaN would in the reference
-          if (sizeof(Real) == 4 && !(s > (Real)1e-30)) {  // FP32: redo an underflowed product in double (see k_prune_clade)
-            double d[NS], ds = 0;
-#pragma unroll
-            for (int j = 0; j < NS; j++) { d[j] = (double)nd[u].vb[j] * (double)nd[u].va[j]; ds += d[j]; }
-            const double di = ds > 0 ? 1.0 / ds : 0.0;
-#pragma unroll
-            for (int j = 0; j < NS; j++) out[j] = (Real)(d[j] * di);
-          } else {
-            const Real inv = s > (Real)0 ? fast_rcp<Real>(s) : (Real)0;
-#pragma unroll
-            for (int j = 0; j < NS; j++) out[j] *= inv;
-          }
-        }
-        if (active) VecIO<Real, NS>::store(PLs + (long long)(nd[u].pn - T) * rowPL, NS, out);
-      }
-    }
-  };
-
-  PruneNode<Real, NS> A[U], B[U];
-  for (int l = 0; l < P.n_up_levels; l++) {
-    const int beg = __ldg(P.up_off + l), end = __ldg(P.up_off + l + 1);
-    const int step = U * nw;
-    int idx = beg + warp;
-    if (idx < end) load(A, idx, end);
-    while (idx < end) {
-      if (idx + step < end) load(B, idx + step, end);
-      compute(A, idx, end);
-      idx += step;
-      if (idx >= end) break;
-      if (idx + step < end) load(A, idx + step, end);
-      compute(B, idx, end);
-      idx += step;
-    }
-    __syncthreads();
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// K1, production arithmetic, clade order.  k_prune_pipe walks the tree level by level, so a partial written at one
-// level is read back from HBM a whole level later: 410 KB of traffic per site, 40 % of it re-reads of what the kernel
-// wrote itself.  Here every warp walks complete subtrees ("clades", pm_tree.hpp) alone, in post-order with the larger
-// child first:
-//   * a parent follows its last child immediately -> that child's partial is taken from registers;
-//   * its other internal child was finished a few nodes earlier by the same lane -> an L2 hit (same thread, same
-//     address: program order makes the store visible to the load);
-//   * jump counts and tip codes never depend on the kernel's own output, so they are fetched DEPTH nodes ahead;
-//   * no block-wide barrier until the clades are done; the few hundred nodes above them go level by level as before.
-// The schedule is uniform over the warp: lanes read 32 entries at once and hand them out with shuffles.
-// Results are bit-identical to k_prune_pipe (same operands, same operation order per node).
-// ------------------------------------------------------------------------------------------------
 // ---- shared-memory ring helpers (32-bit shared addresses, no generic-pointer arithmetic in the loop) ----
 __device__ __forceinline__ void cp_async4(unsigned dst, const void* gsrc, bool pred) {
   const int sz = pred ? 4 : 0;  // src-size 0: the destination is zero-filled, nothing is read
@@ -412,7 +303,7 @@ __device__ __forceinline__ void prune_clade_block(const ChainParams<Real>& P, co
     Real sum = 0;
 #pragma unroll
     for (int j = 0; j < NS; j++) { out[j] = vb[j] * va[j]; sum += out[j]; }
-    if (sizeof(Real) == 4 && !(sum > (Real)1e-30) && !(P.tune & 2)) {
+    if (sizeof(Real) == 4 && !(sum > (Real)1e-30)) {
       // FP32 only, rare: two clades that each all but settle a DIFFERENT state (1e-20 x 1e-20): the products underflow
       // although both factors are representable.  Redo this node in double, where they cannot.
       double d[NS], ds = 0;
@@ -1986,7 +1877,7 @@ __global__ void __launch_bounds__(128, MINB) k_paths_hard(ChainParams<Real> P, u
           while (b2) { s_stage[warp][pos++] = (unsigned short)(lane * 32 + __ffs((int)b2) - 1); b2 &= b2 - 1u; }
         }
         __syncwarp();
-        short_ok = !first && !(P.tune & 1) && PN::mul(rate_max, __ldg(P.e_len + e)) <= (Real)(PM_LAMBDA_INV - 0.5);  // (sums of two products stay below PM_LAMBDA_INV)
+        short_ok = !first && PN::mul(rate_max, __ldg(P.e_len + e)) <= (Real)(PM_LAMBDA_INV - 0.5);  // (sums of two products stay below PM_LAMBDA_INV)
         prow = (long long)__ldg(P.e_parent + e) * S; crow = (long long)__ldg(P.e_child + e) * S; erow = (long long)e * S;
       }
     }

@@ -8,9 +8,8 @@ namespace pm {
 
 template <typename Real, int NS, bool EXACT>
 struct Sweep {
-  static void prune(const ChainParams<Real>& P, int grid, size_t smem, cudaStream_t st, int variant);
+  static void prune(const ChainParams<Real>& P, int grid, size_t smem, cudaStream_t st);
   static void nodes(const ChainParams<Real>& P, int grid, size_t smem, cudaStream_t st, uint32_t iter);
-  // production, n = 2 / 4: the fused persistent prune + node-draw kernel over the site blocks [b0, b1); phases 1 = prune only
   // production, n = 2 / 4: the fused prune + node-draw kernel over the site blocks [b0, b0 + grid); phases 1 = prune only.
   // slot_busy: slots_per_sm flags per SM (nullptr: block i uses slot i).  fused_blocks_per_sm: resident blocks per SM.
   static int fused_blocks_per_sm(size_t smem_nodes);

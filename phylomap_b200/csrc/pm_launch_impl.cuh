@@ -4,24 +4,14 @@
 namespace pm {
 
 template <typename Real, int NS, bool EXACT>
-void Sweep<Real, NS, EXACT>::prune(const ChainParams<Real>& P, int grid, size_t smem, cudaStream_t st, int variant) {
+void Sweep<Real, NS, EXACT>::prune(const ChainParams<Real>& P, int grid, size_t smem, cudaStream_t st) {
   if constexpr (!EXACT && (NS == 2 || NS == 4)) {
-    const size_t spipe = 2 * PM_SMEM_POW * NS * NS * sizeof(Real);
-    // 4x: clade order (default); 2x: level order (the kernel it replaced, kept for comparison)
-    auto clade = [&](auto kern, int depth) {
-      const size_t sm = spipe + (size_t)PM_CLADE_SLOT * 8 * depth;
-      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-      kern<<<grid, 256, sm, st>>>(P);
-    };
-    if (variant == 20) k_prune_pipe<Real, NS, 2, 3><<<grid, 256, spipe, st>>>(P);  // two nodes per round
-    else if (variant == 21) k_prune_pipe<Real, NS, 1, 4><<<grid, 256, spipe, st>>>(P);
-    else if (variant == 41) clade(k_prune_clade<Real, NS, 4, 4>, 4);
-    else if (variant == 43) clade(k_prune_clade<Real, NS, 8, 3>, 8);
-    else if (variant == 44) clade(k_prune_clade<Real, NS, 16, 4>, 16);
-    else if (variant == 45) clade(k_prune_clade<Real, NS, 6, 3>, 6);
-    else if (variant == 46) clade(k_prune_clade<Real, NS, 6, 5>, 6);
-    else if (variant == 47) clade(k_prune_clade<Real, NS, 8, 4>, 8);
-    else clade(k_prune_clade<Real, NS, 8, (sizeof(Real) == 8 ? 2 : 3)>, 8);  // FP64 needs the registers of 2 blocks / SM
+    constexpr int D = 8, MB = sizeof(Real) == 8 ? 2 : 3;  // FP64 needs the registers of 2 blocks / SM
+    const size_t spow = 2 * PM_SMEM_POW * NS * NS * sizeof(Real);  // the power table and its transpose
+    const size_t sm = spow + (size_t)PM_CLADE_SLOT * 8 * D;
+    auto kern = k_prune_clade<Real, NS, D, MB>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    kern<<<grid, 256, sm, st>>>(P);
   }
   else k_prune<Real, NS, EXACT><<<grid, 256, smem, st>>>(P);
 }
@@ -93,8 +83,7 @@ void Sweep<Real, NS, EXACT>::small_chain(const ChainParams<Real>& P, int sites, 
                                          const SmallOut& out, bool two_per_sm) {
   if constexpr (!EXACT && (NS == 2 || NS == 4)) {
     const size_t sm = (size_t)SmallSmem<Real, NS>(P.T).total;
-    const bool two = (P.tune & 8) ? false : (P.tune & 16) ? true : two_per_sm;  // (PHYLOMAP_B200_TUNE 8 / 16 force either)
-    auto kern = two ? k_small_chain<Real, NS, 2> : k_small_chain<Real, NS, 1>;
+    auto kern = two_per_sm ? k_small_chain<Real, NS, 2> : k_small_chain<Real, NS, 1>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
     kern<<<sites, 256, sm, st>>>(P, iter0, nsweeps, out);
   }

@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
     Real sum = 0;
 #pragma unroll
     for (int j = 0; j < NS; j++) { o[j] = vb[j] * va[j]; sum += o[j]; }
-    if (sizeof(Real) == 4 && !(sum > (Real)1e-30) && !(P.tune & 2)) {
+    if (sizeof(Real) == 4 && !(sum > (Real)1e-30)) {
       double d[NS], ds = 0;
 #pragma unroll
       for (int j = 0; j < NS; j++) { d[j] = (double)vb[j] * (double)va[j]; ds += d[j]; }

@@ -1,6 +1,5 @@
 """Where the one-block-per-site chain kernel (pm_small.cuh) stops paying: microseconds per sweep of a resident chain, one
-character, against the 32-sites-per-warp kernels, as the work of a site (branches + jump points) grows; and one or two
-blocks per SM when there are more sites than SMs."""
+character, against the 32-sites-per-warp kernels, as the work of a site (branches + jump points) grows."""
 import os, sys, time, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
@@ -9,8 +8,8 @@ import cases
 import phylomap_b200 as pb
 from phylomap_b200 import capi, synth
 
-def resident(z, Q, pid, Om, n_sweeps, prec="f32", variant=capi.PM_V_BIGTREE):
-    ch = pb.Chain(variant, z, Q, pid, Om, 5 * n_sweeps, precision=prec, seed=5)
+def resident(z, Q, pid, Om, n_sweeps, prec="f32"):
+    ch = pb.Chain(capi.PM_V_BIGTREE, z, Q, pid, Om, 5 * n_sweeps, precision=prec, seed=5)
     ch.run(n_sweeps)
     best = 1e30
     for _ in range(3):
@@ -33,13 +32,4 @@ for name, T, mb, Om, S, n_sw in [("T100_Om2.4", 100, 1.0, 2.4, 1, 400), ("T100_O
         os.environ["PHYLOMAP_B200_SMALL"] = small
         row["one_block_per_site" if small == "1" else "wide"] = resident(z, Q4.copy(), pid4, Om, n_sw)
     out[name] = row
-os.environ["PHYLOMAP_B200_SMALL"] = "1"
-z1 = cases.tree2(T=100, S=1, seed=1, mean_branch=5.0)
-z592 = cases.tree2(T=100, S=592, seed=1, mean_branch=5.0)
-z296 = cases.tree2(T=100, S=296, seed=1, mean_branch=5.0)
-for tune, label in (("8", "one_block_per_sm"), ("16", "two_blocks_per_sm")):
-    os.environ["PHYLOMAP_B200_TUNE"] = tune
-    out["cfg0_S1_" + label] = resident(z1, cases.Q2, cases.PID2, 0.2, 1000, variant=capi.PM_V_PLAIN)
-    out["cfg0_S296_" + label] = resident(z296, cases.Q2, cases.PID2, 0.2, 200, variant=capi.PM_V_PLAIN)
-    out["cfg0_S592_" + label] = resident(z592, cases.Q2, cases.PID2, 0.2, 200, variant=capi.PM_V_PLAIN)
 print(json.dumps(out))
