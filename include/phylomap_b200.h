@@ -228,6 +228,7 @@ void pm_chain_overheads(pm_chain* c, double ms[2]);
 int pm_chain_get_node_states(pm_chain* c, int32_t tree, int32_t* out /* [S][2T-1] 0-based */);
 int pm_chain_get_piece_counts(pm_chain* c, int32_t tree, int32_t* out /* [S][E] */);
 int pm_chain_get_path(pm_chain* c, int32_t tree, int64_t site, int32_t e, double* len, int32_t* st, int32_t cap);
+/* Partials of the current chain state at `site`, computed by a pruning pass that the call runs; tip rows are zero. */
 int pm_chain_get_partials(pm_chain* c, int32_t tree, int64_t site, double* out /* [2T-1][n], tip rows zero */);
 int64_t pm_chain_device_bytes(pm_chain* c);
 /* Rate-updating samplers: per rate parameter, in the order of the trace columns (l01, l10, then for the hidden-rate

@@ -21,6 +21,7 @@
 #include <memory>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/phylomap_b200.h"
@@ -222,6 +223,51 @@ long long chernoff_records_cap(const std::vector<double>& lams, double eps, doub
   return (long long)std::ceil(best);
 }
 
+// The run-time switches of INTEGRATION.md §5, read once: when a chain is created (and by the one-call entries, for the
+// site tile).  PHYLOMAP_B200_CACHE belongs to the process-wide device pool and is read there.
+struct Switches {
+  bool small = true;             // PHYLOMAP_B200_SMALL=0: never the one-block-per-site kernel
+  bool small_sites_set = false;  // PHYLOMAP_B200_SMALL_SITES=k: its site limit instead of the cost rule
+  long long small_sites = 0;
+  double small_work = 1.0;       // PHYLOMAP_B200_SMALL_WORK=f: scales its limit on the expected path cost
+  bool rec_pool = true;          // PHYLOMAP_B200_REC_POOL=0: one record slice per site
+  bool fused = true;             // PHYLOMAP_B200_FUSED=0: pruning and node draws as two kernels
+  int graph = -1;                // PHYLOMAP_B200_GRAPH: 0 never, 1 always replay a captured sweep, otherwise by problem size
+  bool trace = false;            // PHYLOMAP_B200_TRACE=1: host wall time of the phases of create(), on stderr
+  bool debug_sync = false;       // PHYLOMAP_B200_DEBUG_SYNC=1: stop at the first sweep kernel that raises a device error flag
+  bool small_prof = false;       // PHYLOMAP_B200_SMALL_PROF (any value): k_small_chain counts the cycles of its phases
+  long long site_tile = 0;       // PHYLOMAP_B200_SITE_TILE=k: fixed-Q one-call entries run k sites at a time (0: all)
+};
+
+Switches read_switches() {
+  const auto env = [](const char* name) -> const char* { return getenv((std::string("PHYLOMAP_B200_") + name).c_str()); };
+  const auto starts = [&](const char* name, char c) { const char* v = env(name); return v && v[0] == c; };
+  Switches s;
+  s.small = !starts("SMALL", '0');
+  if (const char* v = env("SMALL_SITES")) { s.small_sites_set = true; s.small_sites = atoll(v); }
+  if (const char* v = env("SMALL_WORK")) s.small_work = atof(v);
+  s.rec_pool = !starts("REC_POOL", '0');
+  s.fused = !starts("FUSED", '0');
+  if (const char* v = env("GRAPH")) s.graph = atoi(v);
+  s.trace = starts("TRACE", '1');
+  s.debug_sync = starts("DEBUG_SYNC", '1');
+  s.small_prof = env("SMALL_PROF") != nullptr;
+  if (const char* v = env("SITE_TILE")) s.site_tile = atoll(v);
+  return s;
+}
+
+// Host wall time of the phases of a chain's construction (PHYLOMAP_B200_TRACE=1), on stderr.
+struct PhaseTrace {
+  bool on;
+  std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+  void mark(const char* what) {
+    if (!on) return;
+    const auto now = std::chrono::steady_clock::now();
+    fprintf(stderr, "[phylomap_b200] create: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - t0).count());
+    t0 = now;
+  }
+};
+
 }  // namespace
 
 // Range of %smid on a device (asked once per device with a one-thread kernel, see k_nsmid).
@@ -286,13 +332,256 @@ struct pm_chain {
 
 namespace {
 
+// ---- the plan of a tree's chain state: functions of the tree, the model and the options alone ----
+
+// One block per site, state in shared memory (pm_small.cuh), when the sites are few and the tree fits: production
+// arithmetic, 2 / 4 states (`eligible`; `smem`: the kernel's dynamic shared memory for this tree).  PHYLOMAP_B200_SMALL=0
+// keeps the 32-sites-per-warp kernels (same rows: the tests compare), PHYLOMAP_B200_SMALL_SITES moves the site limit.
+struct SmallChoice { bool ok, two; };  // two: more sites than SMs, two blocks per SM (128 registers) instead of one
+template <typename Real>
+SmallChoice choose_small_kernel(bool eligible, const std::vector<Real>& elen, double Omega, int T, long long S, int sms,
+                                size_t smem, const Switches& sw) {
+  long long small_sites = 16LL * sms;   // (hard cap; the cost rule below decides before it)
+  if (sw.small_sites_set) small_sites = sw.small_sites;
+  // ... and the paths of one site are short: a block walks its site's branches with 256 threads, one branch per thread
+  // at a time, while the wide kernels spread the branch-sites of a long-path problem (the Squamate vignette: 877 000
+  // jump points per site and sweep) over the whole device.  What costs is the general item routine: hard = the sum
+  // over the branches of P(two or more jump points) x (2 + expected jump points), jump points ~ Poisson(Omega t).
+  // Measured (scripts/small_calib.py, us per sweep, one character): this kernel ~ 20 + 0.05 hard + 0.03 T, the wide
+  // ones ~ 65 + 0.13 T: it pays up to hard ~ 1500 + 0.7 T.  PHYLOMAP_B200_SMALL_WORK scales that limit.
+  double hard = 0;
+  for (size_t e = 0; e < elen.size(); e++) {
+    const double lam = Omega * (double)elen[e];
+    hard += (1.0 - std::exp(-lam) * (1.0 + lam)) * (2.0 + lam);
+  }
+  const double work_limit = sw.small_work * (1500.0 + 0.7 * T);
+  SmallChoice c;
+  c.two = S > sms;
+  // More sites than SMs: two blocks per SM, waves of 2 x SMs sites; measured (profiles/r2_warp_per_site_attempt.log,
+  // 100-800 tips, 296-2368 sites) a wave takes ~ 10 + 0.28 T + 0.05 hard us and the wide kernels ~ 160 + 0.09 T + 0.01 S.
+  bool sites_ok = S <= small_sites;
+  if (c.two && !sw.small_sites_set) {
+    const double waves = std::ceil((double)S / (2.0 * sms));
+    sites_ok = sites_ok && waves * (10.0 + 0.28 * T + 0.05 * hard) < 160.0 + 0.09 * T + 0.01 * (double)S;
+  }
+  c.ok = sw.small && eligible && sites_ok && smem <= (size_t)200 * 1024 && hard <= work_limit;
+  return c;
+}
+
+// Launch geometry of the path kernels and the record capacity of every branch chunk, with slices shared by groups of
+// 2^rec_shift consecutive sites.  (Production: the offset of a path's records inside its slice is a 16-bit field of the
+// state word, so a chunk whose slice would be longer is split.)  Production slices are shared by groups of 32 consecutive
+// sites (rec_shift = 5): the bound on the records of 32 independent sites together is far tighter, relative to its mean,
+// than 32 bounds on one site each (3.8 -> 0.3 bytes per branch-site at the benchmark's size).  Where such a slice would
+// not fit the 16-bit offset (long paths: the Squamate vignette) the plan is returned with fits = false, and the caller
+// plans again with rec_shift = 0: every site keeps its own.
+struct RecordPlan {
+  int rec_shift = 0;
+  long long gx = 0, ny = 0;  // path-kernel grid: site blocks x branch chunks
+  int chunk = 0;             // consecutive branches per chunk
+  std::vector<int> cap_off;  // [ny + 1] prefix sums of the chunks' record capacities (per slice)
+  bool fits = true;
+};
+template <typename Real>
+RecordPlan plan_records(int rec_shift, const std::vector<Real>& elen, const std::vector<long long>& moff, long long S,
+                        double Omega, bool exact, bool no_paths, int path_capacity) {
+  const int E = (int)elen.size();
+  RecordPlan p;
+  p.rec_shift = rec_shift;
+  // a thread owns one site x one chunk of consecutive branches
+  p.gx = (S + 127) / 128;
+  long long ny = (148LL * 16 * 6 + p.gx - 1) / p.gx;
+  ny = std::max(1LL, std::min<long long>(ny, (E + 15) / 16));
+  ny = std::min<long long>(ny, 65535);
+  ny = std::max<long long>(ny, (E + 2047) / 2048);  // the easy path kernel stages a chunk's topology in shared memory
+  ny = std::max<long long>(ny, (E + ((1LL << 32) - 1) / S - 1) / std::max<long long>(1, ((1LL << 32) - 1) / S));  // ... and indexes the rows of a chunk with 32 bits: chunk x S < 2^32
+  const double G = (double)(1 << rec_shift);
+  for (;;) {
+    p.chunk = (int)((E + ny - 1) / ny);
+    ny = (E + p.chunk - 1) / p.chunk;
+    long long cap_max = 0;
+    // Real jumps sit on uniformization points, and in equilibrium the points of a chunk are Poisson(Omega x total
+    // length), so the Poisson tail bounds them; a path with j real jumps stores j + 1 runs (<= 2j).  The first sweep
+    // instead finds its points in the caller's maps (m_e - 1 per branch), so the initial segmentation is a second lower
+    // bound.
+    p.cap_off.assign(ny + 1, 0);
+    for (long long c = 0; c < ny; c++) {
+      const int b0 = (int)c * p.chunk, b1 = std::min(E, b0 + p.chunk);
+      double len = 0;
+      long long init_records = 0;
+      for (int e = b0; e < b1; e++) {
+        len += (double)elen[e];
+        const long long m0 = moff[e + 1] - moff[e];
+        if (exact || m0 >= 2) init_records += m0;
+      }
+      long long cap;
+      if (no_paths) cap = 4;
+      else if (path_capacity > 0) cap = (long long)path_capacity * (b1 - b0) * (long long)G;
+      else if (exact) {
+        const int jumps = poisson_cap(1.5 * Omega * len + 1.0, 1e-18);
+        cap = std::max<long long>((long long)(b1 - b0) + jumps, init_records);
+      } else {
+        // production: only paths with >= 2 real jumps keep records (j + 1 of them); Chernoff bound on their sum
+        // over the chunk with every branch's jump count dominated by Poisson(1.5 Omega t)
+        std::vector<double> lams;
+        long long init3 = 0;
+        for (int e = b0; e < b1; e++) {
+          lams.push_back(1.5 * Omega * (double)elen[e]);
+          const long long m0 = moff[e + 1] - moff[e];
+          if (m0 >= 3) init3 += m0;
+        }
+        // ... or, simpler and valid for any rate: every path stores at most (jumps + 1) records (+ a header), and the
+        // jumps of the chunk together are dominated by one Poisson variable
+        double lam_sum = 0, lam_max = 0;
+        for (double l : lams) { lam_sum += l; lam_max = std::max(lam_max, l); }
+        const long long simple = (long long)poisson_cap(G * lam_sum, 1e-18) + 2LL * (b1 - b0) * (long long)G;
+        long long stat = simple;
+        if (lam_max < 200.0) stat = std::min(stat, chernoff_records_cap(lams, 1e-18, G));  // (its series stops at 400 terms)
+        cap = std::max<long long>(stat, init3 * (long long)G) + 4;
+      }
+      if (cap > (1 << 28)) { if (rec_shift) cap = 1 << 28; else fail(PM_ERR_CAPACITY, "path capacity of a branch chunk too large"); }
+      cap = (cap + 3) & ~3;  // keep every slice 16-byte aligned
+      cap_max = std::max(cap_max, cap);
+      p.cap_off[c + 1] = p.cap_off[c] + (int)cap;
+    }
+    if (exact || no_paths || cap_max <= 65535) break;
+    if (rec_shift) { p.fits = false; break; }  // shared slices too long for the offset field
+    if (p.chunk <= 1 || ny >= 65535) fail(PM_ERR_CAPACITY, "a branch needs more than 65 535 path records per site");
+    ny = std::min<long long>(std::min<long long>(2 * ny, E), 65535);
+  }
+  p.ny = ny;
+  return p;
+}
+
+// The clade schedule of the production pruning and node-draw kernels (n = 2, 4), encoded as the byte offsets the kernels
+// add to their per-lane bases.  rowPL: bytes of one node row of the partials buffer.
+struct CladeCode {
+  pm::host::CladeSchedule cs;   // (cs.top_off relative to the first top entry)
+  std::vector<int> e16, top;    // bottom-up: the warps' entries, PM_CLADE_ENTRY_INTS ints each; the top levels
+  std::vector<int> d16;         // top-down (k_nodes_clade): 16 ints per node
+  std::vector<long long> tips;  // redrawn tips: entry v = tip v: the parent's node-state row, the jump-count row of its branch (bytes)
+};
+CladeCode encode_clade_schedule(const pm::host::Schedule& sch, long long S, long long TS, long long rowPL, bool redraw_tips) {
+  const int T = sch.T;
+  CladeCode c;
+  pm::host::CladeSchedule& cs = c.cs;
+  // clades of ~1/64 of the tree: ~8 per warp to balance, and only ~100 nodes left above them.  Small trees (where a
+  // sweep is a matter of latency, not throughput): ~1/8 of the tree, so that almost every node is walked inside a
+  // warp's prefetched sequence and only a few levels with block barriers are left above.  (A function of the tree
+  // alone: the node draws are keyed by schedule position, and a site must not depend on how many others run.)
+  const int clade_max = (T - 1 < 512) ? std::max(8, (T - 1) / 8) : std::max(8, std::min(512, (T - 1) / 64));
+  pm::host::build_clade_schedule(sch, 8, clade_max, cs);
+  const int n1 = cs.warp_off.back();
+  c.e16.assign((size_t)PM_CLADE_ENTRY_INTS * (n1 + 17), 0);  // padded: the kernel forms addresses up to 16 entries ahead
+  auto put64 = [](int* dst, long long v) { dst[0] = (int)(unsigned)(v & 0xffffffffLL); dst[1] = (int)(v >> 32); };
+  for (int i = 0; i < n1; i++) {
+    const int* en = &cs.entries[(size_t)8 * i];
+    int* o = &c.e16[(size_t)PM_CLADE_ENTRY_INTS * i];
+    const int pn = en[0], a = en[1], ea = en[2], b = en[3], eb = en[4];
+    int fl = en[5] & 3;
+    const int x = (en[5] & 4) ? a : (en[5] & 8) ? b : -1;
+    if (a < T) fl |= 16;
+    if (b < T) fl |= 32;
+    put64(o + 0, (long long)(pn - T) * rowPL);
+    put64(o + 2, x >= 0 ? (long long)(x - T) * rowPL : -1LL);
+    put64(o + 4, (long long)ea * S * 4);
+    put64(o + 6, (long long)eb * S * 4);
+    put64(o + 8, a < T ? (long long)a * TS : -1LL);
+    put64(o + 10, b < T ? (long long)b * TS : -1LL);
+    o[12] = fl;
+  }
+  c.top.assign(cs.entries.begin() + (size_t)8 * n1, cs.entries.end());
+  for (int& v : cs.top_off) v -= n1;
+  const int n2 = cs.down_warp_off.back();
+  c.d16.assign((size_t)16 * (n2 + 17), 0);
+  for (int i = 0; i < n2; i++) {
+    const int* en = &cs.down_seq[(size_t)4 * i];
+    int* o = &c.d16[(size_t)16 * i];
+    put64(o + 0, (long long)(en[0] - T) * rowPL);
+    put64(o + 2, (long long)en[2] * S * 4);
+    put64(o + 4, (long long)en[0] * S);
+    put64(o + 6, en[3] ? -1LL : (long long)en[1] * S);
+  }
+  if (redraw_tips)
+    for (int v = 0; v < T; v++) {
+      const int e = sch.parent_edge[v];
+      c.tips.push_back((long long)sch.e_parent[e] * S); c.tips.push_back((long long)e * S * 4);
+    }
+  return c;
+}
+
+// The one-block-per-site kernel's node draws and branch order.
+struct SmallOrder {
+  std::vector<int> down;    // 4 ints per drawn node: the generic schedule's (v, parent, edge) and the clade kernel's draw key
+  std::vector<int> border;  // which thread takes which branch (-1: none)
+};
+template <typename Real>
+SmallOrder small_draw_order(const pm::host::Schedule& sch, const pm::host::CladeSchedule& cs, const std::vector<Real>& elen) {
+  const int T = sch.T, E = (int)elen.size();
+  SmallOrder so;
+  // the same draws node by node: every drawn node with the Philox block and word the clade kernel gives it
+  // (k_small_chain decodes the key), grouped by depth like the generic schedule
+  std::vector<uint32_t> key(2 * (size_t)T - 1, 0u);
+  for (int i = 0; i < (int)cs.down_top.size() / 4; i++) key[cs.down_top[(size_t)4 * i]] = 0x80000000u | (uint32_t)i;
+  for (int i = 0; i < cs.down_warp_off.back(); i++) key[cs.down_seq[(size_t)4 * i]] = (uint32_t)i;
+  for (int v = 0; v < T; v++) key[v] = 0x40000000u | (uint32_t)v;
+  const int nd = (int)sch.down_entries.size() / 3;
+  so.down.assign((size_t)4 * std::max(nd, 1), 0);
+  for (int i = 0; i < nd; i++) {
+    const int* en = &sch.down_entries[(size_t)3 * i];
+    so.down[(size_t)4 * i] = en[0]; so.down[(size_t)4 * i + 1] = en[1]; so.down[(size_t)4 * i + 2] = en[2]; so.down[(size_t)4 * i + 3] = (int)key[en[0]];
+  }
+  // Which thread takes which branch.  A warp runs the general item routine in lockstep: it takes as long as its
+  // longest path, plus a share for every other shape among its items.  Up to 256 branches (one per thread): the
+  // branches sorted by decreasing length are DEALT over the 8 warps, so that every warp gets one of the longest,
+  // one of the next eight, ... (measured on configs[0]: all long branches in one warp 30 300 cycles for the path
+  // phase, edge order 26 000).  Larger trees: decreasing length (warps of similar paths: throughput).
+  std::vector<int> sorted(E);
+  for (int e = 0; e < E; e++) sorted[e] = e;
+  std::stable_sort(sorted.begin(), sorted.end(), [&](int x, int y) { return elen[x] > elen[y]; });
+  if (E <= 256) {
+    so.border.assign(256, -1);
+    for (int k = 0; k < E; k++) so.border[(size_t)(k % 8) * 32 + k / 8] = sorted[k];   // warp k % 8, lane k / 8
+  } else so.border = sorted;
+  return so;
+}
+
+// Branch-major ballot array and the general path kernel's work items: branch e is cut into items of g_e ballot words
+// (32 g_e sites), g_e chosen so that an item holds ~96 branch-sites with two or more jump points in equilibrium (their
+// number on a branch of length t is Poisson(Omega t)).
+struct WorkItems {
+  std::vector<long long> off;  // [E + 1] first item of every branch
+  std::vector<int> g;          // ballot words per item, per branch
+  std::vector<int> hint;       // branch of item 64 i
+};
+template <typename Real>
+WorkItems build_work_items(const std::vector<Real>& elen, double Omega, long long S) {
+  const int E = (int)elen.size();
+  const long long Wl = (S + 31) / 32;
+  WorkItems w;
+  w.off.assign(E + 1, 0);
+  w.g.resize(E);
+  for (int e = 0; e < E; e++) {
+    const double lam = Omega * (double)elen[e];
+    const double h = std::max(1e-6, 1.0 - std::exp(-lam) * (1.0 + lam));
+    long long g = (long long)std::ceil(96.0 / (32.0 * h));
+    g = std::max(1LL, std::min<long long>(std::min<long long>(g, 32), Wl));
+    w.g[e] = (int)g;
+    w.off[e + 1] = w.off[e] + (Wl + g - 1) / g;
+  }
+  w.hint.resize((size_t)(w.off[E] >> 6) + 1);
+  for (long long i = 0, e = 0; i < (long long)w.hint.size(); i++) {
+    while (e + 1 < E && w.off[e + 1] <= (i << 6)) e++;
+    w.hint[i] = (int)e;
+  }
+  return w;
+}
+
 template <typename Real>
 struct TreeDev {
   pm::host::Schedule sch;
   long long S = 0, TS = 0;
-  DevBuf cl_entries, cl_warp_off, cl_top_entries, cl_top_off, cd_top, cd_top_off, cd_entries, cd_warp_off, cd_tips;
-  int n_cd_top_levels = 0, n_cd_tips = 0;  // clade schedule of the production pruning kernel
-  int n_cl_top_levels = 0;
+  DevBuf cl_entries, cl_warp_off, cl_top_entries, cl_top_off, cd_top, cd_top_off, cd_entries, cd_warp_off, cd_tips;  // clade schedule
   DevBuf up_entries, up_off, down_entries, down_off, e_parent, e_child, e_len, maps_off, maps_len, cap_off;
   DevBuf tipcode, node_state, meta, PL, rec_len[2], rec_st[2], dw_partial, hard_ballot, wk_off, wk_g, wk_hint, wk_item, rec_cursor, shape;
   long long wk_total = 0, dw_rows = 0;
@@ -350,7 +639,7 @@ struct ChainT : pm_chain {
   std::unique_ptr<pm::host::ReplaySource> replay;
   size_t smem_prune = 0, smem_nodes = 0, smem_paths = 0;
   int rows_cap = 0;
-  bool debug_sync = false; int debug_kernel = 0;
+  int debug_kernel = 0;
   struct Timed { cudaEvent_t a, b; int k; };
   std::vector<Timed> timed;
   // CUDA-graph replay of one sweep (fixed-Q samplers on small problems: a sweep of a 100-tip tree is seven launches of a
@@ -361,8 +650,8 @@ struct ChainT : pm_chain {
   cudaGraphExec_t sweep_graph = nullptr;
   void* graph_rows = nullptr;         // the rows buffer the graph writes to (re-captured if it moves)
   bool capturing = false;
-  int graph_mode = -1;                // PHYLOMAP_B200_GRAPH: 0 never, 1 always, otherwise by problem size
   int launches_per_sweep = 0;
+  Switches sw;
 
   ~ChainT() override {
     cudaSetDevice(opt.device);
@@ -432,8 +721,20 @@ struct ChainT : pm_chain {
   }
 
   // ---- kernel dispatch ----
-  int prune_grid(const TreeDev<Real>& t) const { return (int)((t.S + 31) / 32); }
-  size_t prune_smem(const TreeDev<Real>&) const { return smem_prune; }
+  // f(std::integral_constant<int, NS>) with the chain's compile-time state count: 2, 4, or 0 (run-time n)
+  template <typename F>
+  auto with_ns(F&& f) const {
+    if (NS == 2) return f(std::integral_constant<int, 2>{});
+    if (NS == 4) return f(std::integral_constant<int, 4>{});
+    return f(std::integral_constant<int, 0>{});
+  }
+  // ... and f(ns, std::bool_constant<EXACT>): the deterministic kernels exist in FP64 only
+  template <typename F>
+  auto with_ns_exact(F&& f) const {
+    if constexpr (std::is_same_v<Real, double>)
+      if (exact) return with_ns([&](auto ns) { return f(ns, std::true_type{}); });
+    return with_ns([&](auto ns) { return f(ns, std::false_type{}); });
+  }
 
   template <int NSc, bool EX>
   void launch_sweep_t(TreeDev<Real>& t, uint32_t iter, double* row) {
@@ -450,7 +751,7 @@ struct ChainT : pm_chain {
         end_timed();
       } else {
         begin_timed(0);
-        pm::Sweep<Real, NSc, EX>::prune(P, gx, prune_smem(t), stream);
+        pm::Sweep<Real, NSc, EX>::prune(P, gx, smem_prune, stream);
         end_timed();
         begin_timed(1);
         pm::Sweep<Real, NSc, EX>::nodes(P, gx, smem_nodes, stream, iter);
@@ -476,7 +777,7 @@ struct ChainT : pm_chain {
   }
   // Few sites on a small tree: sweeps [iter0, iter0 + nsweeps) of every site in one launch, a block per site, the state in
   // shared memory (pm_small.cuh); a second launch sums the sites and assembles the rows (WR doubles per sweep, from rows_d).
-  bool use_small(const TreeDev<Real>& t) const { return t.small_ok && !timing && !debug_sync && !capturing; }
+  bool use_small(const TreeDev<Real>& t) const { return t.small_ok && !timing && !sw.debug_sync && !capturing; }
   void launch_small(TreeDev<Real>& t, uint32_t iter0, int nsweeps, double* rows_d) {
     const long long S = t.S;
     pm::SmallOut o;
@@ -485,13 +786,12 @@ struct ChainT : pm_chain {
     o.br_order = t.small_border.template as<int>(); o.n_order = t.small_order_n;
     o.part = nullptr; o.cnt = nullptr; o.root = nullptr; o.rows = nullptr; o.row_stride = WR; o.err_slot = W;
     o.prof = nullptr;
-    if (getenv("PHYLOMAP_B200_SMALL_PROF")) {
+    if (sw.small_prof) {
       if (!t.small_prof.p) { t.small_prof.alloc(12 * sizeof(long long)); CK(cudaMemsetAsync(t.small_prof.p, 0, t.small_prof.bytes, stream)); }
       o.prof = t.small_prof.template as<long long>();
     }
     auto launch = [&](uint32_t it0, int nb) {
-      if (NS == 2) pm::Sweep<Real, 2, false>::small_chain(t.P, (int)S, stream, it0, nb, o, t.small_two);
-      else pm::Sweep<Real, 4, false>::small_chain(t.P, (int)S, stream, it0, nb, o, t.small_two);
+      with_ns([&](auto ns) { pm::Sweep<Real, decltype(ns)::value, false>::small_chain(t.P, (int)S, stream, it0, nb, o, t.small_two); });
     };
     if (S == 1) {  // the one block writes the rows itself: one launch, whatever the number of sweeps
       o.rows = rows_d;
@@ -524,9 +824,9 @@ struct ChainT : pm_chain {
     pm::k_transprob<Real><<<(E + 127) / 128, 128, 0, stream>>>(q_dev.as<double>(), t.e_len_d.template as<double>(), E, n,
                                                               t.TP.template as<Real>());
     const int gx = (int)((t.S + 31) / 32);
-    if (NS == 2) pm::k_loglik<Real, 2><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>());
-    else if (NS == 4) pm::k_loglik<Real, 4><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>());
-    else pm::k_loglik<Real, 0><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>());
+    with_ns([&](auto ns) {
+      pm::k_loglik<Real, decltype(ns)::value><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>());
+    });
     pm::k_reduce_ll<<<1, 256, 0, stream>>>(t.ll_partial.template as<double>(), gx, row + n + n * n + 1);
     launches += 3;
   }
@@ -539,24 +839,16 @@ struct ChainT : pm_chain {
       if (only_site >= 0) pm::Sweep<Real, NSc, EX>::prune_nodes(t.P, 1, smem_nodes, stream, 0u, only_site / 32, 1, nullptr, 0, nullptr);
       else pm::Sweep<Real, NSc, EX>::prune_nodes(t.P, (int)nb, smem_nodes, stream, 0u, 0, 1, t.slots_per_sm ? t.slot_busy.template as<int>() : nullptr,
                                                  t.slots_per_sm, nullptr);
-    } else pm::Sweep<Real, NSc, EX>::prune(t.P, (int)nb, prune_smem(t), stream);
+    } else pm::Sweep<Real, NSc, EX>::prune(t.P, (int)nb, smem_prune, stream);
     launches++;
   }
 
-  template <bool EX>
-  void launch_sweep_e(TreeDev<Real>& t, uint32_t iter, double* row) {
-    if (NS == 2) launch_sweep_t<2, EX>(t, iter, row);
-    else if (NS == 4) launch_sweep_t<4, EX>(t, iter, row);
-    else launch_sweep_t<0, EX>(t, iter, row);
+  void launch_sweep(TreeDev<Real>& t, uint32_t iter, double* row) {
+    with_ns_exact([&](auto ns, auto ex) { launch_sweep_t<decltype(ns)::value, decltype(ex)::value>(t, iter, row); });
   }
-  template <bool EX>
-  void launch_prune_e(TreeDev<Real>& t, long long only_site) {
-    if (NS == 2) launch_prune_t<2, EX>(t, only_site);
-    else if (NS == 4) launch_prune_t<4, EX>(t, only_site);
-    else launch_prune_t<0, EX>(t, only_site);
+  void launch_prune(TreeDev<Real>& t, long long only_site = -1) {
+    with_ns_exact([&](auto ns, auto ex) { launch_prune_t<decltype(ns)::value, decltype(ex)::value>(t, only_site); });
   }
-  void launch_sweep(TreeDev<Real>& t, uint32_t iter, double* row);
-  void launch_prune(TreeDev<Real>& t, long long only_site = -1);
 
   void begin_timed(int k) {
     debug_kernel = k;
@@ -568,7 +860,7 @@ struct ChainT : pm_chain {
   }
   void end_timed() {
     if (timing) CK(cudaEventRecord(timed.back().b, stream));
-    if (debug_sync) {  // PHYLOMAP_B200_DEBUG_SYNC=1: stop at the first kernel that raises a device error flag
+    if (sw.debug_sync) {  // PHYLOMAP_B200_DEBUG_SYNC=1: stop at the first kernel that raises a device error flag
       try { check_device_errors(); }
       catch (Fail& f) { f.msg += " [raised by sweep kernel #" + std::to_string(debug_kernel) + ": 0 prune, 1 nodes, 2 paths, 3 reduce]"; throw; }
     }
@@ -620,19 +912,82 @@ struct ChainT : pm_chain {
     V = variant_of(variant);
     n = n_; ntrees = ntr; N_total = Ntot; Q = Q_; B = B_; Omega = Om;
     opt = *o;
-    // PHYLOMAP_B200_TRACE=1: host wall time of the phases of a chain's construction, on stderr
-    const bool trace = getenv("PHYLOMAP_B200_TRACE") && getenv("PHYLOMAP_B200_TRACE")[0] == '1';
-    auto trace_t0 = std::chrono::steady_clock::now();
-    auto mark = [&](const char* what) {
-      if (!trace) return;
-      const auto now = std::chrono::steady_clock::now();
-      fprintf(stderr, "[phylomap_b200] create: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(now - trace_t0).count());
-      trace_t0 = now;
-    };
+    sw = read_switches();
+    PhaseTrace trace{sw.trace};
+    std::vector<pm::host::Schedule> schedules = validate(variant, tr, pid_, prior_, nprior);
+    trace.mark("validation + schedules");
+    const int sms = open_device();
+    trace.mark("device queries + stream");
+    err_flag.alloc(sizeof(unsigned));
+    CK(cudaMemsetAsync(err_flag.p, 0, err_flag.bytes, stream));
+    // a second stream for the upload of the tip states (the largest transfer of create()): everything else -- schedule
+    // uploads, the set-up kernels -- goes on `stream` meanwhile; the two are joined before create() returns
+    cudaStream_t aux = nullptr;
+    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
+    struct AuxGuard {
+      cudaStream_t& s; cudaEvent_t& a; cudaEvent_t& b;
+      ~AuxGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
+    } aux_guard{aux, ev_a, ev_b};
+    CK(cudaStreamCreateWithFlags(&aux, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&ev_a, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&ev_b, cudaEventDisableTiming));
+    CK(cudaEventRecord(ev_a, stream));   // (the error flag is zeroed on `stream`)
+    CK(cudaStreamWaitEvent(aux, ev_a, 0));
+    double tmax = 0;
+    for (int ti = 0; ti < ntr; ti++) trees.push_back(create_tree(tr[ti], ti, std::move(schedules[ti]), sms, aux, tmax, trace));
+
+    alloc_model_and_host_buffers(tmax);
+    if (opt.rng == PM_RNG_TABLE) upload_replay_table();
+    mt.reseed((uint32_t)opt.seed);
+    trace.mark("pinned buffers, replay table");
+    // shared-memory sizes
+    const int np_fast = exact ? 0 : ((NS == 2 || NS == 4) ? std::min(PM_SMEM_POW, jcap) : 0);
+    smem_prune = ((size_t)n * n + (size_t)np_fast * n * n) * sizeof(Real);
+    smem_nodes = ((size_t)n * n + 3 * n + (size_t)np_fast * n * n) * sizeof(Real);
+    smem_paths = (size_t)4 * n * sizeof(double) + ((size_t)n * n + ((n * n) & 1)) * sizeof(unsigned) +
+                 ((size_t)2 * n * n + 5 * n + (size_t)np_fast * n * n) * sizeof(Real);
+
+    for (int ti = 0; ti < ntr; ti++) {
+      TreeDev<Real>& t = *trees[ti];
+      fill_params(t, ti);
+      // (the jump-count / shape words of every branch-site -- 15 GB of writes at the benchmark size -- do not depend on the
+      // tip states, which are still on their way on the second stream)
+      const pm::ChainParams<Real>& P = t.P;
+      if (!V.exp && !V.llonly)
+        pm::k_init_meta<Real><<<dim3((unsigned)((t.S + 255) / 256), (unsigned)std::min(P.E, 65535)), 256, 0, stream>>>(P.maps_off, P.maps_len, t.S, P.E, P.meta,
+                                                                                                                         P.e_len, exact ? nullptr : P.shape);
+      trace.mark("set-up kernels issued");
+      CK(cudaGetLastError());
+    }
+    CK(cudaEventRecord(ev_b, aux));          // join: the tip states of every tree are in place
+    CK(cudaStreamWaitEvent(stream, ev_b, 0));
+    stage_model(true);
+    if (V.exp) {
+      std::vector<double> eg;
+      eg.insert(eg.end(), eig_L.begin(), eig_L.end());
+      eg.insert(eg.end(), eig_R.begin(), eig_R.end());
+      eg.insert(eg.end(), eig_d.begin(), eig_d.end());
+      upload(eig_dev, eg, stream);
+      TreeDev<Real>& t = *trees[0];
+      const int E = t.sch.E;
+      const double* g = eig_dev.as<double>();
+      pm::k_transprob_eig<Real><<<(E + 127) / 128, 128, 0, stream>>>(g, g + (size_t)n * n, g + (size_t)2 * n * n,
+                                                                    t.e_len_d.template as<double>(), E, n, t.TP.template as<Real>());
+      CK(cudaGetLastError());
+    }
+    check_device_errors();
+    for (auto& t : trees) t->tip_stage.alloc(0);   // (everything is on the device now)
+    trace.mark("tip states: H2D + transpose, init kernels, sync");
+  }
+
+  // The checks of the arguments and the trees that need no device (malformed input is reported as PM_ERR_ARG even where
+  // no device exists); sets the chain's shape and returns the trees' schedules.
+  std::vector<pm::host::Schedule> validate(int variant, const pm_tree* tr, const double* pid_, const double* prior_, int nprior) {
+    const int ntr = ntrees;
     if (n < 2 || n > PM_NMAX) fail(PM_ERR_ARG, "number of states must be in 2..%d", PM_NMAX);
     if (!V.multi && ntr != 1) fail(PM_ERR_ARG, "this sampler takes exactly one tree");
     if (ntr < 1) fail(PM_ERR_ARG, "no trees");
-    if (Ntot < 0) fail(PM_ERR_ARG, "N must be non-negative");
+    if (N_total < 0) fail(PM_ERR_ARG, "N must be non-negative");
     if (V.hidden && (n < 4 || (n & 1))) fail(PM_ERR_ARG, "hidden-rate samplers need an even number of states >= 4");
     if (V.two_state && n != 2) fail(PM_ERR_ARG, "this sampler is 2-state only");
     if (V.dic && n > PM_DIC_NMAX) fail(PM_ERR_ARG, "the DIC samplers support at most %d states", PM_DIC_NMAX);
@@ -655,8 +1010,7 @@ struct ChainT : pm_chain {
     WR = W + 1;
     ncols = ncols_of(variant, n);
 
-    // host-only validation of the trees first: malformed input is reported as PM_ERR_ARG even where no device exists
-    if (!(Om > 0)) fail(PM_ERR_ARG, "Omega must be positive");
+    if (!(Omega > 0)) fail(PM_ERR_ARG, "Omega must be positive");
     std::vector<pm::host::Schedule> schedules(ntr);
     for (int ti = 0; ti < ntr; ti++) {
       const pm_tree& x = tr[ti];
@@ -679,384 +1033,206 @@ struct ChainT : pm_chain {
         }
       }
     }
+    return schedules;
+  }
 
-    mark("validation + schedules");
-    const auto mark_dev = [&] { mark("device queries + stream"); };
+  // Selects and checks the device, sets up the chain's stream; returns the number of SMs.
+  int open_device() {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) fail(PM_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
     if (opt.device < 0 || opt.device >= ndev) fail(PM_ERR_CUDA, "device %d not present", opt.device);
     CK(cudaSetDevice(opt.device));
     // (three attributes, not cudaGetDeviceProperties: that call reads every property of the device and takes 10-150 ms,
     // a quarter of a short call)
-    struct { int major = 0, minor = 0, multiProcessorCount = 0; } prop;
-    CK(cudaDeviceGetAttribute(&prop.major, cudaDevAttrComputeCapabilityMajor, opt.device));
-    CK(cudaDeviceGetAttribute(&prop.minor, cudaDevAttrComputeCapabilityMinor, opt.device));
-    CK(cudaDeviceGetAttribute(&prop.multiProcessorCount, cudaDevAttrMultiProcessorCount, opt.device));
-    if (prop.major != 10) fail(PM_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", opt.device, prop.major, prop.minor);
+    int major = 0, minor = 0, sms = 0;
+    CK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, opt.device));
+    CK(cudaDeviceGetAttribute(&minor, cudaDevAttrComputeCapabilityMinor, opt.device));
+    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, opt.device));
+    if (major != 10) fail(PM_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", opt.device, major, minor);
     if (opt.cuda_stream) stream = (cudaStream_t)opt.cuda_stream;
     else { CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking)); own_stream = true; }
+    return sms;
+  }
 
-    mark_dev();
-    err_flag.alloc(sizeof(unsigned));
-    CK(cudaMemsetAsync(err_flag.p, 0, err_flag.bytes, stream));
-    // a second stream for the upload of the tip states (the largest transfer of create()): everything else -- schedule
-    // uploads, the set-up kernels -- goes on `stream` meanwhile; the two are joined before create() returns
-    cudaStream_t aux = nullptr;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
-    struct AuxGuard {
-      cudaStream_t& s; cudaEvent_t& a; cudaEvent_t& b;
-      ~AuxGuard() { if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } if (a) cudaEventDestroy(a); if (b) cudaEventDestroy(b); }
-    } aux_guard{aux, ev_a, ev_b};
-    CK(cudaStreamCreateWithFlags(&aux, cudaStreamNonBlocking));
-    CK(cudaEventCreateWithFlags(&ev_a, cudaEventDisableTiming));
-    CK(cudaEventCreateWithFlags(&ev_b, cudaEventDisableTiming));
-    CK(cudaEventRecord(ev_a, stream));   // (the error flag is zeroed on `stream`)
-    CK(cudaStreamWaitEvent(aux, ev_a, 0));
-    const int T0 = tr[0].n_tips, E0 = tr[0].n_edges;
-    double tmax = 0, qmax = 0;
-    for (int s = 0; s < n; s++) qmax = std::max(qmax, -Q[s + (size_t)s * n]);
-
-    for (int ti = 0; ti < ntr; ti++) {
-      const pm_tree& x = tr[ti];
-      std::unique_ptr<TreeDev<Real>> t(new TreeDev<Real>());
-      t->sch = std::move(schedules[ti]);
-      t->S = x.n_sites;
-      t->TS = (t->S + 15) / 16 * 16;  // tip-code rows are padded: every row starts 16-byte aligned whatever S is
-      const int E = x.n_edges, T = x.n_tips;
-      // The tip states start their way over PCIe FIRST: [S][T] rows staged in blocks and transposed to [T][S] on the
-      // device, all asynchronous on the second stream, so that the host work below (record capacities, schedules) and the set-up kernels run
-      // while they travel.  (The staging buffer is kept until the end of create(): the pool must not hand it out again.)
-      {
-        t->tipcode.alloc((size_t)T * t->TS);
-        CK(cudaMemsetAsync(t->tipcode.p, 0, t->tipcode.bytes, aux));
-        t->node_state.alloc((size_t)(2 * T - 1) * t->S);
-        CK(cudaMemsetAsync(t->node_state.p, 0, t->node_state.bytes, aux));
-        const size_t esz = x.states_u8 ? 1 : 4;
-        long long rows_per = std::max<long long>(32, (256LL << 20) / ((long long)T * (long long)esz));
-        rows_per = std::min<long long>(rows_per, std::min<long long>(t->S, 32LL * 65535));
-        t->tip_stage.alloc((size_t)rows_per * T * esz);
-        for (long long s0 = 0; s0 < t->S; s0 += rows_per) {
-          const int ns = (int)std::min<long long>(rows_per, t->S - s0);
-          const void* src = x.states_u8 ? (const void*)(x.states_u8 + s0 * T) : (const void*)(x.states + s0 * T);
-          CK(cudaMemcpyAsync(t->tip_stage.p, src, (size_t)ns * T * esz, cudaMemcpyHostToDevice, aux));
-          dim3 g((T + 31) / 32, (ns + 31) / 32), b(32, 8);
-          if (x.states_u8)
-            pm::k_init_tips<uint8_t><<<g, b, 0, aux>>>(t->tip_stage.template as<uint8_t>(), ns, s0, t->S, t->TS, T, n, V.parity_tips,
-                                                          t->tipcode.template as<uint8_t>(), t->node_state.template as<uint8_t>(), err_flag.as<unsigned>());
-          else
-            pm::k_init_tips<int32_t><<<g, b, 0, aux>>>(t->tip_stage.template as<int32_t>(), ns, s0, t->S, t->TS, T, n, V.parity_tips,
-                                                          t->tipcode.template as<uint8_t>(), t->node_state.template as<uint8_t>(), err_flag.as<unsigned>());
-        }
-        CK(cudaGetLastError());
-      }
-      std::vector<long long> moff(E + 1);
-      std::vector<Real> elen(E);
-      for (int e = 0; e <= E; e++) moff[e] = x.maps_off[e];
-      for (int e = 0; e < E; e++) {
-        double tot = 0;
-        for (long long p = moff[e]; p < moff[e + 1]; p++) tot = tot + x.maps_len[p];
-        elen[e] = (Real)tot;
-        tmax = std::max(tmax, tot);
-      }
-      std::vector<double> mlen(x.maps_len, x.maps_len + moff[E]);
-      const long long S = t->S;
-      // launch geometry of the path kernel: a thread owns one site x one chunk of consecutive branches
-      const long long gx = (S + 127) / 128;
-      long long ny = (148LL * 16 * 6 + gx - 1) / gx;
-      ny = std::max(1LL, std::min<long long>(ny, (E + 15) / 16));
-      ny = std::min<long long>(ny, 65535);
-      ny = std::max<long long>(ny, (E + 2047) / 2048);  // the easy path kernel stages a chunk's topology in shared memory
-      ny = std::max<long long>(ny, (E + ((1LL << 32) - 1) / S - 1) / std::max<long long>(1, ((1LL << 32) - 1) / S));  // ... and indexes the rows of a chunk with 32 bits: chunk x S < 2^32
-      // (production: the offset of a path's records inside its slice is a 16-bit field of the state word, so a chunk
-      // whose slice would be longer is split).  Production slices are shared by groups of 32 consecutive sites: the
-      // bound on the records of 32 independent sites together is far tighter, relative to its mean, than 32 bounds on
-      // one site each (3.8 -> 0.3 bytes per branch-site at the benchmark's size).  Where such a slice would not fit the
-      // 16-bit offset (long paths: the Squamate vignette) every site keeps its own.
-      // One block per site, state in shared memory (pm_small.cuh), when the sites are few and the tree fits: production
-      // arithmetic, 2 / 4 states.  PHYLOMAP_B200_SMALL=0 keeps the 32-sites-per-warp kernels (same rows: the tests compare),
-      // PHYLOMAP_B200_SMALL_SITES moves the site limit (default: four blocks per SM).
-      {
-        long long small_sites = 16LL * prop.multiProcessorCount;   // (hard cap; the cost rule below decides before it)
-        const bool sites_forced = getenv("PHYLOMAP_B200_SMALL_SITES") != nullptr;
-        if (sites_forced) small_sites = atoll(getenv("PHYLOMAP_B200_SMALL_SITES"));
-        const bool off = getenv("PHYLOMAP_B200_SMALL") && getenv("PHYLOMAP_B200_SMALL")[0] == '0';
-        const size_t need = NS == 2 ? pm::Sweep<Real, 2, false>::small_smem(T) : NS == 4 ? pm::Sweep<Real, 4, false>::small_smem(T) : (size_t)-1;
-        // ... and the paths of one site are short: a block walks its site's branches with 256 threads, one branch per thread
-        // at a time, while the wide kernels spread the branch-sites of a long-path problem (the Squamate vignette: 877 000
-        // jump points per site and sweep) over the whole device.  What costs is the general item routine: hard = the sum
-        // over the branches of P(two or more jump points) x (2 + expected jump points), jump points ~ Poisson(Omega t).
-        // Measured (scripts/small_calib.py, us per sweep, one character): this kernel ~ 20 + 0.05 hard + 0.03 T, the wide
-        // ones ~ 65 + 0.13 T: it pays up to hard ~ 1500 + 0.7 T.  PHYLOMAP_B200_SMALL_WORK scales that limit.
-        double hard = 0;
-        for (int e = 0; e < E; e++) {
-          const double lam = Omega * (double)elen[e];
-          hard += (1.0 - std::exp(-lam) * (1.0 + lam)) * (2.0 + lam);
-        }
-        double small_work = 1.0;
-        if (const char* v = getenv("PHYLOMAP_B200_SMALL_WORK")) small_work = atof(v);
-        const double work = hard, work_limit = small_work * (1500.0 + 0.7 * T);
-        t->small_two = S > prop.multiProcessorCount;
-        // More sites than SMs: two blocks per SM, waves of 2 x SMs sites; measured (profiles/r2_warp_per_site_attempt.log,
-        // 100-800 tips, 296-2368 sites) a wave takes ~ 10 + 0.28 T + 0.05 hard us and the wide kernels ~ 160 + 0.09 T + 0.01 S.
-        bool sites_ok = S <= small_sites;
-        if (t->small_two && !sites_forced) {
-          const double waves = std::ceil((double)S / (2.0 * prop.multiProcessorCount));
-          sites_ok = sites_ok && waves * (10.0 + 0.28 * T + 0.05 * hard) < 160.0 + 0.09 * T + 0.01 * (double)S;
-        }
-        t->small_ok = !off && !exact && (NS == 2 || NS == 4) && !V.exp && !V.llonly && opt.rng != PM_RNG_TABLE && sites_ok &&
-                      need <= (size_t)200 * 1024 && work <= work_limit;
-      }
-      const bool pooled_ok = !t->small_ok && !exact && !V.exp && !V.llonly && !(getenv("PHYLOMAP_B200_REC_POOL") && getenv("PHYLOMAP_B200_REC_POOL")[0] == '0');
-      const long long ny_first = ny;
-      for (int attempt = pooled_ok ? 0 : 1; attempt < 2; attempt++) {
-      t->rec_shift = attempt == 0 ? 5 : 0;
-      const double G = (double)(1 << t->rec_shift);
-      t->rec_groups = (S + (1LL << t->rec_shift) - 1) >> t->rec_shift;
-      ny = ny_first;
-      bool fits = true;
-      for (;;) {
-      t->chunk = (int)((E + ny - 1) / ny);
-      ny = (E + t->chunk - 1) / t->chunk;
-      t->paths_grid = dim3((unsigned)gx, (unsigned)ny, 1);
-      t->nblocks = gx * ny;
-      long long cap_max = 0;
-      // record capacity of every chunk.  Real jumps sit on uniformization points, and in equilibrium the points of a
-      // chunk are Poisson(Omega x total length), so the Poisson tail bounds them; a path with j real jumps stores
-      // j + 1 runs (<= 2j).  The first sweep instead finds its points in the caller's maps (m_e - 1 per branch), so
-      // the initial segmentation is a second lower bound.
-      t->cap_off_h.assign(ny + 1, 0);
-      for (long long c = 0; c < ny; c++) {
-        const int b0 = (int)c * t->chunk, b1 = std::min(E, b0 + t->chunk);
-        double len = 0;
-        long long init_records = 0;
-        for (int e = b0; e < b1; e++) {
-          len += (double)elen[e];
-          const long long m0 = moff[e + 1] - moff[e];
-          if (exact || m0 >= 2) init_records += m0;
-        }
-        long long cap;
-        if (V.exp || V.llonly) cap = 4;  // no path state
-        else if (opt.path_capacity > 0) cap = (long long)opt.path_capacity * (b1 - b0) * (long long)G;
-        else if (exact) {
-          const int jumps = poisson_cap(1.5 * Omega * len + 1.0, 1e-18);
-          cap = std::max<long long>((long long)(b1 - b0) + jumps, init_records);
-        } else {
-          // production: only paths with >= 2 real jumps keep records (j + 1 of them); Chernoff bound on their sum
-          // over the chunk with every branch's jump count dominated by Poisson(1.5 Omega t)
-          std::vector<double> lams;
-          long long init3 = 0;
-          for (int e = b0; e < b1; e++) {
-            lams.push_back(1.5 * Omega * (double)elen[e]);
-            const long long m0 = moff[e + 1] - moff[e];
-            if (m0 >= 3) init3 += m0;
-          }
-          // ... or, simpler and valid for any rate: every path stores at most (jumps + 1) records (+ a header), and the
-          // jumps of the chunk together are dominated by one Poisson variable
-          double lam_sum = 0, lam_max = 0;
-          for (double l : lams) { lam_sum += l; lam_max = std::max(lam_max, l); }
-          const long long simple = (long long)poisson_cap(G * lam_sum, 1e-18) + 2LL * (b1 - b0) * (long long)G;
-          long long stat = simple;
-          if (lam_max < 200.0) stat = std::min(stat, chernoff_records_cap(lams, 1e-18, G));  // (its series stops at 400 terms)
-          cap = std::max<long long>(stat, init3 * (long long)G) + 4;
-        }
-        if (cap > (1 << 28)) { if (t->rec_shift) cap = 1 << 28; else fail(PM_ERR_CAPACITY, "path capacity of a branch chunk too large"); }
-        cap = (cap + 3) & ~3;  // keep every slice 16-byte aligned
-        cap_max = std::max(cap_max, cap);
-        t->cap_off_h[c + 1] = t->cap_off_h[c] + (int)cap;
-      }
-      if (exact || V.exp || V.llonly || cap_max <= 65535) break;
-      if (t->rec_shift) { fits = false; break; }  // shared slices too long for the offset field: per-site slices instead
-      if (t->chunk <= 1 || ny >= 65535) fail(PM_ERR_CAPACITY, "a branch needs more than 65 535 path records per site");
-      ny = std::min<long long>(std::min<long long>(2 * ny, E), 65535);
-      }
-      if (fits) break;
-      }
-      const long long R = t->cap_off_h[ny];
-      t->small_chunks = (int)ny;
-      mark("record capacities");
-      // Partials are scratch between the pruning pass and the node draws of one sweep, and a block's partials are read by
-      // nobody but the same block's node draws: the production kernels (n = 2, 4) run both passes in ONE kernel whose
-      // blocks keep their partials in a slot of 32 sites, claimed for the life of the block (k_prune_nodes_clade): as many
-      // slots per SM as blocks can be resident there (3 in FP32, 2 in FP64: the occupancy the runtime reports for the
-      // smallest shared-memory configuration, an upper bound).  The DIC chains evaluate log p(y | Q) over all sites after
-      // the sweep and keep the whole array, like the generic and the deterministic kernels.
-      // PHYLOMAP_B200_FUSED=0: the two separate kernels and the full array (for comparison).
-      t->pl_slots = 0;
-      t->pl_sites = S;
-      if (!exact && (NS == 2 || NS == 4) && !V.dic && !V.exp && !V.llonly && !(getenv("PHYLOMAP_B200_FUSED") && getenv("PHYLOMAP_B200_FUSED")[0] == '0')) {
-        const size_t smem_lo = ((size_t)n * n + 3 * n) * sizeof(Real);
-        const int per_sm = NS == 2 ? pm::Sweep<Real, 2, false>::fused_blocks_per_sm(smem_lo) : pm::Sweep<Real, 4, false>::fused_blocks_per_sm(smem_lo);
-        if (per_sm < 1) fail(PM_ERR_CUDA, "cudaOccupancyMaxActiveBlocksPerMultiprocessor failed for the fused prune + node-draw kernel");
-        t->slots_per_sm = per_sm;
-        t->pl_slots = sm_id_range(opt.device, prop.multiProcessorCount) * per_sm;  // slots are indexed by %smid
-        t->pl_sites = 32LL * t->pl_slots;
-        if (t->pl_sites >= ((S + 31) / 32) * 32) {  // fewer site blocks than slots: block i uses slot i
-          t->pl_slots = (int)((S + 31) / 32); t->pl_sites = 32LL * t->pl_slots; t->slots_per_sm = 0;
-        } else {
-          t->slot_busy.alloc((size_t)t->pl_slots * sizeof(int));
-          CK(cudaMemsetAsync(t->slot_busy.p, 0, t->slot_busy.bytes, stream));
-        }
-      }
-      upload(t->up_entries, t->sch.up_entries, stream);
-      upload(t->up_off, t->sch.up_off, stream);
-      if (!exact && (NS == 2 || NS == 4)) {
-        // clades of ~1/64 of the tree: ~8 per warp to balance, and only ~100 nodes left above them.  Small trees (where a
-        // sweep is a matter of latency, not throughput): ~1/8 of the tree, so that almost every node is walked inside a
-        // warp's prefetched sequence and only a few levels with block barriers are left above.  (A function of the tree
-        // alone: the node draws are keyed by schedule position, and a site must not depend on how many others run.)
-        const int clade_max = (T - 1 < 512) ? std::max(8, (T - 1) / 8) : std::max(8, std::min(512, (T - 1) / 64));
-        pm::host::CladeSchedule cs;
-        pm::host::build_clade_schedule(t->sch, 8, clade_max, cs);
-        // phase-1 entries as byte offsets (PM_CLADE_ENTRY_INTS ints each): the kernel only adds them to per-lane bases
-        const int n1 = cs.warp_off.back();
-        std::vector<int> e16((size_t)PM_CLADE_ENTRY_INTS * (n1 + 17), 0);  // padded: the kernel forms addresses up to 16 entries ahead
-        auto put64 = [](int* dst, long long v) { dst[0] = (int)(unsigned)(v & 0xffffffffLL); dst[1] = (int)(v >> 32); };
-        const long long rowPL = (long long)t->pl_sites * n * (long long)sizeof(Real);
-        for (int i = 0; i < n1; i++) {
-          const int* en = &cs.entries[(size_t)8 * i];
-          int* o = &e16[(size_t)PM_CLADE_ENTRY_INTS * i];
-          const int pn = en[0], a = en[1], ea = en[2], b = en[3], eb = en[4];
-          int fl = en[5] & 3;
-          const int x = (en[5] & 4) ? a : (en[5] & 8) ? b : -1;
-          if (a < T) fl |= 16;
-          if (b < T) fl |= 32;
-          put64(o + 0, (long long)(pn - T) * rowPL);
-          put64(o + 2, x >= 0 ? (long long)(x - T) * rowPL : -1LL);
-          put64(o + 4, (long long)ea * S * 4);
-          put64(o + 6, (long long)eb * S * 4);
-          put64(o + 8, a < T ? (long long)a * t->TS : -1LL);
-          put64(o + 10, b < T ? (long long)b * t->TS : -1LL);
-          o[12] = fl;
-        }
-        std::vector<int> top(cs.entries.begin() + (size_t)8 * n1, cs.entries.end());
-        for (int& v : cs.top_off) v -= n1;
-        upload(t->cl_entries, e16, stream);
-        upload(t->cl_warp_off, cs.warp_off, stream);
-        upload(t->cl_top_entries, top, stream);
-        upload(t->cl_top_off, cs.top_off, stream);
-        t->n_cl_top_levels = (int)cs.top_off.size() - 1;
-        // the same clades top-down for the node draws (k_nodes_clade): 16 ints per node, byte offsets
-        const int n2 = cs.down_warp_off.back();
-        std::vector<int> d16((size_t)16 * (n2 + 17), 0);
-        for (int i = 0; i < n2; i++) {
-          const int* en = &cs.down_seq[(size_t)4 * i];
-          int* o = &d16[(size_t)16 * i];
-          put64(o + 0, (long long)(en[0] - T) * rowPL);
-          put64(o + 2, (long long)en[2] * S * 4);
-          put64(o + 4, (long long)en[0] * S);
-          put64(o + 6, en[3] ? -1LL : (long long)en[1] * S);
-        }
-        upload(t->cd_entries, d16, stream);
-        upload(t->cd_warp_off, cs.down_warp_off, stream);
-        upload(t->cd_top, cs.down_top, stream);
-        upload(t->cd_top_off, cs.down_top_off, stream);
-        t->n_cd_top_levels = (int)cs.down_top_off.size() - 1;
-        std::vector<long long> tips;  // entry v = tip v: the parent's node-state row, the jump-count row of its branch (bytes)
-        if (V.redraw_tips)
-          for (int v = 0; v < T; v++) {
-            const int e = t->sch.parent_edge[v];
-            tips.push_back((long long)t->sch.e_parent[e] * S); tips.push_back((long long)e * S * 4);
-          }
-        t->n_cd_tips = (int)tips.size() / 2;
-        upload(t->cd_tips, tips, stream);
-        if (t->small_ok) {
-          // the same draws node by node: every drawn node with the Philox block and word the clade kernel gives it
-          // (k_small_chain decodes the key), grouped by depth like the generic schedule
-          std::vector<uint32_t> key(2 * (size_t)T - 1, 0u);
-          for (int i = 0; i < (int)cs.down_top.size() / 4; i++) key[cs.down_top[(size_t)4 * i]] = 0x80000000u | (uint32_t)i;
-          for (int i = 0; i < n2; i++) key[cs.down_seq[(size_t)4 * i]] = (uint32_t)i;
-          for (int v = 0; v < T; v++) key[v] = 0x40000000u | (uint32_t)v;
-          const int nd = (int)t->sch.down_entries.size() / 3;
-          std::vector<int> d4((size_t)4 * std::max(nd, 1), 0);
-          for (int i = 0; i < nd; i++) {
-            const int* en = &t->sch.down_entries[(size_t)3 * i];
-            d4[(size_t)4 * i] = en[0]; d4[(size_t)4 * i + 1] = en[1]; d4[(size_t)4 * i + 2] = en[2]; d4[(size_t)4 * i + 3] = (int)key[en[0]];
-          }
-          upload(t->small_down, d4, stream);
-          // Which thread takes which branch.  A warp runs the general item routine in lockstep: it takes as long as its
-          // longest path, plus a share for every other shape among its items.  Up to 256 branches (one per thread): the
-          // branches sorted by decreasing length are DEALT over the 8 warps, so that every warp gets one of the longest,
-          // one of the next eight, ... (measured on configs[0]: all long branches in one warp 30 300 cycles for the path
-          // phase, edge order 26 000).  Larger trees: decreasing length (warps of similar paths: throughput).
-          std::vector<int> sorted(E);
-          for (int e = 0; e < E; e++) sorted[e] = e;
-          std::stable_sort(sorted.begin(), sorted.end(), [&](int x, int y) { return elen[x] > elen[y]; });
-          std::vector<int> border;
-          if (E <= 256) {
-            border.assign(256, -1);
-            for (int k = 0; k < E; k++) border[(size_t)(k % 8) * 32 + k / 8] = sorted[k];   // warp k % 8, lane k / 8
-          } else border = sorted;
-          t->small_order_n = (int)border.size();
-          upload(t->small_border, border, stream);
-        }
-      }
-      upload(t->down_entries, t->sch.down_entries, stream);
-      upload(t->down_off, t->sch.down_off, stream);
-      upload(t->e_parent, t->sch.e_parent, stream);
-      upload(t->e_child, t->sch.e_child, stream);
-      upload(t->e_len, elen, stream);
-      if (V.dic || V.exp) {
-        std::vector<double> eld(E);
-        for (int e = 0; e < E; e++) eld[e] = x.edge_length ? x.edge_length[e] : (double)elen[e];
-        if (x.edge_length) for (int e = 0; e < E; e++) if (!(eld[e] >= 0)) fail(PM_ERR_ARG, "tree %d: negative or NA edge.length", ti);
-        upload(t->e_len_d, eld, stream);
-        t->TP.alloc((size_t)E * n * n * sizeof(Real));
-        t->ll_partial.alloc((size_t)((S + 31) / 32) * sizeof(double));
-      }
-      mark("clade schedules + uploads");
-      upload(t->maps_off, moff, stream);
-      upload(t->maps_len, mlen, stream);
-      upload(t->cap_off, t->cap_off_h, stream);
-      if (!V.exp && !V.llonly) t->meta.alloc((size_t)E * S * sizeof(uint32_t));
-      t->PL.alloc((size_t)(T - 1) * t->pl_sites * n * sizeof(Real));
-      for (int b = 0; b < 2 && !V.exp && !V.llonly; b++) {
-        t->rec_len[b].alloc((size_t)R * t->rec_groups * sizeof(Real));
-        t->rec_st[b].alloc((size_t)R * t->rec_groups);
-      }
-      if (!exact && !V.exp && !V.llonly) {
-        // Branch-major ballot array and the general kernel's work items: branch e is cut into items of g_e ballot words
-        // (32 g_e sites), g_e chosen so that an item holds ~96 branch-sites with two or more jump points in equilibrium
-        // (their number on a branch of length t is Poisson(Omega t)).
-        const long long Wl = (S + 31) / 32;
-        t->hard_ballot.alloc((size_t)E * Wl * sizeof(uint32_t));
-        std::vector<long long> woff(E + 1, 0);
-        std::vector<int> wg(E);
-        for (int e = 0; e < E; e++) {
-          const double lam = Omega * (double)elen[e];
-          const double h = std::max(1e-6, 1.0 - std::exp(-lam) * (1.0 + lam));
-          long long g = (long long)std::ceil(96.0 / (32.0 * h));
-          g = std::max(1LL, std::min<long long>(std::min<long long>(g, 32), Wl));
-          wg[e] = (int)g;
-          woff[e + 1] = woff[e] + (Wl + g - 1) / g;
-        }
-        t->wk_total = woff[E];
-        std::vector<int> hint((size_t)(t->wk_total >> 6) + 1);
-        for (long long i = 0, e = 0; i < (long long)hint.size(); i++) {
-          while (e + 1 < E && woff[e + 1] <= (i << 6)) e++;
-          hint[i] = (int)e;
-        }
-        upload(t->wk_hint, hint, stream);
-        upload(t->wk_off, woff, stream);
-        upload(t->wk_g, wg, stream);
-        t->wk_item.alloc((size_t)std::max<long long>(t->wk_total, 1) * sizeof(unsigned long long));
-        pm::k_build_items<<<(unsigned)((t->wk_total + 255) / 256), 256, 0, stream>>>(t->wk_off.template as<long long>(), t->wk_g.template as<int>(), E, Wl,
-                                                                                    t->wk_total, t->wk_item.template as<unsigned long long>());
-        t->rec_cursor.alloc((size_t)ny * t->rec_groups * sizeof(int));
-        t->shape.alloc((size_t)E * S * sizeof(uint16_t));
-        // persistent: 4 blocks of 4 warps per SM, fewer when there are not that many work items (a handful of sites)
-        t->hard_blocks = (int)std::max<long long>(1, std::min<long long>(prop.multiProcessorCount * 4LL, (t->wk_total + 3) / 4));
-      }
-      // partial dwell sums per block: [0, nblocks) easy / deterministic / direct-sampler kernel, then the general path kernel's
-      t->dw_rows = t->nblocks + 3 * t->hard_blocks;  // general kernel: hard_blocks rows; short kernel: 2 hard_blocks (after them)
-      t->dw_partial.alloc((size_t)t->dw_rows * n * sizeof(double));
-      CK(cudaMemsetAsync(t->dw_partial.p, 0, t->dw_partial.bytes, stream));
-      dev_bytes += t->tipcode.bytes + t->node_state.bytes + t->meta.bytes + t->PL.bytes + 2 * (t->rec_len[0].bytes + t->rec_st[0].bytes) +
-                   t->dw_partial.bytes + t->hard_ballot.bytes + t->rec_cursor.bytes + t->shape.bytes + t->wk_item.bytes;
-      trees.push_back(std::move(t));
-      mark("device buffers");
+  // One tree's device state: tip upload on `aux` first, then the plan, the schedules and the buffers on `stream`.
+  // tmax: the longest branch so far.
+  std::unique_ptr<TreeDev<Real>> create_tree(const pm_tree& x, int ti, pm::host::Schedule&& sch, int sms, cudaStream_t aux,
+                                             double& tmax, PhaseTrace& trace) {
+    std::unique_ptr<TreeDev<Real>> tp(new TreeDev<Real>());
+    TreeDev<Real>& t = *tp;
+    t.sch = std::move(sch);
+    t.S = x.n_sites;
+    t.TS = (t.S + 15) / 16 * 16;  // tip-code rows are padded: every row starts 16-byte aligned whatever S is
+    const int E = x.n_edges, T = x.n_tips;
+    const long long S = t.S;
+    const bool no_paths = V.exp || V.llonly;  // log-likelihood-only and direct-sampler chains keep no path state
+    upload_tips(t, x, aux);
+    std::vector<long long> moff(x.maps_off, x.maps_off + E + 1);
+    std::vector<Real> elen(E);
+    for (int e = 0; e < E; e++) {
+      double tot = 0;
+      for (long long p = moff[e]; p < moff[e + 1]; p++) tot = tot + x.maps_len[p];
+      elen[e] = (Real)tot;
+      tmax = std::max(tmax, tot);
     }
+    std::vector<double> mlen(x.maps_len, x.maps_len + moff[E]);
 
-    // table of powers
+    const size_t small_smem = with_ns([&](auto ns) { return pm::Sweep<Real, decltype(ns)::value, false>::small_smem(T); });
+    const SmallChoice small = choose_small_kernel(!exact && (NS == 2 || NS == 4) && !no_paths && opt.rng != PM_RNG_TABLE, elen,
+                                                  Omega, T, S, sms, small_smem, sw);
+    t.small_ok = small.ok;
+    t.small_two = small.two;
+    const bool pooled_ok = !t.small_ok && !exact && !no_paths && sw.rec_pool;
+    RecordPlan rp = plan_records(pooled_ok ? 5 : 0, elen, moff, S, Omega, exact, no_paths, opt.path_capacity);
+    if (!rp.fits) rp = plan_records(0, elen, moff, S, Omega, exact, no_paths, opt.path_capacity);
+    t.rec_shift = rp.rec_shift;
+    t.rec_groups = (S + (1LL << t.rec_shift) - 1) >> t.rec_shift;
+    t.chunk = rp.chunk;
+    t.paths_grid = dim3((unsigned)rp.gx, (unsigned)rp.ny, 1);
+    t.nblocks = rp.gx * rp.ny;
+    t.small_chunks = (int)rp.ny;
+    t.cap_off_h = std::move(rp.cap_off);
+    trace.mark("record capacities");
+
+    plan_partials_slots(t, sms);
+    upload(t.up_entries, t.sch.up_entries, stream);
+    upload(t.up_off, t.sch.up_off, stream);
+    if (!exact && (NS == 2 || NS == 4)) {
+      CladeCode cc = encode_clade_schedule(t.sch, S, t.TS, (long long)t.pl_sites * n * (long long)sizeof(Real), V.redraw_tips);
+      upload(t.cl_entries, cc.e16, stream);
+      upload(t.cl_warp_off, cc.cs.warp_off, stream);
+      upload(t.cl_top_entries, cc.top, stream);
+      upload(t.cl_top_off, cc.cs.top_off, stream);
+      upload(t.cd_entries, cc.d16, stream);
+      upload(t.cd_warp_off, cc.cs.down_warp_off, stream);
+      upload(t.cd_top, cc.cs.down_top, stream);
+      upload(t.cd_top_off, cc.cs.down_top_off, stream);
+      upload(t.cd_tips, cc.tips, stream);
+      t.P.n_cl_top_levels = (int)cc.cs.top_off.size() - 1;
+      t.P.n_cd_top_levels = (int)cc.cs.down_top_off.size() - 1;
+      t.P.n_cd_tips = (int)cc.tips.size() / 2;
+      if (t.small_ok) {
+        const SmallOrder so = small_draw_order(t.sch, cc.cs, elen);
+        upload(t.small_down, so.down, stream);
+        upload(t.small_border, so.border, stream);
+        t.small_order_n = (int)so.border.size();
+      }
+    }
+    upload(t.down_entries, t.sch.down_entries, stream);
+    upload(t.down_off, t.sch.down_off, stream);
+    upload(t.e_parent, t.sch.e_parent, stream);
+    upload(t.e_child, t.sch.e_child, stream);
+    upload(t.e_len, elen, stream);
+    if (V.dic || V.exp) {
+      std::vector<double> eld(E);
+      for (int e = 0; e < E; e++) eld[e] = x.edge_length ? x.edge_length[e] : (double)elen[e];
+      if (x.edge_length) for (int e = 0; e < E; e++) if (!(eld[e] >= 0)) fail(PM_ERR_ARG, "tree %d: negative or NA edge.length", ti);
+      upload(t.e_len_d, eld, stream);
+      t.TP.alloc((size_t)E * n * n * sizeof(Real));
+      t.ll_partial.alloc((size_t)((S + 31) / 32) * sizeof(double));
+    }
+    trace.mark("clade schedules + uploads");
+    alloc_path_state(t, moff, mlen, elen, sms);
+    trace.mark("device buffers");
+    return tp;
+  }
+
+  // The tip states start their way over PCIe FIRST: [S][T] rows staged in blocks and transposed to [T][S] on the device,
+  // all asynchronous on the second stream, so that the host work of create() (record capacities, schedules) and the
+  // set-up kernels run while they travel.  (The staging buffer is kept until the end of create(): the pool must not hand
+  // it out again.)
+  void upload_tips(TreeDev<Real>& t, const pm_tree& x, cudaStream_t aux) {
+    const int T = x.n_tips;
+    t.tipcode.alloc((size_t)T * t.TS);
+    CK(cudaMemsetAsync(t.tipcode.p, 0, t.tipcode.bytes, aux));
+    t.node_state.alloc((size_t)(2 * T - 1) * t.S);
+    CK(cudaMemsetAsync(t.node_state.p, 0, t.node_state.bytes, aux));
+    const size_t esz = x.states_u8 ? 1 : 4;
+    long long rows_per = std::max<long long>(32, (256LL << 20) / ((long long)T * (long long)esz));
+    rows_per = std::min<long long>(rows_per, std::min<long long>(t.S, 32LL * 65535));
+    t.tip_stage.alloc((size_t)rows_per * T * esz);
+    for (long long s0 = 0; s0 < t.S; s0 += rows_per) {
+      const int ns = (int)std::min<long long>(rows_per, t.S - s0);
+      const void* src = x.states_u8 ? (const void*)(x.states_u8 + s0 * T) : (const void*)(x.states + s0 * T);
+      CK(cudaMemcpyAsync(t.tip_stage.p, src, (size_t)ns * T * esz, cudaMemcpyHostToDevice, aux));
+      dim3 g((T + 31) / 32, (ns + 31) / 32), b(32, 8);
+      if (x.states_u8)
+        pm::k_init_tips<uint8_t><<<g, b, 0, aux>>>(t.tip_stage.template as<uint8_t>(), ns, s0, t.S, t.TS, T, n, V.parity_tips,
+                                                     t.tipcode.template as<uint8_t>(), t.node_state.template as<uint8_t>(), err_flag.as<unsigned>());
+      else
+        pm::k_init_tips<int32_t><<<g, b, 0, aux>>>(t.tip_stage.template as<int32_t>(), ns, s0, t.S, t.TS, T, n, V.parity_tips,
+                                                     t.tipcode.template as<uint8_t>(), t.node_state.template as<uint8_t>(), err_flag.as<unsigned>());
+    }
+    CK(cudaGetLastError());
+  }
+
+  // Partials are scratch between the pruning pass and the node draws of one sweep, and a block's partials are read by
+  // nobody but the same block's node draws: the production kernels (n = 2, 4) run both passes in ONE kernel whose
+  // blocks keep their partials in a slot of 32 sites, claimed for the life of the block (k_prune_nodes_clade): as many
+  // slots per SM as blocks can be resident there (3 in FP32, 2 in FP64: the occupancy the runtime reports for the
+  // smallest shared-memory configuration, an upper bound).  The DIC chains evaluate log p(y | Q) over all sites after
+  // the sweep and keep the whole array, like the generic and the deterministic kernels.
+  // PHYLOMAP_B200_FUSED=0: the two separate kernels and the full array (for comparison).
+  void plan_partials_slots(TreeDev<Real>& t, int sms) {
+    t.pl_slots = 0;
+    t.pl_sites = t.S;
+    if (exact || !(NS == 2 || NS == 4) || V.dic || V.exp || V.llonly || !sw.fused) return;
+    const size_t smem_lo = ((size_t)n * n + 3 * n) * sizeof(Real);
+    const int per_sm = with_ns([&](auto ns) { return pm::Sweep<Real, decltype(ns)::value, false>::fused_blocks_per_sm(smem_lo); });
+    if (per_sm < 1) fail(PM_ERR_CUDA, "cudaOccupancyMaxActiveBlocksPerMultiprocessor failed for the fused prune + node-draw kernel");
+    t.slots_per_sm = per_sm;
+    t.pl_slots = sm_id_range(opt.device, sms) * per_sm;  // slots are indexed by %smid
+    t.pl_sites = 32LL * t.pl_slots;
+    if (t.pl_sites >= ((t.S + 31) / 32) * 32) {  // fewer site blocks than slots: block i uses slot i
+      t.pl_slots = (int)((t.S + 31) / 32); t.pl_sites = 32LL * t.pl_slots; t.slots_per_sm = 0;
+    } else {
+      t.slot_busy.alloc((size_t)t.pl_slots * sizeof(int));
+      CK(cudaMemsetAsync(t.slot_busy.p, 0, t.slot_busy.bytes, stream));
+    }
+  }
+
+  // The per-site state of the sweeps: piece counts, partials, path records, the general path kernel's work items and
+  // the per-block partial sums.
+  void alloc_path_state(TreeDev<Real>& t, const std::vector<long long>& moff, const std::vector<double>& mlen,
+                        const std::vector<Real>& elen, int sms) {
+    const int E = t.sch.E, T = t.sch.T;
+    const long long S = t.S, R = t.cap_off_h.back();
+    const bool no_paths = V.exp || V.llonly;
+    upload(t.maps_off, moff, stream);
+    upload(t.maps_len, mlen, stream);
+    upload(t.cap_off, t.cap_off_h, stream);
+    if (!no_paths) t.meta.alloc((size_t)E * S * sizeof(uint32_t));
+    t.PL.alloc((size_t)(T - 1) * t.pl_sites * n * sizeof(Real));
+    for (int b = 0; b < 2 && !no_paths; b++) {
+      t.rec_len[b].alloc((size_t)R * t.rec_groups * sizeof(Real));
+      t.rec_st[b].alloc((size_t)R * t.rec_groups);
+    }
+    if (!exact && !no_paths) {
+      const long long Wl = (S + 31) / 32;
+      t.hard_ballot.alloc((size_t)E * Wl * sizeof(uint32_t));
+      const WorkItems w = build_work_items(elen, Omega, S);
+      t.wk_total = w.off.back();
+      upload(t.wk_hint, w.hint, stream);
+      upload(t.wk_off, w.off, stream);
+      upload(t.wk_g, w.g, stream);
+      t.wk_item.alloc((size_t)std::max<long long>(t.wk_total, 1) * sizeof(unsigned long long));
+      pm::k_build_items<<<(unsigned)((t.wk_total + 255) / 256), 256, 0, stream>>>(t.wk_off.template as<long long>(), t.wk_g.template as<int>(), E, Wl,
+                                                                                 t.wk_total, t.wk_item.template as<unsigned long long>());
+      t.rec_cursor.alloc((size_t)t.small_chunks * t.rec_groups * sizeof(int));
+      t.shape.alloc((size_t)E * S * sizeof(uint16_t));
+      // persistent: 4 blocks of 4 warps per SM, fewer when there are not that many work items (a handful of sites)
+      t.hard_blocks = (int)std::max<long long>(1, std::min<long long>(sms * 4LL, (t.wk_total + 3) / 4));
+    }
+    // partial dwell sums per block: [0, nblocks) easy / deterministic / direct-sampler kernel, then the general path kernel's
+    t.dw_rows = t.nblocks + 3 * t.hard_blocks;  // general kernel: hard_blocks rows; short kernel: 2 hard_blocks (after them)
+    t.dw_partial.alloc((size_t)t.dw_rows * n * sizeof(double));
+    CK(cudaMemsetAsync(t.dw_partial.p, 0, t.dw_partial.bytes, stream));
+    dev_bytes += t.tipcode.bytes + t.node_state.bytes + t.meta.bytes + t.PL.bytes + 2 * (t.rec_len[0].bytes + t.rec_st[0].bytes) +
+                 t.dw_partial.bytes + t.hard_ballot.bytes + t.rec_cursor.bytes + t.shape.bytes + t.wk_item.bytes;
+  }
+
+  // The model buffer with the table of powers, the pinned host buffers and the chain's small device buffers.
+  void alloc_model_and_host_buffers(double tmax) {
     jcap = opt.power_capacity > 0 ? opt.power_capacity : 64;
     if (V.exp) jcap = 302;  // newunifSample looks at up to 300 jumps (:120)
     else if (opt.power_capacity <= 0) {
@@ -1076,108 +1252,69 @@ struct ChainT : pm_chain {
     ctl.alloc(2 * sizeof(uint32_t));
     phase_ns.alloc(2 * sizeof(unsigned long long));
     CK(cudaMemsetAsync(phase_ns.p, 0, phase_ns.bytes, stream));
-    if (const char* v = getenv("PHYLOMAP_B200_GRAPH")) graph_mode = atoi(v);
     if (V.dic) { CK(cudaMallocHost((void**)&q_h, (size_t)n * n * sizeof(double))); q_dev.alloc((size_t)n * n * sizeof(double)); }
     cnt.alloc((size_t)n * n * sizeof(unsigned long long));
     root_out.alloc(sizeof(int));
     CK(cudaMemsetAsync(cnt.p, 0, cnt.bytes, stream));
     CK(cudaMemsetAsync(root_out.p, 0, root_out.bytes, stream));
+  }
 
-    // replay table
-    const int T = T0, E = E0;
-    const int spi = (2 * T - 1) + 2 * E;
-    if (opt.rng == PM_RNG_TABLE) {
-      const long long nslots = (long long)ntrees * trees[0]->S * N_total * spi;
-      std::vector<long long> off(nslots + 1);
-      for (long long i = 0; i <= nslots; i++) off[i] = opt.tab_off[i];
-      std::vector<double> u(opt.tab_u, opt.tab_u + off[nslots]);
-      upload(tab_off, off, stream);
-      upload(tab_u, u, stream);
-      if (opt.host_tab) replay.reset(new pm::host::ReplaySource(opt.host_tab, opt.host_tab_n));
-    }
-    mt.reseed((uint32_t)opt.seed);
-    if (const char* v = getenv("PHYLOMAP_B200_DEBUG_SYNC")) debug_sync = v[0] == '1';
+  // slots of the replay table per site and sweep: one per node, two per branch
+  int replay_slots_per_iter() const { return (2 * trees[0]->sch.T - 1) + 2 * trees[0]->sch.E; }
+  void upload_replay_table() {
+    const long long nslots = (long long)ntrees * trees[0]->S * N_total * replay_slots_per_iter();
+    std::vector<long long> off(nslots + 1);
+    for (long long i = 0; i <= nslots; i++) off[i] = opt.tab_off[i];
+    std::vector<double> u(opt.tab_u, opt.tab_u + off[nslots]);
+    upload(tab_off, off, stream);
+    upload(tab_u, u, stream);
+    if (opt.host_tab) replay.reset(new pm::host::ReplaySource(opt.host_tab, opt.host_tab_n));
+  }
 
-    mark("pinned buffers, replay table");
-    // shared-memory sizes
-    const int np_fast = exact ? 0 : ((NS == 2 || NS == 4) ? std::min(PM_SMEM_POW, jcap) : 0);
-    smem_prune = ((size_t)n * n + (size_t)np_fast * n * n) * sizeof(Real);
-    smem_nodes = ((size_t)n * n + 3 * n + (size_t)np_fast * n * n) * sizeof(Real);
-    smem_paths = (size_t)4 * n * sizeof(double) + ((size_t)n * n + ((n * n) & 1)) * sizeof(unsigned) +
-                 ((size_t)2 * n * n + 5 * n + (size_t)np_fast * n * n) * sizeof(Real);
-
-    for (int ti = 0; ti < ntr; ti++) {
-      TreeDev<Real>& t = *trees[ti];
-      const pm_tree& x = tr[ti];
-      pm::ChainParams<Real>& P = t.P;
-      P.n = n; P.T = T; P.E = E; P.S = t.S;
-      P.cap_off = t.cap_off.template as<int>();
-      P.hard_ballot = t.hard_ballot.template as<uint32_t>(); P.W = (int)((t.S + 31) / 32);
-      P.wk_off = t.wk_off.template as<long long>(); P.wk_g = t.wk_g.template as<int>(); P.wk_total = t.wk_total;
-      P.wk_hint = t.wk_hint.template as<int>(); P.wk_item = t.wk_item.template as<unsigned long long>();
-      P.rec_cursor = t.rec_cursor.template as<int>(); P.chunk = t.chunk; P.easy_blocks = t.nblocks;
-      P.shape = t.shape.template as<uint16_t>();
-      P.model = model.as<Real>(); P.ppow = model.as<Real>() + model_stride(); P.jcap = jcap;
-      P.up_entries = t.up_entries.template as<int>(); P.up_off = t.up_off.template as<int>();
-      P.n_up_levels = (int)t.sch.up_off.size() - 1;
-      P.cl_entries = t.cl_entries.template as<int>(); P.cl_warp_off = t.cl_warp_off.template as<int>();
-      P.cl_top_entries = t.cl_top_entries.template as<int>();
-      P.cl_top_off = t.cl_top_off.template as<int>(); P.n_cl_top_levels = t.n_cl_top_levels;
-      P.cd_top = t.cd_top.template as<int>(); P.cd_top_off = t.cd_top_off.template as<int>(); P.n_cd_top_levels = t.n_cd_top_levels;
-      P.cd_entries = t.cd_entries.template as<int>(); P.cd_warp_off = t.cd_warp_off.template as<int>();
-      P.cd_tips = t.cd_tips.template as<long long>(); P.n_cd_tips = t.n_cd_tips;
-      P.down_entries = t.down_entries.template as<int>(); P.down_off = t.down_off.template as<int>();
-      P.n_down_levels = (int)t.sch.down_off.size() - 1;
-      P.e_parent = t.e_parent.template as<int>(); P.e_child = t.e_child.template as<int>();
-      P.e_len = t.e_len.template as<Real>();
-      P.maps_off = t.maps_off.template as<long long>(); P.maps_len = t.maps_len.template as<double>();
-      P.root = t.sch.root;
-      P.tipcode = t.tipcode.template as<uint8_t>(); P.TS = t.TS; P.node_state = t.node_state.template as<uint8_t>();
-      P.meta = t.meta.template as<uint32_t>(); P.PL = t.PL.template as<Real>();
-      P.tile_base = 0; P.pl_S = t.pl_sites; P.rec_shift = t.rec_shift; P.rec_groups = t.rec_groups; P.ctl = nullptr;
-      for (int b = 0; b < 2; b++) { P.rec_len[b] = t.rec_len[b].template as<Real>(); P.rec_st[b] = t.rec_st[b].template as<uint8_t>(); }
-      // per-node rescaling (makePLrcpp_bigtree :525) only rescales the weights of each draw: the production
-      // arithmetic always applies it (FP32 partials underflow after ~40 tips otherwise); the deterministic mode
-      // follows the variant, underflow included.  No floor is applied: structural zeros stay exact.
-      P.normalize = V.normalize || !exact; P.full_counts = V.full_counts; P.parity_tips = V.parity_tips;
-      P.dw_partial = t.dw_partial.template as<double>(); P.cnt = cnt.as<unsigned long long>();
-      P.root_out = root_out.as<int>(); P.err_flag = err_flag.as<unsigned>();
-      const uint64_t key = opt.seed + (uint64_t)ti * 0x9E3779B97F4A7C15ull;
-      P.rng.k0 = (uint32_t)key; P.rng.k1 = (uint32_t)(key >> 32);
-      for (int r = 0; r < 10; r++) { P.rng.rk[2 * r] = P.rng.k0 + (uint32_t)r * 0x9E3779B9u; P.rng.rk[2 * r + 1] = P.rng.k1 + (uint32_t)r * 0xBB67AE85u; }
-      P.rng.site0 = (uint32_t)opt.site_offset;
-      P.rng.tab_off = opt.rng == PM_RNG_TABLE ? (const int64_t*)tab_off.p : nullptr;
-      P.rng.tab_u = opt.rng == PM_RNG_TABLE ? tab_u.as<double>() : nullptr;
-      P.rng.tab_site_stride = (int64_t)N_total * spi;
-      P.rng.tab_base = (int64_t)ti * t.S * N_total * spi;
-      P.rng.slots_per_iter = spi; P.rng.n_nodes = 2 * T - 1;
-
-      // (the jump-count / shape words of every branch-site -- 15 GB of writes at the benchmark size -- do not depend on the
-      // tip states, which are still on their way on the second stream)
-      if (!V.exp && !V.llonly)
-        pm::k_init_meta<Real><<<dim3((unsigned)((t.S + 255) / 256), (unsigned)std::min(E, 65535)), 256, 0, stream>>>(P.maps_off, P.maps_len, t.S, E, P.meta, P.e_len,
-                                                                                                                       exact ? nullptr : P.shape);
-      mark("set-up kernels issued");
-      CK(cudaGetLastError());
-    }
-    CK(cudaEventRecord(ev_b, aux));          // join: the tip states of every tree are in place
-    CK(cudaStreamWaitEvent(stream, ev_b, 0));
-    stage_model(true);
-    if (V.exp) {
-      std::vector<double> eg;
-      eg.insert(eg.end(), eig_L.begin(), eig_L.end());
-      eg.insert(eg.end(), eig_R.begin(), eig_R.end());
-      eg.insert(eg.end(), eig_d.begin(), eig_d.end());
-      upload(eig_dev, eg, stream);
-      TreeDev<Real>& t = *trees[0];
-      const double* g = eig_dev.as<double>();
-      pm::k_transprob_eig<Real><<<(E + 127) / 128, 128, 0, stream>>>(g, g + (size_t)n * n, g + (size_t)2 * n * n,
-                                                                    t.e_len_d.template as<double>(), E, n, t.TP.template as<Real>());
-      CK(cudaGetLastError());
-    }
-    check_device_errors();
-    for (auto& t : trees) t->tip_stage.alloc(0);   // (everything is on the device now)
-    mark("tip states: H2D + transpose, init kernels, sync");
+  // The kernels' view of tree ti.
+  void fill_params(TreeDev<Real>& t, int ti) {
+    pm::ChainParams<Real>& P = t.P;
+    const int T = t.sch.T, E = t.sch.E, spi = replay_slots_per_iter();
+    P.n = n; P.T = T; P.E = E; P.S = t.S;
+    P.cap_off = t.cap_off.template as<int>();
+    P.hard_ballot = t.hard_ballot.template as<uint32_t>(); P.W = (int)((t.S + 31) / 32);
+    P.wk_off = t.wk_off.template as<long long>(); P.wk_g = t.wk_g.template as<int>(); P.wk_total = t.wk_total;
+    P.wk_hint = t.wk_hint.template as<int>(); P.wk_item = t.wk_item.template as<unsigned long long>();
+    P.rec_cursor = t.rec_cursor.template as<int>(); P.chunk = t.chunk; P.easy_blocks = t.nblocks;
+    P.shape = t.shape.template as<uint16_t>();
+    P.model = model.as<Real>(); P.ppow = model.as<Real>() + model_stride(); P.jcap = jcap;
+    P.up_entries = t.up_entries.template as<int>(); P.up_off = t.up_off.template as<int>();
+    P.n_up_levels = (int)t.sch.up_off.size() - 1;
+    P.cl_entries = t.cl_entries.template as<int>(); P.cl_warp_off = t.cl_warp_off.template as<int>();
+    P.cl_top_entries = t.cl_top_entries.template as<int>(); P.cl_top_off = t.cl_top_off.template as<int>();
+    P.cd_top = t.cd_top.template as<int>(); P.cd_top_off = t.cd_top_off.template as<int>();
+    P.cd_entries = t.cd_entries.template as<int>(); P.cd_warp_off = t.cd_warp_off.template as<int>();
+    P.cd_tips = t.cd_tips.template as<long long>();
+    P.down_entries = t.down_entries.template as<int>(); P.down_off = t.down_off.template as<int>();
+    P.n_down_levels = (int)t.sch.down_off.size() - 1;
+    P.e_parent = t.e_parent.template as<int>(); P.e_child = t.e_child.template as<int>();
+    P.e_len = t.e_len.template as<Real>();
+    P.maps_off = t.maps_off.template as<long long>(); P.maps_len = t.maps_len.template as<double>();
+    P.root = t.sch.root;
+    P.tipcode = t.tipcode.template as<uint8_t>(); P.TS = t.TS; P.node_state = t.node_state.template as<uint8_t>();
+    P.meta = t.meta.template as<uint32_t>(); P.PL = t.PL.template as<Real>();
+    P.tile_base = 0; P.pl_S = t.pl_sites; P.rec_shift = t.rec_shift; P.rec_groups = t.rec_groups; P.ctl = nullptr;
+    for (int b = 0; b < 2; b++) { P.rec_len[b] = t.rec_len[b].template as<Real>(); P.rec_st[b] = t.rec_st[b].template as<uint8_t>(); }
+    // per-node rescaling (makePLrcpp_bigtree :525) only rescales the weights of each draw: the production
+    // arithmetic always applies it (FP32 partials underflow after ~40 tips otherwise); the deterministic mode
+    // follows the variant, underflow included.  No floor is applied: structural zeros stay exact.
+    P.normalize = V.normalize || !exact; P.full_counts = V.full_counts; P.parity_tips = V.parity_tips;
+    P.dw_partial = t.dw_partial.template as<double>(); P.cnt = cnt.as<unsigned long long>();
+    P.root_out = root_out.as<int>(); P.err_flag = err_flag.as<unsigned>();
+    const uint64_t key = opt.seed + (uint64_t)ti * 0x9E3779B97F4A7C15ull;
+    P.rng.k0 = (uint32_t)key; P.rng.k1 = (uint32_t)(key >> 32);
+    for (int r = 0; r < 10; r++) { P.rng.rk[2 * r] = P.rng.k0 + (uint32_t)r * 0x9E3779B9u; P.rng.rk[2 * r + 1] = P.rng.k1 + (uint32_t)r * 0xBB67AE85u; }
+    P.rng.site0 = (uint32_t)opt.site_offset;
+    P.rng.tab_off = opt.rng == PM_RNG_TABLE ? (const int64_t*)tab_off.p : nullptr;
+    P.rng.tab_u = opt.rng == PM_RNG_TABLE ? tab_u.as<double>() : nullptr;
+    P.rng.tab_site_stride = (int64_t)N_total * spi;
+    P.rng.tab_base = (int64_t)ti * t.S * N_total * spi;
+    P.rng.slots_per_iter = spi; P.rng.n_nodes = 2 * T - 1;
   }
 
   // sum `count` doubles at device address `buf` over the ranks, in stream order (no-op for a single process)
@@ -1222,22 +1359,19 @@ struct ChainT : pm_chain {
     Real* TP = t.TP.template as<Real>();
     double* llp = t.ll_partial.template as<double>();
     const size_t smem_b = (size_t)4 * n * sizeof(double) + ((size_t)n * n + ((n * n) & 1)) * sizeof(unsigned) + (size_t)n * n * sizeof(Real);
-    begin_timed(0);
-    if (NS == 2) pm::k_loglik<Real, 2><<<gx, 256, 0, stream>>>(t.P, TP, llp);
-    else if (NS == 4) pm::k_loglik<Real, 4><<<gx, 256, 0, stream>>>(t.P, TP, llp);
-    else pm::k_loglik<Real, 0><<<gx, 256, 0, stream>>>(t.P, TP, llp);
-    end_timed();
-    begin_timed(1);
-    if (NS == 2) pm::k_exp_nodes<Real, 2><<<gx, 256, 0, stream>>>(t.P, TP, iter);
-    else if (NS == 4) pm::k_exp_nodes<Real, 4><<<gx, 256, 0, stream>>>(t.P, TP, iter);
-    else pm::k_exp_nodes<Real, 0><<<gx, 256, 0, stream>>>(t.P, TP, iter);
-    end_timed();
-    begin_timed(2);
     const double* el = t.e_len_d.template as<double>();
-    if (NS == 2) pm::k_exp_branches<Real, 2><<<t.paths_grid, 128, smem_b, stream>>>(t.P, TP, el, (Real)Omega, iter, t.chunk);
-    else if (NS == 4) pm::k_exp_branches<Real, 4><<<t.paths_grid, 128, smem_b, stream>>>(t.P, TP, el, (Real)Omega, iter, t.chunk);
-    else pm::k_exp_branches<Real, 0><<<t.paths_grid, 128, smem_b, stream>>>(t.P, TP, el, (Real)Omega, iter, t.chunk);
-    end_timed();
+    with_ns([&](auto ns) {
+      constexpr int NSc = decltype(ns)::value;
+      begin_timed(0);
+      pm::k_loglik<Real, NSc><<<gx, 256, 0, stream>>>(t.P, TP, llp);
+      end_timed();
+      begin_timed(1);
+      pm::k_exp_nodes<Real, NSc><<<gx, 256, 0, stream>>>(t.P, TP, iter);
+      end_timed();
+      begin_timed(2);
+      pm::k_exp_branches<Real, NSc><<<t.paths_grid, 128, smem_b, stream>>>(t.P, TP, el, (Real)Omega, iter, t.chunk);
+      end_timed();
+    });
     begin_timed(3);
     pm::k_reduce<<<1, 256, 0, stream>>>(t.dw_partial.template as<double>(), t.dw_rows, n, cnt.as<unsigned long long>(),
                                         root_out.as<int>(), row, 0, err_flag.as<unsigned>(), W);
@@ -1257,7 +1391,7 @@ struct ChainT : pm_chain {
       // others replay a captured sweep
       const bool small = (double)t.S * t.sch.E <= (double)(1 << 22);
       const bool one_launch = !V.exp && !exact && use_small(t);  // every sweep of the call inside one launch
-      const bool use_graph = !one_launch && !V.exp && !timing && !debug_sync && count > 1 && (graph_mode == 1 || (graph_mode != 0 && small));
+      const bool use_graph = !one_launch && !V.exp && !timing && !sw.debug_sync && count > 1 && (sw.graph == 1 || (sw.graph != 0 && small));
       if (one_launch) launch_small(t, (uint32_t)iters_done, count, rows.as<double>());
       for (int i = 0; i < count && !one_launch; i++) {
         if (V.exp) launch_exp_iteration(t, (uint32_t)(iters_done + i), rows.as<double>() + (size_t)i * WR);
@@ -1554,34 +1688,24 @@ struct ChainT : pm_chain {
     check_device_errors();
     return rows_h[0];
   }
+  // partials of the current state: a pruning pass over the site's block (into slot 0 of the fused kernel's partials) or
+  // over all sites, then the site's column
   void partials(int tree, int64_t site, double* out) override {
     TreeDev<Real>& t = *trees.at(tree);
     const int T = t.sch.T;
     if (site < 0 || site >= t.S) fail(PM_ERR_ARG, "bad site");
+    CK(cudaSetDevice(opt.device));
+    launch_prune(t, site);
+    CK(cudaStreamSynchronize(stream));
+    const long long col = t.pl_slots ? site % 32 : site;
     std::fill(out, out + (size_t)(2 * T - 1) * n, 0.0);
     std::vector<Real> v(n);
-    long long lsite = site;
-    if (t.pl_slots && t.slots_per_sm) {  // the slots hold whatever site blocks came last: prune the block of `site` on the current state (into slot 0)
-      CK(cudaSetDevice(opt.device));
-      launch_prune(t, site);
-      CK(cudaStreamSynchronize(stream));
-      lsite = site % 32;
-    }  // (fewer site blocks than slots: block i uses slot i, column = site)
     for (int i = 0; i < T - 1; i++) {
-      CK(cudaMemcpy(v.data(), t.PL.template as<Real>() + ((size_t)i * t.pl_sites + lsite) * n, n * sizeof(Real), cudaMemcpyDeviceToHost));
+      CK(cudaMemcpy(v.data(), t.PL.template as<Real>() + ((size_t)i * t.pl_sites + col) * n, n * sizeof(Real), cudaMemcpyDeviceToHost));
       for (int j = 0; j < n; j++) out[(size_t)(T + i) * n + j] = (double)v[j];
     }
   }
 };
-
-template <> void ChainT<double>::launch_sweep(TreeDev<double>& t, uint32_t iter, double* row) {
-  if (exact) launch_sweep_e<true>(t, iter, row); else launch_sweep_e<false>(t, iter, row);
-}
-template <> void ChainT<float>::launch_sweep(TreeDev<float>& t, uint32_t iter, double* row) { launch_sweep_e<false>(t, iter, row); }
-template <> void ChainT<double>::launch_prune(TreeDev<double>& t, long long only_site) {
-  if (exact) launch_prune_e<true>(t, only_site); else launch_prune_e<false>(t, only_site);
-}
-template <> void ChainT<float>::launch_prune(TreeDev<float>& t, long long only_site) { launch_prune_e<false>(t, only_site); }
 
 struct EigenIn { const double* lefts; const double* rights; const double* d; };
 
@@ -1644,8 +1768,7 @@ int one_call(int variant, const pm_tree* trees, int ntrees, int n, double* Q, co
     if (!opt) { pm_default_options(&def); opt = &def; }
     const bool fixed_q = variant == PM_V_PLAIN || variant == PM_V_SPARSE || variant == PM_V_BIGTREE || variant == PM_V_EXP;
     const bool single_process = !opt->allreduce && opt->nccl_world <= 1;
-    long long tile = 0;  // sites per chain; 0 = all at once
-    if (const char* v = getenv("PHYLOMAP_B200_SITE_TILE")) tile = atoll(v);
+    long long tile = read_switches().site_tile;  // sites per chain; 0 = all at once
     if (!fixed_q || !trees || ntrees != 1 || opt->rng == PM_RNG_TABLE || trees[0].n_sites < 2) tile = 0;
     const long long S = trees ? trees[0].n_sites : 0;
     // A call whose state does not fit in device memory is cut into site tiles, run one after the other (each an

@@ -497,6 +497,33 @@ def test_partials_match_exact_pruning(name, precision, monkeypatch):
                     tree_index=t, what=name.split("_")[0])
 
 
+PARTIALS_LAYOUTS = ([(name, p) for name in ["plain2_small1", "bigtree4_S40000_f1p1", "bigtree4_S37_f1p1", "bigtree4_S37_f0p1",
+                                             "dic2s"] for p in ("f32", "f64")] + [("bigtree4_S37_deterministic", "f64")])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name,precision", PARTIALS_LAYOUTS)
+def test_partials_prune_the_current_state(name, precision, monkeypatch):
+    """partials(s) right after run(k), with no time_prune before it, against exact_partials with the piece counts read back:
+    the call prunes the current state itself, whichever kernels the chain runs.  The layouts: the one-block-per-site chain
+    (which writes no partials array of its own), the fused kernel with more site blocks than slots, with fewer, the separate
+    kernels, a DIC chain (whose log-likelihood pass reuses the partials array) and the deterministic mode."""
+    if name == "bigtree4_S40000_f1p1":          # more site blocks than any B200 has slots (at most 8 x 148 x 32 sites)
+        c = _gpu_case("bigtree4_S37_f1p1")
+        c["trees"] = [cases.tree_n(cases.q4(), T=40, S=40000, seed=5, mean_branch=1.5, segments=3)]
+    elif name == "bigtree4_S37_deterministic":
+        c = _gpu_case("bigtree4_S37")
+        c["opts"] = {"mode": "deterministic"}
+    else:
+        c = _gpu_case(name)
+    ch = _chain(c, 3, precision, monkeypatch)
+    ch.run(3)
+    tree = c["trees"][0]
+    S = tree.n_sites()
+    _audit_partials(ch, tree, sorted(set([0, S // 2, S - 1])), ch.piece_counts(), np.array(ch.B), precision,
+                    what=name.split("_")[0])
+
+
 def _underflow_sites(tree, m, B, limit=1e-30):
     """Sites of `tree` where some node's unnormalised product of the two (normalised) child contributions sums to less
     than `limit` in FP64: where FP32 pruning redoes the node in double."""
