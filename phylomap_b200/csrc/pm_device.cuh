@@ -342,6 +342,41 @@ __device__ __forceinline__ void pair_block(const RngDesc& d, uint32_t local_site
   philox4x32_10_rk(e >> 1, make_slot(K_BRPAIR, 0u), it, d.site0 + local_site, d.rk, o);
 }
 
+// pair_block for a kernel that draws many pair blocks of ONE sweep: of the counter (e >> 1, K_BRPAIR slot, sweep, site)
+// only the site differs between threads and only e >> 1 between pairs, so what the first three rounds compute from the
+// other words is computed once (the same integer operations, regrouped: the same words)
+struct PairBlocks {
+  uint32_t a, k2, k3, k5;
+  // hi and lo word of m * c as ONE wide multiply (written as two, the products are sometimes issued as two instructions)
+  static __device__ __forceinline__ void mulw(uint32_t m, uint32_t c, uint32_t& hi, uint32_t& lo) {
+    const uint64_t p = (uint64_t)m * c;
+    hi = (uint32_t)(p >> 32); lo = (uint32_t)p;
+  }
+  __device__ __forceinline__ PairBlocks(const RngDesc& d, uint32_t it) {
+    a = __umulhi(0xCD9E8D57u, it) ^ make_slot(K_BRPAIR, 0u) ^ d.rk[0];  // round 1: c0' (c2 = it)
+    k2 = (0xCD9E8D57u * it) ^ d.rk[2];                                  // round 2: c1 ^ key (c1 = round 1's lo(M1 it))
+    k3 = __umulhi(0xD2511F53u, a) ^ d.rk[3];                            // round 2: hi(M0 c0) ^ key
+    k5 = (0xD2511F53u * a) ^ d.rk[5];                                   // round 3: c3 ^ key (c3 = round 2's lo(M0 c0))
+  }
+  // the block of pair j = e >> 1 at global site gsite (= d.site0 + local site)
+  __device__ __forceinline__ void block(const RngDesc& d, uint32_t j, uint32_t gsite, uint32_t o[4]) const {
+    uint32_t h0, l0, h1, l1;
+    mulw(0xD2511F53u, j, h0, l0);                                       // round 1: c2' = h0 ^ site ^ key, c3' = l0
+    mulw(0xCD9E8D57u, h0 ^ gsite ^ d.rk[1], h1, l1);                    // round 2
+    uint32_t c0 = h1 ^ k2, c1 = l1, c2 = l0 ^ k3, c3;
+    mulw(0xD2511F53u, c0, h0, l0);                                      // round 3
+    mulw(0xCD9E8D57u, c2, h1, l1);
+    c0 = h1 ^ c1 ^ d.rk[4]; c2 = h0 ^ k5; c1 = l1; c3 = l0;
+#pragma unroll
+    for (int r = 3; r < 10; r++) {
+      mulw(0xD2511F53u, c0, h0, l0);
+      mulw(0xCD9E8D57u, c2, h1, l1);
+      c0 = h1 ^ c1 ^ d.rk[2 * r]; c2 = h0 ^ c3 ^ d.rk[2 * r + 1]; c1 = l1; c3 = l0;
+    }
+    o[0] = c0; o[1] = c1; o[2] = c2; o[3] = c3;
+  }
+};
+
 // ------------------------------------------------------------------------------------------------
 // Categorical draw.
 //  EXACT: RcppArmadillo::sample(sts, 1, TRUE, w): FixProb (validate, divide by the sum of the positive entries),

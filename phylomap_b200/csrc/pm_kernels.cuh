@@ -1118,26 +1118,53 @@ __device__ __forceinline__ float lds_real(unsigned a, float) { float v; asm vola
 __device__ __forceinline__ double lds_real(unsigned a, double) { double v; asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
 __device__ __forceinline__ unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
-// Shared-memory layout of k_paths_easy, in bytes from the start of the dynamic window (all offsets multiples of 16):
-//   [0, dw) dwell partials [4 warps][n] f64 | cnt: transition counters [n*n] u32 | rate [n] | unit: identity matrix [n][n]
-//   | topo: one 16-byte entry per branch of the chunk: parent node, child node (int), branch length (Real)
+// Shared-memory layout of k_paths_easy, in bytes from the start of the dynamic window (offsets up to topo multiples of 16):
+//   [0, dw) dwell partials [4 warps][n] f64 | cnt: transition counters [n*n] u32 | rate [n] | acc: every thread's dwell
+//   sums, [NS][128 threads] of Real (the current stretch of 32 branch pairs), then [NS][128] of f64 (the flushed
+//   stretches; NS > 0 only) | topo: the chunk's topology, parent and child node (int2) per branch | len: its branch lengths
 // With a compile-time state count every offset but the entry index is an immediate, so the kernel keeps ONE base address
 // in a register (formed from several pointers, the compiler rebuilds the shared window base at every use: ~10 % of the
 // loop's instructions).
-template <typename Real>
+template <typename Real, int NS>
 struct EasySmem {
-  int cnt, rate, unit, topo;
+  int cnt, rate, acc, sum, topo;
   __host__ __device__ static int up16(int x) { return (x + 15) & ~15; }
   __host__ __device__ explicit EasySmem(int n) {
     cnt = up16(4 * n * (int)sizeof(double));
     rate = up16(cnt + n * n * (int)sizeof(unsigned));
-    unit = up16(rate + n * (int)sizeof(Real));
-    topo = up16(unit + n * n * (int)sizeof(Real));
+    acc = up16(rate + n * (int)sizeof(Real));
+    sum = acc + (NS > 0 ? NS * 128 * (int)sizeof(Real) : 0);
+    topo = sum + (NS > 0 ? NS * 128 * (int)sizeof(double) : 0);
   }
-  __host__ __device__ size_t bytes(int chunk) const { return (size_t)topo + (size_t)chunk * 16; }
+  __host__ __device__ int len(int chunk) const { return topo + chunk * 8; }
+  __host__ __device__ size_t bytes(int chunk) const { return (size_t)len(chunk) + (size_t)chunk * sizeof(Real); }
 };
 __device__ __forceinline__ void lds_v2s32(unsigned a, int& x, int& y) { asm volatile("ld.shared.v2.s32 {%0,%1}, [%2];" : "=r"(x), "=r"(y) : "r"(a)); }
-__device__ __forceinline__ void red_shared_inc(unsigned a) { asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(a) : "memory"); }
+// Predicated forms (one set-predicate, then @p instructions): guarded by an `if`, the compiler branches around them.
+__device__ __forceinline__ void red_shared_inc_if(bool p, unsigned a) {
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %1, 0;\n\t@q red.shared.add.u32 [%0], 1;\n\t}" ::"r"(a), "r"((unsigned)p) : "memory");
+}
+// *a += x in shared memory, rounded once (the same bits as a register sum: fma(1, x, s) = s + x)
+__device__ __forceinline__ void sts_add_if(bool p, unsigned a, float x) {
+  asm volatile("{\n\t.reg .pred q;\n\t.reg .f32 v;\n\tsetp.ne.b32 q, %2, 0;\n\t@q ld.shared.f32 v, [%0];\n\t@q add.rn.f32 v, v, %1;\n\t"
+               "@q st.shared.f32 [%0], v;\n\t}" ::"r"(a), "f"(x), "r"((unsigned)p));
+}
+__device__ __forceinline__ void sts_add_if(bool p, unsigned a, double x) {
+  asm volatile("{\n\t.reg .pred q;\n\t.reg .f64 v;\n\tsetp.ne.b32 q, %2, 0;\n\t@q ld.shared.f64 v, [%0];\n\t@q add.rn.f64 v, v, %1;\n\t"
+               "@q st.shared.f64 [%0], v;\n\t}" ::"r"(a), "d"(x), "r"((unsigned)p));
+}
+__device__ __forceinline__ void sts_real(unsigned a, float x) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(x)); }
+__device__ __forceinline__ void sts_real(unsigned a, double x) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(x)); }
+// global loads and stores through pointers the kernel keeps in registers (asm outputs): the compiler no longer knows
+// they point to global memory and would emit generic accesses
+__device__ __forceinline__ uint32_t ldg_u32(const uint32_t* a) { uint32_t v; asm volatile("ld.global.u32 %0, [%1];" : "=r"(v) : "l"(a)); return v; }
+__device__ __forceinline__ int ldg_u8(const uint8_t* a) { uint32_t v; asm volatile("ld.global.u8 %0, [%1];" : "=r"(v) : "l"(a)); return (int)v; }
+__device__ __forceinline__ void stg_u32_if(bool p, uint32_t* a, uint32_t x) {
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.u32 [%0], %1;\n\t}" ::"l"(a), "r"(x), "r"((unsigned)p));
+}
+__device__ __forceinline__ void stg_u16_if(bool p, uint16_t* a, uint16_t x) {
+  asm volatile("{\n\t.reg .pred q;\n\tsetp.ne.b32 q, %2, 0;\n\t@q st.global.u16 [%0], %1;\n\t}" ::"l"(a), "h"(x), "r"((unsigned)p));
+}
 
 template <typename Real, int NS>
 __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy(ChainParams<Real> P, uint32_t iter, int chunk) {
@@ -1146,63 +1173,68 @@ __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy
   typedef Pin<Real> PN;
   const int n = NS > 0 ? NS : P.n;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  const EasySmem<Real> lay(n);
+  const EasySmem<Real, NS> lay(n);
   double* s_dw = reinterpret_cast<double*>(smem_raw);                       // [4 warps][n] (NS>0) or [n] atomics (NS==0)
   unsigned* s_cnt = reinterpret_cast<unsigned*>(smem_raw + lay.cnt);       // [n*n] (a copy per warp was tried: +2 % time)
   Real* s_rate = reinterpret_cast<Real*>(smem_raw + lay.rate);             // [n] Omega + Q_ss of this sweep
-  // dwell of state s: Racc += e_s * L with the unit vector e_s read from shared memory (one vector load + NS fused
-  // multiply-adds; fma(1, L, acc) = acc + L and fma(0, L, acc) = acc exactly) instead of NS compare / select / add triples
-  Real* s_unit = reinterpret_cast<Real*>(smem_raw + lay.unit);             // [n][n]
+  // dwell of state s: the thread's running sum acc[s][thread] += L in shared memory (address = state * 128 * sizeof(Real)
+  // + the thread's own column: conflict-free, one load / add / store per run, skipped where the lane has nothing to add);
+  // every 32 branch pairs it is added to sum[s][thread] in double.  Neither takes registers in the loop.
+  Real* s_acc = reinterpret_cast<Real*>(smem_raw + lay.acc);               // [NS][128]
+  double* s_sum = reinterpret_cast<double*>(smem_raw + lay.sum);           // [NS][128]
   // topology of the chunk (the same for every thread of the block): parent / child node and branch length per branch
-  unsigned char* s_topo = smem_raw + lay.topo;
+  int2* s_topo = reinterpret_cast<int2*>(smem_raw + lay.topo);
+  Real* s_len = reinterpret_cast<Real*>(smem_raw + lay.len(chunk));
   const int e0 = blockIdx.y * chunk, e1 = min(P.E, e0 + chunk);
-  for (int i = threadIdx.x; i < n * n; i += blockDim.x) { s_cnt[i] = 0; s_unit[i] = (i / n == i % n) ? (Real)1 : (Real)0; }
+  for (int i = threadIdx.x; i < n * n; i += blockDim.x) s_cnt[i] = 0;
   for (int i = threadIdx.x; i < n; i += blockDim.x) {  // a state without a valid rate draws no virtual jumps
     const Real r = P.model[2 * n * n + 4 * n + i];
     s_rate[i] = rate_ok(r) ? r : (Real)0;
   }
   for (int i = threadIdx.x; i < 4 * n; i += blockDim.x) s_dw[i] = 0.0;
+  if (NS > 0) for (int j = 0; j < NS; j++) { s_acc[j * 128 + threadIdx.x] = 0; s_sum[j * 128 + threadIdx.x] = 0.0; }
   for (int i = threadIdx.x; i < e1 - e0; i += blockDim.x) {
-    int* en = reinterpret_cast<int*>(s_topo + 16 * (size_t)i);
-    en[0] = P.e_parent[e0 + i]; en[1] = P.e_child[e0 + i];
-    *reinterpret_cast<Real*>(en + 2) = P.e_len[e0 + i];
+    s_topo[i] = make_int2(P.e_parent[e0 + i], P.e_child[e0 + i]);
+    s_len[i] = P.e_len[e0 + i];
   }
   __syncthreads();
   // ONE 32-bit shared-memory base, kept in a register; everything else is base + immediate (+ scaled index)
   unsigned a_base = smem_addr(smem_raw);
   asm volatile("" : "+r"(a_base));
-  const unsigned a_cnt = a_base + (unsigned)lay.cnt, a_rate = a_base + (unsigned)lay.rate, a_unit = a_base + (unsigned)lay.unit,
-                 a_topo = a_base + (unsigned)lay.topo;
+  const unsigned a_cnt = a_base + (unsigned)lay.cnt, a_rate = a_base + (unsigned)lay.rate, a_topo = a_base + (unsigned)lay.topo,
+                 a_len = a_base + (unsigned)lay.len(chunk);
+  const unsigned a_acc = a_base + (unsigned)lay.acc + (unsigned)sizeof(Real) * threadIdx.x,
+                 a_sum = a_base + (unsigned)lay.sum + (unsigned)sizeof(double) * threadIdx.x;
   const long long S = P.S;
-  const uint32_t Su = (uint32_t)S;  // S < 2^31 (checked by the host): 32 x 32 -> 64-bit offsets are one instruction
+  uint32_t Su = (uint32_t)S;  // S < 2^31 (checked by the host): 32 x 32 -> 64-bit offsets are one instruction
   const long long site_raw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long site = site_raw < S ? site_raw : S - 1;
   const bool full = P.full_counts != 0;
   const long long wglob = site_raw >> 5;  // ballot word of this warp (the same for its 32 lanes)
   // Rows of the chunk are addressed as base + 32-bit element index (the host keeps chunk x S below 2^32): one wide
   // multiply-add per access and one add per branch, instead of a 64-bit pointer bump per array
-  uint32_t* __restrict__ const bal_b = P.hard_ballot + (long long)e0 * P.W + wglob;
-  const bool bal_writer = (threadIdx.x & 31) == 0 && wglob < (long long)P.W;
-  const uint32_t Wu = (uint32_t)P.W;
-  uint32_t* __restrict__ const meta_b = P.meta + (long long)e0 * S + site;   // row i of the chunk: meta_b[i * S]
-  uint16_t* __restrict__ const shape_b = P.shape + (long long)e0 * S + site;
+  uint32_t* __restrict__ bal_b = P.hard_ballot + (long long)e0 * P.W + wglob;
+  unsigned bal_writer = (threadIdx.x & 31) == 0 && wglob < (long long)P.W;
+  uint32_t Wu = (uint32_t)P.W;
+  uint32_t* __restrict__ meta_b = P.meta + (long long)e0 * S + site;   // row i of the chunk: meta_b[i * S]
+  uint16_t* __restrict__ shape_b = P.shape + (long long)e0 * S + site;
   uint32_t row = 0, rowf = 0, rowb = 0;  // i * S of the store cursor and of the fetch cursor, i * W of the ballot cursor
   const uint8_t* __restrict__ nstate = P.node_state + site;
-  Real Racc[NR]; double Rsum[NR];
-#pragma unroll
-  for (int j = 0; j < NR; j++) { Racc[j] = 0; Rsum[j] = 0; }
-  auto add_dwell = [&](int s, Real L) {
-    if (NS > 0) {
-      Real u[NR];
-      lds_vec<Real, NS>(a_unit + (unsigned)s * (unsigned)(NR * sizeof(Real)), u);
-#pragma unroll
-      for (int j = 0; j < NR; j++) Racc[j] = fma(u[j], L, Racc[j]);
-    } else if (L != (Real)0) atomicAdd(&s_dw[s], (double)L);
+  // kept in registers for the whole loop (left to itself, the compiler reloads them from the parameter bank and redoes
+  // the 64-bit additions at every use; the FP64 kernel has no registers to spare for them: it would spill)
+  if (sizeof(Real) == 4) asm volatile("" : "+l"(bal_b), "+l"(meta_b), "+l"(shape_b), "+l"(nstate), "+r"(Wu), "+r"(Su), "+r"(bal_writer));
+  auto add_dwell = [&](int s, Real L, bool p) {
+    if (NS > 0) sts_add_if(p, a_acc + (unsigned)s * (unsigned)(128 * sizeof(Real)), L);
+    else if (p && L != (Real)0) atomicAdd(&s_dw[s], (double)L);
   };
   auto flush_dwell = [&]() {
     if (NS > 0) {
 #pragma unroll
-      for (int j = 0; j < NR; j++) { Rsum[j] += (double)Racc[j]; Racc[j] = 0; }
+      for (int j = 0; j < NR; j++) {
+        const unsigned a = a_acc + (unsigned)j * (unsigned)(128 * sizeof(Real)), b = a_sum + (unsigned)j * (128u * 8u);
+        sts_real(b, lds_real(b, 0.0) + (double)lds_real(a, (Real)0));
+        sts_real(a, (Real)0);
+      }
     }
   };
   // Software pipeline over pairs of branches (2j, 2j + 1: they share a Philox block): at the top of a trip the state
@@ -1212,13 +1244,15 @@ __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy
   struct Ahead { uint32_t mt; int ps, cs; };
   Ahead X = {0, 0, 0}, Y = {0, 0, 0};
   auto fetch = [&](int i, Ahead& a) {
-    a.mt = meta_b[rowf]; rowf += Su;
+    a.mt = ldg_u32(meta_b + rowf); rowf += Su;
     int par, chi;
-    lds_v2s32(a_topo + 16u * (unsigned)i, par, chi);
-    a.ps = nstate[(uint64_t)(uint32_t)par * Su];
-    a.cs = nstate[(uint64_t)(uint32_t)chi * Su];
+    lds_v2s32(a_topo + 8u * (unsigned)i, par, chi);
+    a.ps = ldg_u8(nstate + (uint64_t)(uint32_t)par * Su);
+    a.cs = ldg_u8(nstate + (uint64_t)(uint32_t)chi * Su);
   };
   uint32_t po[4] = {0, 0, 0, 0};
+  const PairBlocks pb(P.rng, iter);
+  const uint32_t gsite = P.rng.site0 + (uint32_t)site;
   // one branch, from what was fetched for it.  ODD: second branch of its Philox pair (the block was drawn by the first,
   // unless NEWBLK: it opens the chunk).  TAIL: the block may hold sites past the end.  Straight-line code: lanes that
   // leave their branch to the general kernels compute along and contribute zeros; only the stores are predicated.
@@ -1226,11 +1260,11 @@ __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy
     constexpr bool ODD = decltype(odd_c)::value, NEWBLK = decltype(newblk_c)::value, TAIL = decltype(tail_c)::value;
     const int e = e0 + i;
     const uint32_t mt = cur.mt; const int ps = cur.ps, cs = cur.cs;
-    if (NEWBLK) pair_block(P.rng, (uint32_t)site, iter, (uint32_t)e, po);
+    if (NEWBLK) pb.block(P.rng, (uint32_t)e >> 1, gsite, po);
     const uint32_t wA = ODD ? po[2] : po[0], wB = ODD ? po[3] : po[1];
     const int m = (int)(mt & 0xffffu);
     const uint32_t q = mt >> 16;
-    const Real Le = lds_real(a_topo + 16u * (unsigned)i + 8u, (Real)0);
+    const Real Le = lds_real(a_len + (unsigned)sizeof(Real) * (unsigned)i, (Real)0);
     // pieces: (Le) or (p1, Le - p1); states ps | cs (a one-piece branch carries the child state, :460-475).  The
     // virtual jumps of a two-run path are counted together: K ~ Poisson(lam0 + lam1) from the A word (their positions,
     // if a later sweep needs them, are regenerated by the general kernels, see RunPieces)
@@ -1245,16 +1279,17 @@ __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy
     const bool hard = (m > 2) || lam > (Real)PM_LAMBDA_INV;
     const bool ok = TAIL ? (!hard && site_raw < S) : !hard;
     const int k = poisson_inv<Real>(lam, wA);
-    if (ok && m == 2 && (full || two)) red_shared_inc(a_cnt + 4u * (unsigned)(ps * n + cs));
-    add_dwell(s0, ok ? L0 : (Real)0);
-    add_dwell(cs, ok ? L1 : (Real)0);
+    red_shared_inc_if(ok && m == 2 && (full || two), a_cnt + 4u * (unsigned)(ps * n + cs));
+    add_dwell(s0, L0, ok);
+    add_dwell(cs, L1, ok && two);  // (a single run adds nothing here)
     // a path that ends up with a single jump point keeps that point in the state word: the real jump stays where it
     // was; a lone new virtual jump is uniform on the branch -- its 16-bit position comes from the B word
     const uint32_t newq = (!two && k == 1) ? pos_rand(wB) : q;
-    if (ok) { meta_b[row] = PM_META((two ? 2 : 1) + k, newq); shape_b[row] = PM_SHAPE(two ? 1 : 0, s0, cs); }
+    stg_u32_if(ok, meta_b + row, (newq << 16) + (uint32_t)((two ? 2 : 1) + k));  // = PM_META (k <= 64)
+    stg_u16_if(ok, shape_b + row, (uint16_t)(((uint32_t)cs << 11) + ((uint32_t)s0 << 6) + (two ? 1u : 0u)));  // = PM_SHAPE
     row += Su;
     const unsigned bal = __ballot_sync(0xffffffffu, TAIL ? (hard && site_raw < S) : hard);
-    if (bal_writer) bal_b[rowb] = bal;
+    stg_u32_if(bal_writer != 0, bal_b + rowb, bal);
     rowb += Wu;
   };
   auto run = [&](auto tail_c) {
@@ -1292,7 +1327,7 @@ __global__ void __launch_bounds__(128, (sizeof(Real) == 8 ? 6 : 8)) k_paths_easy
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
     for (int j = 0; j < NR; j++) {
-      double v = Rsum[j];
+      double v = lds_real(a_sum + (unsigned)j * (128u * 8u), 0.0);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
       if (lane == 0) s_dw[warp * n + j] = v;

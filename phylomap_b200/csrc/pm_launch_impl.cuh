@@ -66,7 +66,7 @@ void Sweep<Real, NS, EXACT>::paths(const ChainParams<Real>& P, dim3 grid, size_t
   else {
     // the easy kernel also serves the first sweep: a map of one or two pieces is a path like any other (pos1 was
     // seeded from it), only longer maps are walked piece by piece by the general kernel
-    const size_t smem_easy = EasySmem<Real>(P.n).bytes(chunk);
+    const size_t smem_easy = EasySmem<Real, NS>(P.n).bytes(chunk);
     k_paths_easy<Real, NS><<<grid, 128, smem_easy, st>>>(P, iter, chunk);
     // (the short shape does not occur in the first sweep: the caller's maps are walked by the general routine)
     if (!first) k_paths_hard<Real, NS, 8, 0><<<2 * hard_blocks, 128, smem, st>>>(P, iter, first);
