@@ -228,6 +228,17 @@ void pm_chain_overheads(pm_chain* c, double ms[2]);
 int pm_chain_get_node_states(pm_chain* c, int32_t tree, int32_t* out /* [S][2T-1] 0-based */);
 int pm_chain_get_piece_counts(pm_chain* c, int32_t tree, int32_t* out /* [S][E] */);
 int pm_chain_get_path(pm_chain* c, int32_t tree, int64_t site, int32_t e, double* len, int32_t* st, int32_t cap);
+/* Stochastic maps of the current chain state: the merged history of every branch of the selected LOCAL sites of tree
+ * `tree`, as stored after the last sweep.  Output is CSR, site-major in the order of `sites`, branches in edge-row order
+ * (x$edge), runs from the parent end to the child end:
+ *   off[i*E + e] .. off[i*E + e + 1]  -> len[], st[] (0-based states), i = position in `sites`;  off has nsel*E + 1 entries.
+ * off is always written.  len / st are written when non-NULL and cap >= off[nsel*E]; when non-NULL with a smaller cap the
+ * call returns PM_ERR_CAPACITY having written off (and nothing beyond len[cap - 1] / st[cap - 1]).  Sites may repeat and
+ * come in any order.  Every run equals what pm_chain_get_path returns for the same (site, branch).  Decoded on the device
+ * in batches of sites; does not modify the chain.  PM_ERR_ARG for a bad tree or site, before the first sweep, and for the
+ * chains that keep no paths (the direct sampler). */
+int pm_chain_get_maps(pm_chain* c, int32_t tree, const int64_t* sites, int64_t nsel, int64_t* off, double* len,
+                      int32_t* st, int64_t cap, char* err, size_t errlen);
 /* Partials of the current chain state at `site`, computed by a pruning pass that the call runs; tip rows are zero. */
 int pm_chain_get_partials(pm_chain* c, int32_t tree, int64_t site, double* out /* [2T-1][n], tip rows zero */);
 int64_t pm_chain_device_bytes(pm_chain* c);

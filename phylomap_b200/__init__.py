@@ -10,4 +10,5 @@ from .api import (Chain, SPARSEmaketreelistMCMC, SPARSEsumstatMCMC, colnames, lo
                   maketreelistMCMCksDICt, maketreelistMCMCksmt, maketreelistMCMCmt, myreorder, pruningwiseedgeorder,
                   sumstatEXP, sumstatMCMC, sumstatMCMC2sDICt, sumstatMCMC_bigtree, sumstatMCMCbf, sumstatMCMCks, sumstatMCMCksDICt,
                   sumstatMCMCksmt, sumstatMCMCmt)
+from .simmap import StochasticMaps, multi_simmap  # noqa: F401
 from .tree import PhyloTree  # noqa: F401

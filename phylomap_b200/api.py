@@ -25,6 +25,7 @@ import os
 import numpy as np
 
 from . import capi
+from .simmap import StochasticMaps
 from .tree import PhyloTree
 
 BF_COLNAMES = ["time_0", "time_1", "n00", "n01", "n10", "n11", "l01", "l10", "root_state"]
@@ -193,6 +194,39 @@ class Chain:
         if k < 0:
             raise capi.PhylomapError(-k, "get_path")
         return ln[:k].copy(), st[:k].copy()
+
+    def maps(self, sites=None, tree=0):
+        """Stochastic maps of the current state (pm_chain_get_maps): the history every selected site holds on every branch of
+        tree `tree` after the last sweep, decoded on the device, as a `simmap.StochasticMaps`.  `sites` are LOCAL site
+        indices (default: all); under site sharding the global index is `site_offset` + local.  Repeated and unsorted
+        indices are allowed.  Does not modify the chain."""
+        L = capi.lib()
+        t = self.trees[tree]
+        sel = np.arange(t.n_sites(), dtype=np.int64) if sites is None else np.ascontiguousarray(sites, dtype=np.int64).reshape(-1)
+        off = np.zeros(len(sel) * t.E + 1, dtype=np.int64)
+        err = C.create_string_buffer(512)
+        capi.check(L.pm_chain_get_maps(self.h, tree, capi.ptr(sel), len(sel), capi.ptr(off), None, None, 0, err, 512), err)
+        total = int(off[-1])
+        length = np.empty(total, dtype=np.float64)
+        state = np.empty(total, dtype=np.int32)
+        capi.check(L.pm_chain_get_maps(self.h, tree, capi.ptr(sel), len(sel), capi.ptr(off), capi.ptr(length), capi.ptr(state),
+                                       total, err, 512), err)
+        return StochasticMaps(sel, off, length, state, self.n, t)
+
+    def sample_maps(self, count, every, sites=None, tree=0):
+        """Run `count` sweeps in blocks of `every` and export the maps after each block: (rows, [StochasticMaps, ...]).  The
+        rows are those one run(count) returns (device uniforms are keyed by sweep index, so a chain resumes bit for bit)."""
+        if every < 1:
+            raise ValueError("every must be >= 1")
+        rows, maps = [], []
+        done = 0
+        while done < count:
+            k = min(every, count - done)
+            rows.append(self.run(k))
+            maps.append(self.maps(sites, tree))
+            done += k
+        out = np.concatenate(rows, axis=0) if rows else np.zeros((0, self.ncols))
+        return np.asfortranarray(out), maps
 
     def partials(self, site=0, tree=0):
         t = self.trees[tree]

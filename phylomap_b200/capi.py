@@ -43,7 +43,7 @@ EXPORTS = ["pm_default_options", "pm_nccl_unique_id", "pm_maketreelistMCMC", "pm
            "pm_ncols", "pm_tree_order", "pm_debug_clade_schedule", "pm_chain_create", "pm_chain_run", "pm_chain_state_bytes",
            "pm_chain_export_state", "pm_chain_import_state", "pm_chain_time_prune",
            "pm_chain_kernel_times", "pm_chain_enable_timing", "pm_chain_overheads", "pm_chain_get_node_states", "pm_chain_get_piece_counts",
-           "pm_chain_get_path", "pm_chain_get_partials", "pm_chain_device_bytes", "pm_chain_acceptance", "pm_chain_destroy",
+           "pm_chain_get_path", "pm_chain_get_maps", "pm_chain_get_partials", "pm_chain_device_bytes", "pm_chain_acceptance", "pm_chain_destroy",
            "pm_rng_probe", "pm_release_cached_memory", "pm_device_count", "pm_version"]
 
 _LIB = None
@@ -97,6 +97,7 @@ def lib():
     L.pm_chain_get_node_states.argtypes = [vp, i32, vp]
     L.pm_chain_get_piece_counts.argtypes = [vp, i32, vp]
     L.pm_chain_get_path.argtypes = [vp, i32, i64, i32, vp, vp, i32]
+    L.pm_chain_get_maps.argtypes = [vp, i32, vp, i64, vp, vp, vp, i64, C.c_char_p, C.c_size_t]
     L.pm_chain_get_partials.argtypes = [vp, i32, i64, vp]
     L.pm_chain_device_bytes.argtypes = [vp]
     L.pm_chain_device_bytes.restype = i64

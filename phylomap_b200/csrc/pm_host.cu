@@ -9,6 +9,7 @@
 // maketreelistMCMC_bigtree :942, maketreelistMCMCbf :1258, maketreelistMCMCks :1802, maketreelistMCMCmt :2267,
 // maketreelistMCMCksmt :2722.
 #include <cuda_runtime.h>
+#include <cub/device/device_scan.cuh>
 
 #include <algorithm>
 #include <chrono>
@@ -28,6 +29,7 @@
 #include "pm_launch.cuh"
 #include "pm_setup_kernels.cuh"
 #include "pm_loglik.cuh"
+#include "pm_maps.cuh"
 #include "pm_exp.cuh"
 #include "pm_nccl.hpp"
 #include "pm_rates.hpp"
@@ -317,6 +319,7 @@ struct pm_chain {
   virtual void node_states(int tree, int32_t* out) = 0;
   virtual void piece_counts(int tree, int32_t* out) = 0;
   virtual int path(int tree, int64_t site, int e, double* len, int32_t* st, int cap) = 0;
+  virtual void maps(int tree, const int64_t* sites, int64_t nsel, int64_t* off, double* len, int32_t* st, int64_t cap) = 0;
   virtual void partials(int tree, int64_t site, double* out) = 0;
   virtual double loglik() = 0;
   virtual int64_t state_bytes() = 0;
@@ -1582,6 +1585,92 @@ struct ChainT : pm_chain {
     records(pos, nj + 1);
     return nj + 1;
   }
+  // Stochastic maps of the selected sites (pm_maps.cuh), in batches of sites whose selection, counts and offsets take at
+  // most half the scratch budget: count, scan, offsets to the caller; then the runs of as many consecutive sites of the
+  // batch as the other half holds at a time (more for a single site that needs it).
+  void maps(int tree, const int64_t* sites, int64_t nsel, int64_t* off, double* len, int32_t* st, int64_t cap) override {
+    if (tree < 0 || tree >= ntrees) fail(PM_ERR_ARG, "bad tree");
+    if (V.exp || V.llonly) fail(PM_ERR_ARG, "this chain keeps no path state");
+    if (nsel < 0 || cap < 0 || !off || (nsel > 0 && !sites)) fail(PM_ERR_ARG, "bad arguments");
+    TreeDev<Real>& t = *trees[tree];
+    for (int64_t i = 0; i < nsel; i++)
+      if (sites[i] < 0 || sites[i] >= t.S) fail(PM_ERR_ARG, "bad site / branch");
+    if (iters_done == 0) fail(PM_ERR_ARG, "no sweep done yet");
+    off[0] = 0;
+    if (nsel == 0) return;
+    CK(cudaSetDevice(opt.device));
+    const long long E = t.sch.E;
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const size_t budget = std::min(pm::kMapsScratchBytes, free_b / 2);
+    const size_t per_site = (size_t)E * (sizeof(int) + sizeof(long long)) + sizeof(long long);
+    const size_t run_bytes = sizeof(double) + sizeof(int32_t);
+    const long long nb = std::min<long long>({(long long)nsel, (long long)(budget / 2 / per_site), 32LL * 65535});
+    if (nb < 1) fail(PM_ERR_CUDA, "the maps of one site need %zu bytes of device scratch, %zu bytes are free", 2 * per_site, free_b);
+    const long long runs_budget = (long long)((budget - (size_t)nb * per_site) / run_bytes);
+
+    struct Scratch {  // stream-ordered device allocation
+      void* p = nullptr;
+      cudaStream_t s;
+      explicit Scratch(cudaStream_t st) : s(st) {}
+      ~Scratch() { if (p) cudaFreeAsync(p, s); }
+      void alloc(size_t n) { if (p) cudaFreeAsync(p, s); p = nullptr; CK(cudaMallocAsync(&p, std::max<size_t>(n, 16), s)); }
+    } d_sel(stream), d_cnt(stream), d_off(stream), d_tmp(stream), d_len(stream), d_st(stream);
+    size_t tmp_bytes = 0;
+    CK(cub::DeviceScan::ExclusiveScan(nullptr, tmp_bytes, (const int*)nullptr, (long long*)nullptr, ::cuda::std::plus<>{}, 0LL,
+                                      nb * E + 1, stream));
+    d_sel.alloc(nb * sizeof(long long));
+    d_cnt.alloc((nb * E + 1) * sizeof(int));
+    d_off.alloc((nb * E + 1) * sizeof(long long));
+    d_tmp.alloc(tmp_bytes);
+
+    pm::MapsSrc<Real> M;
+    const int buf = (iters_done - 1) & 1;
+    M.meta = t.meta.template as<uint32_t>(); M.shape = exact ? nullptr : t.shape.template as<uint16_t>();
+    M.e_len = t.e_len.template as<Real>();
+    M.rec_len = t.rec_len[buf].template as<Real>(); M.rec_st = t.rec_st[buf].template as<uint8_t>();
+    M.cap_off = t.cap_off.template as<int>();
+    M.S = t.S; M.rec_groups = t.rec_groups; M.E = (int)E; M.chunk = t.chunk; M.rec_shift = t.rec_shift; M.exact = exact ? 1 : 0;
+    const dim3 blk(32, 8);
+    const bool want_runs = len && st;
+    long long runs_alloc = 0, base = 0;
+    bool fits = true;
+    for (long long s0 = 0; s0 < nsel; s0 += nb) {
+      const long long nbb = std::min<long long>(nb, nsel - s0), ne = nbb * E;
+      long long* const d_offp = static_cast<long long*>(d_off.p);
+      CK(cudaMemcpyAsync(d_sel.p, sites + s0, nbb * sizeof(long long), cudaMemcpyHostToDevice, stream));
+      CK(cudaMemsetAsync(static_cast<int*>(d_cnt.p) + ne, 0, sizeof(int), stream));
+      pm::k_maps_count<Real><<<dim3((unsigned)((E + 31) / 32), (unsigned)((nbb + 31) / 32)), blk, 0, stream>>>(
+          M, static_cast<const long long*>(d_sel.p), nbb, static_cast<int*>(d_cnt.p));
+      CK(cudaGetLastError());
+      CK(cub::DeviceScan::ExclusiveScan(d_tmp.p, tmp_bytes, static_cast<const int*>(d_cnt.p), d_offp, ::cuda::std::plus<>{}, base,
+                                        ne + 1, stream));
+      CK(cudaMemcpyAsync(off + s0 * E, d_offp, (ne + 1) * sizeof(long long), cudaMemcpyDeviceToHost, stream));
+      CK(cudaStreamSynchronize(stream));
+      const long long end = off[(s0 + nbb) * E];
+      if (want_runs && end > cap) fits = false;
+      for (long long j0 = 0; want_runs && fits && j0 < nbb;) {
+        const long long r0 = off[(s0 + j0) * E];
+        long long j1 = j0 + 1;
+        while (j1 < nbb && off[(s0 + j1 + 1) * E] - r0 <= runs_budget) j1++;
+        const long long nr = off[(s0 + j1) * E] - r0;
+        if (nr > runs_alloc) {
+          runs_alloc = std::max(nr, std::min(runs_budget, end - r0));
+          d_len.alloc(runs_alloc * sizeof(double));
+          d_st.alloc(runs_alloc * sizeof(int32_t));
+        }
+        pm::k_maps_write<Real><<<dim3((unsigned)((E + 31) / 32), (unsigned)((j1 - j0 + 31) / 32)), blk, 0, stream>>>(
+            M, static_cast<const long long*>(d_sel.p), j0, j1, d_offp, r0, static_cast<double*>(d_len.p), static_cast<int32_t*>(d_st.p));
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(len + r0, d_len.p, nr * sizeof(double), cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(st + r0, d_st.p, nr * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+        j0 = j1;
+      }
+      base = end;
+    }
+    CK(cudaStreamSynchronize(stream));
+    if (want_runs && !fits) fail(PM_ERR_CAPACITY, "the maps hold %lld runs, the output arrays %lld", base, (long long)cap);
+  }
   // ---- checkpoint / resume: everything a sweep reads that is not an input of pm_chain_create ----
   static constexpr uint32_t PM_STATE_FORMAT = 6;  // 6: model and table of powers in one buffer; 5: production record slices shared by groups of 32 sites; 1: round 1 (per-site masks); 2: branch-major ballots, global record cursors; 3: two-run paths count their virtual jumps together; 4: 16-bit positions inside meta, shape words
   struct StateHeader {
@@ -2015,6 +2104,13 @@ int pm_chain_get_path(pm_chain* c, int32_t tree, int64_t site, int32_t e, double
   int r = -1;
   const int rc = guarded(nullptr, 0, [&] { r = c->path(tree, site, e, len, st, cap); });
   return rc == PM_OK ? r : -rc;
+}
+int pm_chain_get_maps(pm_chain* c, int32_t tree, const int64_t* sites, int64_t nsel, int64_t* off, double* len, int32_t* st,
+                      int64_t cap, char* err, size_t errlen) {
+  return guarded(err, errlen, [&] {
+    if (!c) fail(PM_ERR_ARG, "null argument");
+    c->maps(tree, sites, nsel, off, len, st, cap);
+  });
 }
 int pm_chain_get_partials(pm_chain* c, int32_t tree, int64_t site, double* out) {
   return guarded(nullptr, 0, [&] { c->partials(tree, site, out); });
