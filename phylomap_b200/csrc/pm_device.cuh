@@ -158,9 +158,8 @@ template <typename Real, bool EXACT> struct StreamSel { typedef StreamD type; };
 template <> struct StreamSel<float, false> { typedef StreamF type; };
 
 // ------------------------------------------------------------------------------------------------
-// Standard exponential deviate.
-//  EXACT: R's exp_rand (sexp.c, Ahrens & Dieter 1972) on the keyed stream — variable uniform consumption.
-//  fast : -log(u), one uniform.
+// Standard exponential deviate of the deterministic mode: R's exp_rand (sexp.c, Ahrens & Dieter 1972) on the keyed
+// stream — variable uniform consumption.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ double exp_rand_R(StreamD& g) {
   const double q[16] = {0.6931471805599453, 0.9333736875190459, 0.9888777961838675, 0.9984589039328340,
@@ -186,17 +185,6 @@ __device__ __forceinline__ double exp_rand_R(StreamD& g) {
   } while (u > q[i]);
   return __dadd_rn(a, __dmul_rn(umin, q[0]));
 }
-
-template <typename Real, bool EXACT> struct ExpDev;
-template <> struct ExpDev<double, true> {
-  static __device__ __forceinline__ double draw(StreamD& g) { return exp_rand_R(g); }
-};
-template <> struct ExpDev<double, false> {
-  static __device__ __forceinline__ double draw(StreamD& g) { return -log(g.next()); }
-};
-template <> struct ExpDev<float, false> {
-  static __device__ __forceinline__ float draw(StreamF& g) { return -logf(g.next()); }
-};
 
 // ------------------------------------------------------------------------------------------------
 // Production model of the virtual jumps (statistically the reference's Poisson process of rate Omega + Q_ss on every

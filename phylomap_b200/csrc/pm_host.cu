@@ -237,7 +237,6 @@ struct Switches {
   int graph = -1;                // PHYLOMAP_B200_GRAPH: 0 never, 1 always replay a captured sweep, otherwise by problem size
   bool trace = false;            // PHYLOMAP_B200_TRACE=1: host wall time of the phases of create(), on stderr
   bool debug_sync = false;       // PHYLOMAP_B200_DEBUG_SYNC=1: stop at the first sweep kernel that raises a device error flag
-  bool small_prof = false;       // PHYLOMAP_B200_SMALL_PROF (any value): k_small_chain counts the cycles of its phases
   long long site_tile = 0;       // PHYLOMAP_B200_SITE_TILE=k: fixed-Q one-call entries run k sites at a time (0: all)
 };
 
@@ -253,7 +252,6 @@ Switches read_switches() {
   if (const char* v = env("GRAPH")) s.graph = atoi(v);
   s.trace = starts("TRACE", '1');
   s.debug_sync = starts("DEBUG_SYNC", '1');
-  s.small_prof = env("SMALL_PROF") != nullptr;
   if (const char* v = env("SITE_TILE")) s.site_tile = atoll(v);
   return s;
 }
@@ -555,7 +553,6 @@ SmallOrder small_draw_order(const pm::host::Schedule& sch, const pm::host::Clade
 struct WorkItems {
   std::vector<long long> off;  // [E + 1] first item of every branch
   std::vector<int> g;          // ballot words per item, per branch
-  std::vector<int> hint;       // branch of item 64 i
 };
 template <typename Real>
 WorkItems build_work_items(const std::vector<Real>& elen, double Omega, long long S) {
@@ -572,11 +569,6 @@ WorkItems build_work_items(const std::vector<Real>& elen, double Omega, long lon
     w.g[e] = (int)g;
     w.off[e + 1] = w.off[e] + (Wl + g - 1) / g;
   }
-  w.hint.resize((size_t)(w.off[E] >> 6) + 1);
-  for (long long i = 0, e = 0; i < (long long)w.hint.size(); i++) {
-    while (e + 1 < E && w.off[e + 1] <= (i << 6)) e++;
-    w.hint[i] = (int)e;
-  }
   return w;
 }
 
@@ -586,7 +578,7 @@ struct TreeDev {
   long long S = 0, TS = 0;
   DevBuf cl_entries, cl_warp_off, cl_top_entries, cl_top_off, cd_top, cd_top_off, cd_entries, cd_warp_off, cd_tips;  // clade schedule
   DevBuf up_entries, up_off, down_entries, down_off, e_parent, e_child, e_len, maps_off, maps_len, cap_off;
-  DevBuf tipcode, node_state, meta, PL, rec_len[2], rec_st[2], dw_partial, hard_ballot, wk_off, wk_g, wk_hint, wk_item, rec_cursor, shape;
+  DevBuf tipcode, node_state, meta, PL, rec_len[2], rec_st[2], dw_partial, hard_ballot, wk_off, wk_g, wk_item, rec_cursor, shape;
   long long wk_total = 0, dw_rows = 0;
   int hard_blocks = 0;
   int pl_slots = 0;          // 32-site slots of the partials buffer (fused prune + node-draw kernel: SMs x resident blocks per SM); 0: separate kernels, partials of all sites
@@ -599,7 +591,7 @@ struct TreeDev {
   bool small_ok = false;
   bool small_two = false;    // more sites than SMs: two blocks per SM (128 registers) instead of one
   int small_chunks = 0;      // record chunks (rows of rec_cursor)
-  DevBuf small_down, small_part, small_cnt, small_root, small_prof, small_border;
+  DevBuf small_down, small_part, small_cnt, small_root, small_border;
   DevBuf tip_stage;          // staging of the tip-state upload (create() only)
   int small_cap = 0;         // sweeps the output buffers hold
   int small_order_n = 0;     // entries of small_border
@@ -665,12 +657,6 @@ struct ChainT : pm_chain {
     if (err_h) cudaFreeHost(err_h);
     if (q_h) cudaFreeHost(q_h);
     if (ctl_h) cudaFreeHost(ctl_h);
-    for (auto& t : trees) if (t && t->small_prof.p) {
-      long long h[12];
-      if (cudaMemcpy(h, t->small_prof.p, sizeof h, cudaMemcpyDeviceToHost) == cudaSuccess)
-        fprintf(stderr, "[phylomap_b200] k_small_chain block 0 (%d + %d levels), cycles over %d sweeps: prune %lld, node draws %lld, paths %lld, row %lld; paths per warp:"
-                        " %lld %lld %lld %lld %lld %lld %lld %lld\n", (int)t->sch.up_off.size() - 1, (int)t->sch.down_off.size() - 1, iters_done, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9], h[10], h[11]);
-    }
     if (sweep_graph) cudaGraphExecDestroy(sweep_graph);
     if (own_stream && stream) cudaStreamDestroy(stream);
   }
@@ -724,6 +710,8 @@ struct ChainT : pm_chain {
   }
 
   // ---- kernel dispatch ----
+  // the production arithmetic for n = 2 / 4 has kernels of its own (pm::Sweep::production)
+  bool production() const { return !exact && (NS == 2 || NS == 4); }
   // f(std::integral_constant<int, NS>) with the chain's compile-time state count: 2, 4, or 0 (run-time n)
   template <typename F>
   auto with_ns(F&& f) const {
@@ -788,11 +776,6 @@ struct ChainT : pm_chain {
     o.n_down_levels = (int)t.sch.down_off.size() - 1; o.n_chunks = t.small_chunks;
     o.br_order = t.small_border.template as<int>(); o.n_order = t.small_order_n;
     o.part = nullptr; o.cnt = nullptr; o.root = nullptr; o.rows = nullptr; o.row_stride = WR; o.err_slot = W;
-    o.prof = nullptr;
-    if (sw.small_prof) {
-      if (!t.small_prof.p) { t.small_prof.alloc(12 * sizeof(long long)); CK(cudaMemsetAsync(t.small_prof.p, 0, t.small_prof.bytes, stream)); }
-      o.prof = t.small_prof.template as<long long>();
-    }
     auto launch = [&](uint32_t it0, int nb) {
       with_ns([&](auto ns) { pm::Sweep<Real, decltype(ns)::value, false>::small_chain(t.P, (int)S, stream, it0, nb, o, t.small_two); });
     };
@@ -944,8 +927,8 @@ struct ChainT : pm_chain {
     mt.reseed((uint32_t)opt.seed);
     trace.mark("pinned buffers, replay table");
     // shared-memory sizes
-    const int np_fast = exact ? 0 : ((NS == 2 || NS == 4) ? std::min(PM_SMEM_POW, jcap) : 0);
-    smem_prune = ((size_t)n * n + (size_t)np_fast * n * n) * sizeof(Real);
+    const int np_fast = production() ? std::min(PM_SMEM_POW, jcap) : 0;
+    smem_prune = (size_t)n * n * sizeof(Real);
     smem_nodes = ((size_t)n * n + 3 * n + (size_t)np_fast * n * n) * sizeof(Real);
     smem_paths = (size_t)4 * n * sizeof(double) + ((size_t)n * n + ((n * n) & 1)) * sizeof(unsigned) +
                  ((size_t)2 * n * n + 5 * n + (size_t)np_fast * n * n) * sizeof(Real);
@@ -1081,7 +1064,7 @@ struct ChainT : pm_chain {
     std::vector<double> mlen(x.maps_len, x.maps_len + moff[E]);
 
     const size_t small_smem = with_ns([&](auto ns) { return pm::Sweep<Real, decltype(ns)::value, false>::small_smem(T); });
-    const SmallChoice small = choose_small_kernel(!exact && (NS == 2 || NS == 4) && !no_paths && opt.rng != PM_RNG_TABLE, elen,
+    const SmallChoice small = choose_small_kernel(production() && !no_paths && opt.rng != PM_RNG_TABLE, elen,
                                                   Omega, T, S, sms, small_smem, sw);
     t.small_ok = small.ok;
     t.small_two = small.two;
@@ -1100,7 +1083,7 @@ struct ChainT : pm_chain {
     plan_partials_slots(t, sms);
     upload(t.up_entries, t.sch.up_entries, stream);
     upload(t.up_off, t.sch.up_off, stream);
-    if (!exact && (NS == 2 || NS == 4)) {
+    if (production()) {
       CladeCode cc = encode_clade_schedule(t.sch, S, t.TS, (long long)t.pl_sites * n * (long long)sizeof(Real), V.redraw_tips);
       upload(t.cl_entries, cc.e16, stream);
       upload(t.cl_warp_off, cc.cs.warp_off, stream);
@@ -1179,7 +1162,7 @@ struct ChainT : pm_chain {
   void plan_partials_slots(TreeDev<Real>& t, int sms) {
     t.pl_slots = 0;
     t.pl_sites = t.S;
-    if (exact || !(NS == 2 || NS == 4) || V.dic || V.exp || V.llonly || !sw.fused) return;
+    if (!production() || V.dic || V.exp || V.llonly || !sw.fused) return;
     const size_t smem_lo = ((size_t)n * n + 3 * n) * sizeof(Real);
     const int per_sm = with_ns([&](auto ns) { return pm::Sweep<Real, decltype(ns)::value, false>::fused_blocks_per_sm(smem_lo); });
     if (per_sm < 1) fail(PM_ERR_CUDA, "cudaOccupancyMaxActiveBlocksPerMultiprocessor failed for the fused prune + node-draw kernel");
@@ -1215,7 +1198,6 @@ struct ChainT : pm_chain {
       t.hard_ballot.alloc((size_t)E * Wl * sizeof(uint32_t));
       const WorkItems w = build_work_items(elen, Omega, S);
       t.wk_total = w.off.back();
-      upload(t.wk_hint, w.hint, stream);
       upload(t.wk_off, w.off, stream);
       upload(t.wk_g, w.g, stream);
       t.wk_item.alloc((size_t)std::max<long long>(t.wk_total, 1) * sizeof(unsigned long long));
@@ -1281,8 +1263,7 @@ struct ChainT : pm_chain {
     P.n = n; P.T = T; P.E = E; P.S = t.S;
     P.cap_off = t.cap_off.template as<int>();
     P.hard_ballot = t.hard_ballot.template as<uint32_t>(); P.W = (int)((t.S + 31) / 32);
-    P.wk_off = t.wk_off.template as<long long>(); P.wk_g = t.wk_g.template as<int>(); P.wk_total = t.wk_total;
-    P.wk_hint = t.wk_hint.template as<int>(); P.wk_item = t.wk_item.template as<unsigned long long>();
+    P.wk_total = t.wk_total; P.wk_item = t.wk_item.template as<unsigned long long>();
     P.rec_cursor = t.rec_cursor.template as<int>(); P.chunk = t.chunk; P.easy_blocks = t.nblocks;
     P.shape = t.shape.template as<uint16_t>();
     P.model = model.as<Real>(); P.ppow = model.as<Real>() + model_stride(); P.jcap = jcap;

@@ -1,24 +1,20 @@
-// The four kernels of one MCMC sweep (SURVEY.md §2.3 / §8(a)):
-//   K1 k_prune   Felsenstein pruning with P_e := B^(m_e - 1)        replaces makePLrcpp* (src/phylomap.cpp:490-529,
-//      (production, n = 2 / 4: k_prune_clade)                        1077-1088, 1938-1949) + mmmmvFORpl (:446-450)
-//   K2 k_nodes   root draw + top-down node (and hidden-tip) draws    replaces sampleinternalnodes* (:535-738, 1091-1164,
-//      (production, n = 2 / 4: k_nodes_clade)                        1314-1403, 1952-2046) + updatenodestates (:460-475)
-//   K3 k_paths   per (site, branch): regenerate the virtual jumps of the previous sweep, redraw the segment states
-//                (resamplebranchstates :264-308), merge + count (shortener :44-73 / shortenerbf :997-1028), draw the
-//                new virtual jumps (:391-410), accumulate dwell times (:745-757), block-level reduction
-//   K4 k_reduce  deterministic reduction of the per-block partial sums into one row of sufficient statistics
-//
-// Data layout in HBM (site-minor everywhere, so a warp = 32 consecutive sites reads/writes contiguous bytes):
-//   tipcode    [T][TS]     u8   observed tip state (0-based) or observed parity (hidden-rate models); TS = S rounded up to 16
-//   node_state [2T-1][S]   u8   current state of every node
-//   meta       [E][S]      u32  m (pieces on the branch, bits 0-15) | real jumps nj (16-23) | first state (24-31)
-//   PL         [T-1][S][n] Real partial likelihoods of the internal nodes (one 16-byte vector per site for n=4 fp32)
-//   rec_len/st [chunk][S][cap_c]  merged real paths as (length Real, state u8) records, double-buffered.  A thread
-//                                 owns one (site, chunk of consecutive branches); it appends the runs of every
-//                                 branch that carries a real jump to its private slice and reads them back in the
-//                                 same order one sweep later.  cap_c comes from the Poisson tail of the chunk's
-//                                 real-jump count, so the slices are ~100x smaller than a per-branch worst case.
-//                                 Virtual jumps are never stored: they are regenerated from their Philox key.
+// The kernels of one MCMC sweep (SURVEY.md §2.3 / §8(a)).  The production arithmetic for n = 2 / 4 has kernels of its
+// own; the deterministic mode and a run-time state count run the generic ones.
+//   K1  pruning with P_e := B^(m_e - 1): replaces makePLrcpp* (src/phylomap.cpp:490-529, 1077-1088, 1938-1949) +
+//       mmmmvFORpl (:446-450).  Production: k_prune_clade (every warp walks whole subtrees alone); generic: k_prune
+//       (level by level).
+//   K2  root draw + top-down node (and hidden-tip) draws: replaces sampleinternalnodes* (:535-738, 1091-1164, 1314-1403,
+//       1952-2046) + updatenodestates (:460-475).  Production: k_nodes_clade (the same clades, pre-order); generic:
+//       k_nodes.  k_prune_nodes_clade runs production K1 and K2 in one launch (the stand-alone pair serves the DIC
+//       chains and PHYLOMAP_B200_FUSED=0).
+//   K3  per (site, branch): regenerate the virtual jumps of the previous sweep, redraw the segment states
+//       (resamplebranchstates :264-308), merge + count (shortener :44-73 / shortenerbf :997-1028), draw the new virtual
+//       jumps (:391-410), accumulate dwell times (:745-757).  Production (any n): k_paths_easy streams over every branch
+//       and completes the paths of at most one jump point, k_paths_hard takes the rest (short shapes first, then the
+//       general routine); deterministic mode: k_paths.
+//   K4  k_reduce (pm_setup_kernels.cuh): deterministic reduction of the per-block partial sums into one row.
+// Few sites on a small tree: k_small_chain (pm_small.cuh) runs whole sweeps in one block per site.
+// Data layout in HBM, and how the production and the deterministic mode encode meta and the path records: DESIGN.md §2.
 #pragma once
 #include <type_traits>
 #include "pm_device.cuh"
@@ -62,13 +58,13 @@ struct ChainParams {
   // run, ctl[1] = row of the statistics block it fills; k_reduce advances both.  nullptr: the arguments hold.
   const uint32_t* ctl;
   // production: branches left to k_paths_hard, one bit per site: hard_ballot[e * W + w] covers sites 32 w .. 32 w + 31.
-  // k_paths_hard walks them as work items of wk_g[e] consecutive words of one branch; branch e owns the items
-  // [wk_off[e], wk_off[e + 1]) (sized on the host so that an item holds ~100 set bits whatever the branch length).
+  // k_paths_hard walks them as wk_total work items, each a run of consecutive ballot words of one branch (sized on the
+  // host so that an item holds ~100 set bits whatever the branch length), flattened by k_build_items: item i = branch
+  // (bits 32-63) | first ballot word (5-31) | words - 1 (0-4), so that a warp finds its next item with ONE load, issued an
+  // item ahead
   uint32_t* hard_ballot; int W;
-  const long long* wk_off; const int* wk_g; long long wk_total;
-  const int* wk_hint;  // [wk_total / 64 + 1] branch that owns work item 64 i
-  // ... flattened (k_build_items): item i = branch (bits 32-63) | first ballot word (5-31) | words - 1 (0-4), so that a warp
-  // finds its next item with ONE load, issued an item ahead, instead of a chain of four dependent ones
+  long long wk_total;
+  long long pad0;  // unused: keeps every field below at its offset modulo 16 (see rec_cursor)
   const unsigned long long* wk_item;
   int chunk;        // branches per record chunk
   long long easy_blocks;  // blocks of k_paths_easy: k_paths_hard's dwell partials follow theirs in dw_partial
@@ -90,25 +86,17 @@ __device__ __forceinline__ void tip_partial(int code, int n, bool parity, Real* 
 
 // v <- Bs^k v
 template <typename Real, int NC, bool EXACT>
-__device__ __forceinline__ void apply_power(const ChainParams<Real>& P, const Real* sBs, const Real* sPow, int npow_s, int n,
-                                            int k, Real* v) {
+__device__ __forceinline__ void apply_power(const ChainParams<Real>& P, const Real* sBs, int n, int k, Real* v) {
   if (k <= 0) return;
-  if (!EXACT) {
-    if (k < npow_s) { matvec<Real, NC, false>(sPow + k * n * n, n, v); return; }
-    if (k < P.jcap) { matvec<Real, NC, false>(P.ppow + (size_t)k * n * n, n, v); return; }
-  }
+  if (!EXACT && k < P.jcap) { matvec<Real, NC, false>(P.ppow + (size_t)k * n * n, n, v); return; }
   for (int r = 0; r < k; r++) matvec<Real, NC, EXACT>(sBs, n, v);
 }
 
 template <typename Real>
-__device__ __forceinline__ void load_model_smem(const ChainParams<Real>& P, int n, Real* sB, Real* sBs, Real* sVec /*3n*/,
-                                                Real* sPow, int npow_s) {
+__device__ __forceinline__ void load_model_smem(const ChainParams<Real>& P, int n, Real* sB, Real* sBs, Real* sVec /*3n*/) {
   for (int i = threadIdx.x; i < n * n; i += blockDim.x) { if (sB) sB[i] = P.model[i]; sBs[i] = P.model[n * n + i]; }
   if (sVec) for (int i = threadIdx.x; i < 3 * n; i += blockDim.x) sVec[i] = P.model[2 * n * n + i];
-  for (int i = threadIdx.x; i < npow_s * n * n; i += blockDim.x) sPow[i] = P.ppow[i];
 }
-
-template <int NS, bool EXACT> __host__ __device__ constexpr int smem_pow_count() { return (!EXACT && NS > 0 && NS <= 4) ? PM_SMEM_POW : 0; }
 
 // ------------------------------------------------------------------------------------------------
 // K1: pruning.  Block = one tile of 32 sites x (blockDim/32) warps; warps stride over the nodes of a level,
@@ -120,9 +108,7 @@ __global__ void __launch_bounds__(256) k_prune(ChainParams<Real> P) {
   const int n = NS > 0 ? NS : P.n;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Real* sBs = reinterpret_cast<Real*>(smem_raw);
-  Real* sPow = sBs + n * n;
-  const int npow_s = min(smem_pow_count<NS, EXACT>(), P.jcap);
-  load_model_smem<Real>(P, n, nullptr, sBs, nullptr, sPow, npow_s);
+  load_model_smem<Real>(P, n, nullptr, sBs, nullptr);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const long long S = P.S;
@@ -142,8 +128,8 @@ __global__ void __launch_bounds__(256) k_prune(ChainParams<Real> P) {
         else VecIO<Real, NS>::load(P.PL + ((long long)(a - P.T) * S + site) * n, n, va);
         if (b < P.T) tip_partial<Real, NC>(P.tipcode[(long long)b * P.TS + site], n, parity, vb);
         else VecIO<Real, NS>::load(P.PL + ((long long)(b - P.T) * S + site) * n, n, vb);
-        apply_power<Real, NC, EXACT>(P, sBs, sPow, npow_s, n, kb, vb);
-        apply_power<Real, NC, EXACT>(P, sBs, sPow, npow_s, n, ka, va);
+        apply_power<Real, NC, EXACT>(P, sBs, n, kb, vb);
+        apply_power<Real, NC, EXACT>(P, sBs, n, ka, va);
         Real out[NC];
 #pragma unroll
         for (int j = 0; j < n; j++) out[j] = Ar<Real, EXACT>::mul(vb[j], va[j]);
@@ -532,9 +518,7 @@ __global__ void __launch_bounds__(256) k_nodes(ChainParams<Real> P, uint32_t ite
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Real* sBs = reinterpret_cast<Real*>(smem_raw);
   Real* sVec = sBs + n * n;  // pid, scale_old, scale_new
-  Real* sPow = sVec + 3 * n;
-  const int npow_s = min(smem_pow_count<NS, EXACT>(), P.jcap);
-  load_model_smem<Real>(P, n, nullptr, sBs, sVec, sPow, npow_s);
+  load_model_smem<Real>(P, n, nullptr, sBs, sVec);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const long long S = P.S;
@@ -563,7 +547,7 @@ __global__ void __launch_bounds__(256) k_nodes(ChainParams<Real> P, uint32_t ite
         Real w[NC], pl[NC];
         bool done = false;
         if (!EXACT && k > 0) {  // row ps of B^k from the table
-          const Real* M = (k < npow_s) ? (sPow + k * n * n) : (k < P.jcap ? P.ppow + (size_t)k * n * n : nullptr);
+          const Real* M = k < P.jcap ? P.ppow + (size_t)k * n * n : nullptr;
           if (M) {
 #pragma unroll
             for (int j = 0; j < n; j++) w[j] = M[ps * n + j];
@@ -595,46 +579,43 @@ template <> __device__ __forceinline__ float u01_from_word<float>(uint32_t x) { 
 template <> __device__ __forceinline__ double u01_from_word<double>(uint32_t x) { return ((double)x + 0.5) * (1.0 / 4294967296.0); }
 
 // ------------------------------------------------------------------------------------------------
-// K3: branch paths.  Thread = one site x a chunk of branches; block = 128 consecutive sites.
+// K3, deterministic mode (FP64, the reference's order of operations).  Thread = one site x a chunk of branches; block =
+// 128 consecutive sites.  Per (site, branch): regenerate the virtual jumps of the previous sweep, redraw the segment
+// states (resamplebranchstates :264-308), merge + count (shortener :44-73 / shortenerbf :997-1028), draw the new virtual
+// jumps (:391-410), accumulate dwell times (:745-757); then a block-level reduction.  meta = m | real jumps nj << 16 |
+// first state << 24, and every path keeps its nj + 1 runs as records.
 // ------------------------------------------------------------------------------------------------
-template <typename Real, int NS, bool EXACT>
-__global__ void __launch_bounds__(128) k_paths(ChainParams<Real> P, uint32_t iter, int first, int chunk) {
+template <int NS>
+__global__ void __launch_bounds__(128) k_paths(ChainParams<double> P, uint32_t iter, int first, int chunk) {
   if (P.ctl) { iter = P.ctl[0]; first = iter == 0u; }
   constexpr int NC = NS > 0 ? NS : PM_NMAX;
-  typedef typename StreamSel<Real, EXACT>::type Stream;
-  typedef ExpDev<Real, EXACT> Exp;
-  typedef Ar<Real, EXACT> A;
-  typedef Ar<Real, true> AX;  // virtual-jump arithmetic is pinned (no FMA contraction) in every mode: the sweep that
-                              // regenerates these pieces must reproduce the sweep that counted them bit for bit
-  typedef typename std::conditional<EXACT, double, Real>::type Acc;
+  typedef Ar<double, true> A;
   const int n = NS > 0 ? NS : P.n;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  double* s_dw = reinterpret_cast<double*>(smem_raw);                 // [4 warps][n] (NS>0) or [n] atomics (NS==0)
-  unsigned* s_cnt = reinterpret_cast<unsigned*>(s_dw + 4 * n);       // [n*n]
-  Real* sB = reinterpret_cast<Real*>(s_cnt + n * n + ((n * n) & 1));  // dense B (forward row)
-  Real* sBs = sB + n * n;
-  Real* sVec = sBs + n * n;
-  Real* sPow = sVec + 3 * n;
-  const int npow_s = min(smem_pow_count<NS, EXACT>(), P.jcap);
-  load_model_smem<Real>(P, n, sB, sBs, sVec, sPow, npow_s);
+  double* s_dw = reinterpret_cast<double*>(smem_raw);                     // [4 warps][n] (NS>0) or [n] atomics (NS==0)
+  unsigned* s_cnt = reinterpret_cast<unsigned*>(s_dw + 4 * n);           // [n*n]
+  double* sB = reinterpret_cast<double*>(s_cnt + n * n + ((n * n) & 1));  // dense B (forward row)
+  double* sBs = sB + n * n;
+  double* sVec = sBs + n * n;
+  load_model_smem<double>(P, n, sB, sBs, sVec);
   for (int i = threadIdx.x; i < n * n; i += blockDim.x) s_cnt[i] = 0;
   for (int i = threadIdx.x; i < 4 * n; i += blockDim.x) s_dw[i] = 0.0;
   __syncthreads();
-  const Real* s_scale_old = sVec + n;
-  const Real* s_scale_new = sVec + 2 * n;
+  const double* s_scale_old = sVec + n;
+  const double* s_scale_new = sVec + 2 * n;
   const long long S = P.S;
   const long long site = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const bool active = site < S;
   const int e0 = blockIdx.y * chunk, e1 = min(P.E, e0 + chunk);
   const int cap0 = __ldg(P.cap_off + blockIdx.y), cap_c = __ldg(P.cap_off + blockIdx.y + 1) - cap0;
   const long long abase = (long long)cap0 * S + (active ? site : 0) * (long long)cap_c;
-  const Real* __restrict__ rd_len = P.rec_len[(iter & 1u) ^ 1u] + abase;
+  const double* __restrict__ rd_len = P.rec_len[(iter & 1u) ^ 1u] + abase;
   const uint8_t* __restrict__ rd_st = P.rec_st[(iter & 1u) ^ 1u] + abase;
-  Real* __restrict__ wr_len = P.rec_len[iter & 1u] + abase;
+  double* __restrict__ wr_len = P.rec_len[iter & 1u] + abase;
   uint8_t* __restrict__ wr_st = P.rec_st[iter & 1u] + abase;
   int rd = 0, wr = 0;
   const bool full = P.full_counts != 0;
-  Acc Racc[NS > 0 ? NS : 1];
+  double Racc[NS > 0 ? NS : 1];
 #pragma unroll
   for (int j = 0; j < (NS > 0 ? NS : 1); j++) Racc[j] = 0;
   unsigned errbits = 0;
@@ -642,30 +623,27 @@ __global__ void __launch_bounds__(128) k_paths(ChainParams<Real> P, uint32_t ite
   if (active) for (int e = e0; e < e1; e++) {
     const long long pe = (long long)e * S + site;
     const uint32_t mt = P.meta[pe];
-    const int m = (int)(mt & 0xffffu), nj = (int)((mt >> 16) & 0xffu), s0 = (int)(mt >> 24);
+    const int m = (int)(mt & 0xffffu), nj = (int)((mt >> 16) & 0xffu);
     const int ps = P.node_state[(long long)__ldg(P.e_parent + e) * S + site];
     const int cs = P.node_state[(long long)__ldg(P.e_child + e) * S + site];
     int nout = 0, newm = 0, sfirst = 0;
-    Stream gnew; gnew.open(P.rng, (uint32_t)site, iter, K_BREXP, (uint32_t)e, P.err_flag);
+    StreamD gnew; gnew.open(P.rng, (uint32_t)site, iter, K_BREXP, (uint32_t)e, P.err_flag);
 
     // emit one merged run: store it, add its dwell time, draw its new virtual jumps (count only)
-    auto emit = [&](Real L, int s, bool final_run) {
+    auto emit = [&](double L, int s) {
       if (nout == 0) sfirst = s;
-      const bool skip = (!EXACT) && final_run && nout == 0;  // single-run path: length == t_e, state in meta
-      if (!skip) {
-        if (wr < cap_c && nout < PM_LOCAL_PATH_MAX) { wr_len[wr] = L; wr_st[wr] = (uint8_t)s; wr++; }
-        else errbits |= (nout >= PM_LOCAL_PATH_MAX) ? PM_DE_JUMP_LIMIT : PM_DE_PATH_CAP;
-      }
+      if (wr < cap_c && nout < PM_LOCAL_PATH_MAX) { wr_len[wr] = L; wr_st[wr] = (uint8_t)s; wr++; }
+      else errbits |= (nout >= PM_LOCAL_PATH_MAX) ? PM_DE_JUMP_LIMIT : PM_DE_PATH_CAP;
       if (NS > 0) {
 #pragma unroll
-        for (int j = 0; j < (NS > 0 ? NS : 1); j++) Racc[j] += (s == j) ? (Acc)L : (Acc)0;
-      } else atomicAdd(&s_dw[s], (double)L);
-      const Real sc = s_scale_new[s];
-      if (isfinite(sc) && sc > (Real)0) {
-        Real tot = 0;
+        for (int j = 0; j < (NS > 0 ? NS : 1); j++) Racc[j] += (s == j) ? L : 0.0;
+      } else atomicAdd(&s_dw[s], L);
+      const double sc = s_scale_new[s];
+      if (isfinite(sc) && sc > 0.0) {
+        double tot = 0;
         for (;;) {
-          const Real g = AX::mul(sc, Exp::draw(gnew));
-          const Real t2 = AX::add(tot, g);
+          const double g = A::mul(sc, exp_rand_R(gnew));
+          const double t2 = A::add(tot, g);
           if (t2 < L) { tot = t2; newm++; if (newm > 70000) break; } else break;
         }
       }
@@ -673,74 +651,65 @@ __global__ void __launch_bounds__(128) k_paths(ChainParams<Real> P, uint32_t ite
       nout++;
     };
 
-    if (!EXACT && !first && nj == 0 && (m == 1 || (m == 2 && ps == cs))) {
-      if (full && m == 2) atomicAdd(&s_cnt[ps * n + cs], 1u);
-      emit(__ldg(P.e_len + e), cs, true);
-    } else {
-      Real in_len[PM_LOCAL_PATH_MAX]; uint8_t in_st[PM_LOCAL_PATH_MAX];
-      int nin = 0;
-      if (!first) {
-        if (!EXACT && nj == 0) { nin = 1; in_len[0] = __ldg(P.e_len + e); in_st[0] = (uint8_t)s0; }
-        else {
-          nin = min(nj + 1, PM_LOCAL_PATH_MAX);
-          for (int c = 0; c < nin; c++) { const int q = min(rd + c, cap_c - 1); in_len[c] = rd_len[q]; in_st[c] = rd_st[q]; }
-          rd += nj + 1;
-        }
-      }
-      Stream gold;  // the stream that drew the virtual jumps of the previous sweep (none before the first one)
-      gold.open(P.rng, (uint32_t)site, first ? iter : iter - 1u, K_BREXP, (uint32_t)e, P.err_flag);
-      Stream gst; gst.open(P.rng, (uint32_t)site, iter, K_BRSTATE, (uint32_t)e, P.err_flag);
-      int j = 0; Real tot = 0; long long cp = first ? P.maps_off[e] : 0;
-      auto next_piece = [&]() -> Real {
-        if (first) return (Real)P.maps_len[cp++];
-        if (j >= nin) { errbits |= PM_DE_INCONSISTENT; return (Real)0; }
-        const Real L = in_len[j];
-        const Real sc = s_scale_old[in_st[j]];
-        if (isfinite(sc) && sc > (Real)0) {
-          const Real g = AX::mul(sc, Exp::draw(gold));
-          const Real t2 = AX::add(tot, g);
-          if (t2 < L) { tot = t2; return g; }
-        }
-        const Real r = AX::sub(L, tot);
-        j++; tot = 0;
-        return r;
-      };
-      int cur_state = (m == 1) ? cs : ps;
-      Real cur_len = next_piece();
-      int prev = cur_state;
-      for (int p = 1; p < m; p++) {
-        int st;
-        if (p == m - 1) st = cs;
-        else {
-          const int jd = m - p - 1;  // beta_jd = Bs^jd e_cs
-          Real w[NC];
-          const Real* M = (jd < npow_s) ? (sPow + jd * n * n) : (jd < P.jcap ? P.ppow + (size_t)jd * n * n : nullptr);
-          if (M) {
-#pragma unroll
-            for (int c = 0; c < n; c++) w[c] = M[c * n + cs];
-          } else {
-#pragma unroll
-            for (int c = 0; c < n; c++) w[c] = (Real)(c == cs);
-            for (int r = 0; r < jd; r++) matvec<Real, NC, EXACT>(sBs, n, w);
-          }
-#pragma unroll
-          for (int c = 0; c < n; c++) w[c] = A::mul(sB[prev * n + c], w[c]);
-          st = categorical<Real, NC, EXACT>(w, n, gst.next(), P.err_flag);
-        }
-        const Real len = next_piece();
-        if (full) atomicAdd(&s_cnt[prev * n + st], 1u);
-        if (st == cur_state) cur_len = A::add(cur_len, len);
-        else {
-          emit(cur_len, cur_state, false);
-          if (!full) atomicAdd(&s_cnt[cur_state * n + st], 1u);
-          cur_state = st; cur_len = len;
-        }
-        prev = st;
-      }
-      // production: a single-run path is not stored, the next sweep takes its length from the tree
-      if (!EXACT && nout == 0) cur_len = __ldg(P.e_len + e);
-      emit(cur_len, cur_state, true);
+    double in_len[PM_LOCAL_PATH_MAX]; uint8_t in_st[PM_LOCAL_PATH_MAX];
+    int nin = 0;
+    if (!first) {
+      nin = min(nj + 1, PM_LOCAL_PATH_MAX);
+      for (int c = 0; c < nin; c++) { const int q = min(rd + c, cap_c - 1); in_len[c] = rd_len[q]; in_st[c] = rd_st[q]; }
+      rd += nj + 1;
     }
+    StreamD gold;  // the stream that drew the virtual jumps of the previous sweep (none before the first one)
+    gold.open(P.rng, (uint32_t)site, first ? iter : iter - 1u, K_BREXP, (uint32_t)e, P.err_flag);
+    StreamD gst; gst.open(P.rng, (uint32_t)site, iter, K_BRSTATE, (uint32_t)e, P.err_flag);
+    int j = 0; double tot = 0; long long cp = first ? P.maps_off[e] : 0;
+    auto next_piece = [&]() -> double {
+      if (first) return P.maps_len[cp++];
+      if (j >= nin) { errbits |= PM_DE_INCONSISTENT; return 0.0; }
+      const double L = in_len[j];
+      const double sc = s_scale_old[in_st[j]];
+      if (isfinite(sc) && sc > 0.0) {
+        const double g = A::mul(sc, exp_rand_R(gold));
+        const double t2 = A::add(tot, g);
+        if (t2 < L) { tot = t2; return g; }
+      }
+      const double r = A::sub(L, tot);
+      j++; tot = 0;
+      return r;
+    };
+    int cur_state = (m == 1) ? cs : ps;
+    double cur_len = next_piece();
+    int prev = cur_state;
+    for (int p = 1; p < m; p++) {
+      int st;
+      if (p == m - 1) st = cs;
+      else {
+        const int jd = m - p - 1;  // beta_jd = Bs^jd e_cs: column cs of the host's power table (built bit for bit as the
+                                   // reference's backward vectors), repeated mat-vecs beyond it
+        double w[NC];
+        if (jd < P.jcap) {
+          const double* M = P.ppow + (size_t)jd * n * n;
+#pragma unroll
+          for (int c = 0; c < n; c++) w[c] = M[c * n + cs];
+        } else {
+#pragma unroll
+          for (int c = 0; c < n; c++) w[c] = (double)(c == cs);
+          for (int r = 0; r < jd; r++) matvec<double, NC, true>(sBs, n, w);
+        }
+#pragma unroll
+        for (int c = 0; c < n; c++) w[c] = A::mul(sB[prev * n + c], w[c]);
+        st = categorical<double, NC, true>(w, n, gst.next(), P.err_flag);
+      }
+      const double len = next_piece();
+      if (full) atomicAdd(&s_cnt[prev * n + st], 1u);
+      if (st == cur_state) cur_len = A::add(cur_len, len);
+      else {
+        emit(cur_len, cur_state);
+        if (!full) atomicAdd(&s_cnt[cur_state * n + st], 1u);
+        cur_state = st; cur_len = len;
+      }
+      prev = st;
+    }
+    emit(cur_len, cur_state);
     if (newm > 65535) { errbits |= PM_DE_M_OVERFLOW; newm = 65535; }
     if (nout > PM_LOCAL_PATH_MAX) nout = PM_LOCAL_PATH_MAX;  // flagged in emit
     P.meta[pe] = (uint32_t)newm | ((uint32_t)(nout - 1) << 16) | ((uint32_t)sfirst << 24);
@@ -752,7 +721,7 @@ __global__ void __launch_bounds__(128) k_paths(ChainParams<Real> P, uint32_t ite
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
     for (int j = 0; j < (NS > 0 ? NS : 1); j++) {
-      double v = (double)Racc[j];
+      double v = Racc[j];
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
       if (lane == 0) s_dw[warp * n + j] = v;
@@ -861,7 +830,8 @@ __device__ __forceinline__ void nodes_clade_block(const ChainParams<Real>& P, co
   Real* sVec = sBs + NS * NS;  // pid, scale_old, scale_new
   Real* sPow = sVec + 3 * NS;
   const int npow_s = min(PM_SMEM_POW, P.jcap);
-  load_model_smem<Real>(P, NS, nullptr, sBs, sVec, sPow, npow_s);
+  load_model_smem<Real>(P, NS, nullptr, sBs, sVec);
+  for (int i = threadIdx.x; i < npow_s * NS * NS; i += blockDim.x) sPow[i] = P.ppow[i];
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const long long S = P.S;
@@ -1839,7 +1809,6 @@ struct PathWorker {
 template <typename Real, int NS, int MINB, int WHICH>
 __global__ void __launch_bounds__(128, MINB) k_paths_hard(ChainParams<Real> P, uint32_t iter, int first) {
   if (P.ctl) { iter = P.ctl[0]; first = iter == 0u; }
-  constexpr int NC = NS > 0 ? NS : PM_NMAX;
   constexpr int NR = NS > 0 ? NS : 1;
   typedef typename StreamSel<Real, false>::type Stream;
   typedef Pin<Real> PN;
@@ -1851,7 +1820,7 @@ __global__ void __launch_bounds__(128, MINB) k_paths_hard(ChainParams<Real> P, u
   Real* sBs = sB + n * n;
   Real* sVec = sBs + n * n;  // pid | scale_old | scale_new | rate_old | rate_new
   Real* sPow = sVec + 5 * n;
-  const int npow_s = min(smem_pow_count<NS, false>(), P.jcap);
+  const int npow_s = min(NS > 0 ? PM_SMEM_POW : 0, P.jcap);  // the first powers of B in shared memory (n = 2, 4)
   for (int i = threadIdx.x; i < n * n; i += blockDim.x) { sB[i] = P.model[i]; sBs[i] = P.model[n * n + i]; s_cnt[i] = 0; }
   for (int i = threadIdx.x; i < 5 * n; i += blockDim.x) sVec[i] = P.model[2 * n * n + i];
   for (int i = threadIdx.x; i < npow_s * n * n; i += blockDim.x) sPow[i] = P.ppow[i];

@@ -67,7 +67,7 @@ void Sweep<Real, NS, EXACT>::prune_nodes(const ChainParams<Real>& P, int grid, s
 template <typename Real, int NS, bool EXACT>
 void Sweep<Real, NS, EXACT>::paths(const ChainParams<Real>& P, dim3 grid, size_t smem, cudaStream_t st, uint32_t iter,
                                    int first, int chunk, int hard_blocks) {
-  if constexpr (EXACT) k_paths<Real, NS, true><<<grid, 128, smem, st>>>(P, iter, first, chunk);
+  if constexpr (EXACT) k_paths<NS><<<grid, 128, smem, st>>>(P, iter, first, chunk);
   else {
     // the easy kernel also serves the first sweep: a map of one or two pieces is a path like any other (pos1 was
     // seeded from it), only longer maps are walked piece by piece by the general kernel

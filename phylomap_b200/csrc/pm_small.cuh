@@ -29,9 +29,6 @@ struct SmallOut {
   // ONE site: the block writes the rows itself, in k_reduce's layout [R(n) | N(n*n) | root | .. | error flag] (device
   // memory or mapped host memory: a rate-updating sampler reads the row right after the launch); nullptr: part / cnt / root
   double* rows; int row_stride, err_slot;
-  // PHYLOMAP_B200_SMALL_PROF=1: clock cycles block 0 spends in [prune, node draws, paths (until the slowest warp is through),
-  // row] summed over the sweeps, and the per-warp cycles of the path phase [4 + warp] (nullptr: nothing is measured)
-  long long* prof;
 };
 
 // shared-memory layout (bytes, every section 16-byte aligned)
@@ -161,11 +158,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
     for (int ck = tid; ck < out.n_chunks; ck += nthr) P.rec_cursor[(long long)ck * P.rec_groups + (site >> P.rec_shift)] = 0;
     for (int i = tid; i < n * n; i += nthr) s_cnt[i] = 0;
 
-    long long tk = 0;
-    if (out.prof && blockIdx.x == 0) tk = clock64();
-    auto lap = [&](int slot) {  // (after a barrier)
-      if (out.prof && blockIdx.x == 0) { const long long t2 = clock64(); if (tid == 0) out.prof[slot] += t2 - tk; tk = t2; }
-    };
     // ---- K1: pruning, level by level, one node per thread (makePLrcpp_bigtree :503-529) ----
     auto prune_node = [&](int pn, int a, int ea, int b, int eb) {
       const int ka = (int)(sMeta[ea] & 0xffffu) - 1, kb = (int)(sMeta[eb] & 0xffffu) - 1;
@@ -194,7 +186,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
       }
     }
 
-    lap(0);
     // ---- K2: root (:618-627), then the nodes top-down by depth, redrawn tips at their depth (sampleinternalnodes* :591) ----
     if (tid == 0) {
       Real w[NS], pl[NS];
@@ -238,7 +229,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
       }
     }
 
-    lap(1);
     // ---- K3: one branch per thread.  At most one jump point and count mode: the body of k_paths_easy; everything else:
     // the general item routine of k_paths_hard (which also reproduces what its short routine computes) ----
     PathWorker<Real, NS> pw(P, iter, first, n, sB, sBs, sPow, npow_s, s_cnt, s_dw, s_rate_old, s_rate_new);
@@ -280,7 +270,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
       }
     }
     if (pw.errbits) atomicOr(P.err_flag, pw.errbits);
-    if (out.prof && blockIdx.x == 0 && lane == 0) out.prof[4 + warp] += clock64() - tk;
 
     // ---- K4: this site's share of the sweep's row ----
 #pragma unroll
@@ -291,7 +280,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
       if (lane == 0) s_dw[warp * n + j] = v;
     }
     __syncthreads();
-    lap(2);
     if (out.rows) {  // one site: the row of this sweep is complete here
       double* const row = out.rows + (size_t)sw * out.row_stride;
       if (tid < n) {
@@ -313,7 +301,6 @@ __global__ void __launch_bounds__(256, MINB) k_small_chain(ChainParams<Real> P, 
       for (int i = tid; i < n * n; i += nthr) if (s_cnt[i]) atomicAdd(&out.cnt[(long long)sw * n * n + i], (unsigned long long)s_cnt[i]);
     }
     __syncthreads();
-    lap(3);
   }
 
   // ---- the state goes back to where the other kernels (and export / read-back) expect it ----
