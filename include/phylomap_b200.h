@@ -18,6 +18,7 @@
  *   pm_maketreelistMCMC2sDICt   <- maketreelistMCMC2sDICt   src/phylomap.cpp:3183 (src/RcppExports.cpp:211)
  *   pm_maketreelistMCMCksDICt   <- maketreelistMCMCksDICt   src/phylomap.cpp:3300 (src/RcppExports.cpp:237)
  *   pm_loglik                   <- the pruning loop of make2stateDIC / make4stateDIC(big), R/sourceme.R:141-177, 248-284, 445-516
+ *   pm_expected_sumstats        (no counterpart: the exact posterior expectations the fixed-Q samplers estimate)
  *   pm_tree_order               <- pruningwiseedgeorder / makenodelist / myreorder, R/sumstatMCMC.R:1-18 (O(E) here)
  *
  * There is no CPU fallback: every entry fails with PM_ERR_CUDA when no sm_100 device is usable.
@@ -162,6 +163,23 @@ int pm_maketreelistMCMCksDICt(const pm_tree* x, int32_t n, double* Q, const doub
  * of make4stateDIC (:264-267); 0: one-hot tips.  Q column-major n x n, n <= 8; not modified. */
 int pm_loglik(const pm_tree* x, int32_t n, const double* Q, const double* pid, int32_t parity_tips, const pm_options* opt,
               double* out, char* err, size_t errlen);
+
+/* Exact posterior expectations under a fixed Q (no sampling, no random numbers): for every site, the expected dwell
+ * times and transition counts given the tip data, in the fixed-Q sampler row layout (n + n(n-1) columns), and log p(y|Q);
+ * for the selected LOCAL sites also per branch (edge-row order) and the marginal state probabilities of every node.
+ *   stats          column-major [S x (n + n(n-1))] or NULL
+ *   loglik         [S] or NULL
+ *   branch_stats   [nsel][E][n + n(n-1)] or NULL        node_marginals  [nsel][2T-1][n] or NULL (0-based node ids)
+ * parity_tips as in pm_loglik; Q column-major n x n, 2 <= n <= 8; not modified.  Branch lengths as in
+ * pm_loglik (edge_length, or the sums of maps when it is NULL).  Sites may repeat and come in any order.  The simulation-free
+ * stochastic mapping of Minin & Suchard (2008): branch integrals by Van Loan's block exponential, an inside and an
+ * outside pruning pass on the device, in tiles of sites that change no output bit.  pm_options.precision and .device
+ * apply; mode, seed and the collective options have no effect.  PM_ERR_ARG before any device work for a null tree, Q or
+ * pid, n out of range, parity tips with an odd n or a site out of range; PM_ERR_SAMPLE when a site's data have zero
+ * likelihood under Q (in FP32 also when its products underflow). */
+int pm_expected_sumstats(const pm_tree* x, int32_t n, const double* Q, const double* pid, int32_t parity_tips,
+                         const int64_t* sites, int64_t nsel, const pm_options* opt, double* stats, double* loglik,
+                         double* branch_stats, double* node_marginals, char* err, size_t errlen);
 
 /* The direct sampler with matrix exponentiation, maketreelistEXP (src/phylomap.cpp:3001, src/RcppExports.cpp:80): N
  * INDEPENDENT histories per site.  lefts / rights / d: eigenvectors, their inverse and diag(eigenvalues) of Q, column-major

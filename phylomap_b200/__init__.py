@@ -4,7 +4,7 @@ Only the hot path lives here: the CUDA kernels and C ABI (csrc/, include/phyloma
 (capi), the host-side mirror of the reference's R functions (api), and synthetic-input generators (synth).
 """
 from . import capi  # noqa: F401
-from .api import (Chain, SPARSEmaketreelistMCMC, SPARSEsumstatMCMC, colnames, loglik, make2stateDIC, make2stateDICbig, make4stateDIC,  # noqa: F401
+from .api import (Chain, ExpectedSumstats, SPARSEmaketreelistMCMC, SPARSEsumstatMCMC, colnames, expected_sumstats, loglik, make2stateDIC, make2stateDICbig, make4stateDIC,  # noqa: F401
                   make4stateDICbig, makenodelist, maketreelistEXP, maketreelistMCMC,  # noqa: F401
                   maketreelistMCMC2sDICt, maketreelistMCMC_bigtree, maketreelistMCMCbf, maketreelistMCMCks,
                   maketreelistMCMCksDICt, maketreelistMCMCksmt, maketreelistMCMCmt, myreorder, pruningwiseedgeorder,

@@ -451,6 +451,59 @@ def loglik(z, Q, pid, parity_tips=False, order=None, **opts):
     return float(out.value)
 
 
+class ExpectedSumstats:
+    """Exact posterior expectations under a fixed Q (`expected_sumstats`).  Columns of a statistic follow the fixed-Q
+    sampler rows: n dwell times, then the n(n-1) changes i -> j, row-major with the diagonal skipped.
+        stats           [S, n^2]           per site
+        loglik          [S]                log p(y_s | Q)
+        sites           [k]                the selected local sites
+        branch_stats    [k, E, n^2]        per selected site and branch (edge-row order)
+        node_marginals  [k, 2T-1, n]       P(X_v = s | y), 0-based node ids (tips 0..T-1)"""
+
+    def __init__(self, n, stats, loglik, sites, branch_stats, node_marginals):
+        self.n, self.stats, self.loglik, self.sites = n, stats, loglik, sites
+        self.branch_stats, self.node_marginals = branch_stats, node_marginals
+
+    def mapped_edge(self):
+        """[k, E, n]: expected time in each state on each branch (the mean of `StochasticMaps.mapped_edge()`)."""
+        return self.branch_stats[:, :, :self.n]
+
+    def transitions(self):
+        """[k, n, n]: expected number of changes a -> b summed over the branches (the mean of `StochasticMaps.transitions()`)."""
+        n = self.n
+        tot = self.branch_stats[:, :, n:].sum(axis=1)
+        out = np.zeros((len(self.sites), n, n))
+        off = np.ones((n, n), dtype=bool)
+        np.fill_diagonal(off, False)
+        out[:, off] = tot
+        return out
+
+
+def expected_sumstats(z, Q, pid, parity_tips=False, sites=None, order=None, **opts):
+    """Exact posterior expected dwell times and transition counts of every site of `z` given its tip data under a fixed Q,
+    and log p(y_s | Q) per site (pm_expected_sumstats): no sampling.  For the local `sites` (repeats and any order allowed)
+    also per branch and the marginal state probabilities of every node.  Returns an `ExpectedSumstats`."""
+    L = capi.lib()
+    z = PhyloTree.from_mapping(z)
+    n = np.asarray(Q).shape[0]
+    Qf = np.asfortranarray(np.asarray(Q, dtype=np.float64))
+    pidc = np.ascontiguousarray(pid, dtype=np.float64)
+    tree, keep = z.flat(*(order if order is not None else (None, None, None)))
+    opt, keep2 = _options(**opts)
+    S, E, NK = z.n_sites(), z.E, n * n
+    sel = np.zeros(0, dtype=np.int64) if sites is None else np.ascontiguousarray(sites, dtype=np.int64).reshape(-1)
+    stats = np.zeros((S, NK), dtype=np.float64, order="F")
+    ll = np.zeros(S, dtype=np.float64)
+    bs = np.zeros((len(sel), E, NK), dtype=np.float64)
+    nm = np.zeros((len(sel), 2 * z.T - 1, n), dtype=np.float64)
+    err = C.create_string_buffer(512)
+    rc = L.pm_expected_sumstats(C.byref(tree), n, capi.ptr(Qf), capi.ptr(pidc), int(bool(parity_tips)), capi.ptr(sel), len(sel),
+                                C.byref(opt), capi.ptr(stats), capi.ptr(ll), capi.ptr(bs) if len(sel) else None,
+                                capi.ptr(nm) if len(sel) else None, err, 512)
+    capi.check(rc, err)
+    return ExpectedSumstats(n, stats, ll, sel, bs, nm)
+
+
 def _col(mat, name, pos):
     """Column of a sampler output by the reference's name (a pandas frame) or by its position (a plain matrix)."""
     if hasattr(mat, "columns"):

@@ -39,7 +39,7 @@ class PmOptions(C.Structure):
 
 EXPORTS = ["pm_default_options", "pm_nccl_unique_id", "pm_maketreelistMCMC", "pm_SPARSEmaketreelistMCMC", "pm_maketreelistMCMC_bigtree",
            "pm_maketreelistMCMCbf", "pm_maketreelistMCMCks", "pm_maketreelistMCMCmt", "pm_maketreelistMCMCksmt",
-           "pm_maketreelistMCMC2sDICt", "pm_maketreelistMCMCksDICt", "pm_maketreelistEXP", "pm_loglik",
+           "pm_maketreelistMCMC2sDICt", "pm_maketreelistMCMCksDICt", "pm_maketreelistEXP", "pm_loglik", "pm_expected_sumstats",
            "pm_ncols", "pm_tree_order", "pm_debug_clade_schedule", "pm_chain_create", "pm_chain_run", "pm_chain_state_bytes",
            "pm_chain_export_state", "pm_chain_import_state", "pm_chain_time_prune",
            "pm_chain_kernel_times", "pm_chain_enable_timing", "pm_chain_overheads", "pm_chain_get_node_states", "pm_chain_get_piece_counts",
@@ -78,6 +78,7 @@ def lib():
         getattr(L, f).argtypes = multi
     L.pm_maketreelistEXP.argtypes = [vp, i32, vp, vp, i32, vp, vp, vp, vp, vp, C.c_char_p, C.c_size_t]
     L.pm_loglik.argtypes = [vp, i32, vp, vp, i32, vp, vp, C.c_char_p, C.c_size_t]
+    L.pm_expected_sumstats.argtypes = [vp, i32, vp, vp, i32, vp, i64, vp, vp, vp, vp, vp, C.c_char_p, C.c_size_t]
     L.pm_ncols.argtypes = [i32, i32]
     L.pm_tree_order.argtypes = [vp, i32, i32, vp, vp, vp, C.c_char_p, C.c_size_t]
     L.pm_debug_clade_schedule.argtypes = [vp, i32, i32, vp, vp, i32, i32, i32, vp, C.c_char_p, C.c_size_t]

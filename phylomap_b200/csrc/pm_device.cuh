@@ -23,6 +23,7 @@
 #define PM_DE_INCONSISTENT 64u
 #define PM_DE_BAD_STATE 128u
 #define PM_DE_JUMP_LIMIT 256u  // deterministic mode: more real jumps on one branch than a path can hold (63)
+#define PM_DE_ZERO_LIK 512u    // pm_expected_sumstats: a site whose data have zero (or, in FP32, underflowed) likelihood
 
 namespace pm {
 

@@ -29,6 +29,7 @@
 #include "pm_launch.cuh"
 #include "pm_setup_kernels.cuh"
 #include "pm_loglik.cuh"
+#include "pm_expect.cuh"
 #include "pm_maps.cuh"
 #include "pm_exp.cuh"
 #include "pm_nccl.hpp"
@@ -320,6 +321,7 @@ struct pm_chain {
   virtual void maps(int tree, const int64_t* sites, int64_t nsel, int64_t* off, double* len, int32_t* st, int64_t cap) = 0;
   virtual void partials(int tree, int64_t site, double* out) = 0;
   virtual double loglik() = 0;
+  virtual void expected(bool write, double* stats, int64_t ld, double* loglik, double* branch_stats, double* node_marginals) = 0;
   virtual int64_t state_bytes() = 0;
   virtual void export_state(void* buf, int64_t bytes) = 0;
   virtual void import_state(const void* buf, int64_t bytes) = 0;
@@ -811,7 +813,7 @@ struct ChainT : pm_chain {
                                                               t.TP.template as<Real>());
     const int gx = (int)((t.S + 31) / 32);
     with_ns([&](auto ns) {
-      pm::k_loglik<Real, decltype(ns)::value><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>());
+      pm::k_loglik<Real, decltype(ns)::value><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>(), nullptr);
     });
     pm::k_reduce_ll<<<1, 256, 0, stream>>>(t.ll_partial.template as<double>(), gx, row + n + n * n + 1);
     launches += 3;
@@ -889,6 +891,10 @@ struct ChainT : pm_chain {
                             "per path (the production arithmetic has no such limit)");
     if (f & PM_DE_PATH_CAP) fail(PM_ERR_CAPACITY, "the run records of a branch chunk overflowed; raise pm_options.path_capacity");
     if (f & PM_DE_M_OVERFLOW) fail(PM_ERR_CAPACITY, "more than 65535 pieces on one branch");
+    if (f & PM_DE_ZERO_LIK)
+      fail(PM_ERR_SAMPLE, opt.precision == PM_F32 ? "the tip data of a site have zero likelihood under Q, or FP32 products underflowed "
+                                                      "(precision f64 has the wider range): no posterior expectation exists"
+                                                    : "the tip data of a site have zero likelihood under Q: no posterior expectation exists");
     fail(PM_ERR_CUDA, "inconsistent chain state (device flag %u)", f);
   }
 
@@ -1347,7 +1353,7 @@ struct ChainT : pm_chain {
     with_ns([&](auto ns) {
       constexpr int NSc = decltype(ns)::value;
       begin_timed(0);
-      pm::k_loglik<Real, NSc><<<gx, 256, 0, stream>>>(t.P, TP, llp);
+      pm::k_loglik<Real, NSc><<<gx, 256, 0, stream>>>(t.P, TP, llp, nullptr);
       end_timed();
       begin_timed(1);
       pm::k_exp_nodes<Real, NSc><<<gx, 256, 0, stream>>>(t.P, TP, iter);
@@ -1758,6 +1764,62 @@ struct ChainT : pm_chain {
     check_device_errors();
     return rows_h[0];
   }
+  // Exact posterior expectations of this log-likelihood chain's sites (pm_expected_sumstats): branch integrals, the inside
+  // pass with its per-site log-likelihoods, the outside pass.  stats: column-major, leading dimension ld; write: the
+  // per-branch statistics and node marginals of every site too.  With PHYLOMAP_B200_TRACE=1 the three kernels' CUDA-event
+  // times go to stderr.
+  void expected(bool write, double* stats, int64_t ld, double* ll, double* branch_stats, double* node_marginals) override {
+    if (!V.llonly) fail(PM_ERR_ARG, "posterior expectations are computed by a log-likelihood chain");
+    CK(cudaSetDevice(opt.device));
+    TreeDev<Real>& t = *trees[0];
+    const int E = t.sch.E, T = t.sch.T, NK = n * n;
+    const long long S = t.S;
+    for (int i = 0; i < n; i++) for (int j = 0; j < n; j++) q_h[(size_t)i * n + j] = Q[i + (size_t)j * n];
+    CK(cudaMemcpyAsync(q_dev.p, q_h, (size_t)n * n * sizeof(double), cudaMemcpyHostToDevice, stream));
+    DevBuf M, site_ll, st_d, br_d, nd_d;
+    M.alloc((size_t)E * NK * NK * sizeof(Real));
+    site_ll.alloc((size_t)S * sizeof(double));
+    st_d.alloc((size_t)NK * S * sizeof(double));
+    if (write) { br_d.alloc((size_t)S * E * NK * sizeof(double)); nd_d.alloc((size_t)S * (2 * T - 1) * n * sizeof(double)); }
+    cudaEvent_t ev[4] = {};
+    struct Events { cudaEvent_t* e; ~Events() { for (int i = 0; i < 4; i++) if (e[i]) cudaEventDestroy(e[i]); } } ev_guard{ev};
+    if (sw.trace) for (int i = 0; i < 4; i++) CK(cudaEventCreate(&ev[i]));
+    const auto mark = [&](int i) { if (sw.trace) CK(cudaEventRecord(ev[i], stream)); };
+    const int gx = (int)((S + 31) / 32);
+    const size_t smem = (size_t)8 * NK * 32 * sizeof(double);
+    mark(0);
+    pm::k_transprob<Real><<<(E + 127) / 128, 128, 0, stream>>>(q_dev.as<double>(), t.e_len_d.template as<double>(), E, n, t.TP.template as<Real>());
+    pm::k_branch_integrals<Real><<<(unsigned)(((long long)E * NK + 127) / 128), 128, 0, stream>>>(q_dev.as<double>(), t.e_len_d.template as<double>(),
+                                                                                              E, n, M.as<Real>());
+    mark(1);
+    with_ns([&](auto ns) {
+      constexpr int NSc = decltype(ns)::value;
+      pm::k_loglik<Real, NSc><<<gx, 256, 0, stream>>>(t.P, t.TP.template as<Real>(), t.ll_partial.template as<double>(), site_ll.as<double>());
+      mark(2);
+      const auto launch = [&](auto kern) {
+        CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<gx, 256, smem, stream>>>(t.P, t.TP.template as<Real>(), M.as<Real>(), st_d.as<double>(), br_d.as<double>(), nd_d.as<double>());
+      };
+      if (write) launch(pm::k_expect<Real, NSc, true>);
+      else launch(pm::k_expect<Real, NSc, false>);
+    });
+    mark(3);
+    CK(cudaGetLastError());
+    launches += 4;
+    if (stats)
+      CK(cudaMemcpy2DAsync(stats, (size_t)ld * sizeof(double), st_d.p, (size_t)S * sizeof(double), (size_t)S * sizeof(double), NK,
+                           cudaMemcpyDeviceToHost, stream));
+    if (ll) CK(cudaMemcpyAsync(ll, site_ll.p, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, stream));
+    if (write && branch_stats) CK(cudaMemcpyAsync(branch_stats, br_d.p, br_d.bytes, cudaMemcpyDeviceToHost, stream));
+    if (write && node_marginals) CK(cudaMemcpyAsync(node_marginals, nd_d.p, nd_d.bytes, cudaMemcpyDeviceToHost, stream));
+    check_device_errors();
+    if (sw.trace) {
+      float ms[3] = {0, 0, 0};
+      for (int i = 0; i < 3; i++) CK(cudaEventElapsedTime(&ms[i], ev[i], ev[i + 1]));
+      fprintf(stderr, "[phylomap_b200] expect: %lld sites%s: P(t) + branch integrals %.4f ms, inside %.4f ms, outside %.4f ms\n", S,
+              write ? " (selected)" : "", ms[0], ms[1], ms[2]);
+    }
+  }
   // partials of the current state: a pruning pass over the site's block (into slot 0 of the fused kernel's partials) or
   // over all sites, then the site's column
   void partials(int tree, int64_t site, double* out) override {
@@ -1873,6 +1935,31 @@ int one_call(int variant, const pm_tree* trees, int ntrees, int n, double* Q, co
   });
 }
 
+// A chain that evaluates log p(y | Q) and keeps no path state (pm_loglik, pm_expected_sumstats), with the copy of Q it reads.
+// The chain machinery wants a uniformization pair (Omega, B) although neither computation uses it.
+struct LoglikChain {
+  std::vector<double> q, b;
+  std::unique_ptr<pm_chain> c;
+  LoglikChain(const pm_tree* x, int n, const double* Q, const double* pid, int parity_tips, const pm_options* opt)
+      : q(Q, Q + (size_t)n * n), b((size_t)n * n, 0.0) {
+    double om = 0;
+    for (int i = 0; i < n; i++) om = std::max(om, 2 * std::fabs(q[i + (size_t)i * n]));
+    if (!(om > 0)) om = 1;
+    for (int i = 0; i < n; i++) for (int j = 0; j < n; j++) b[i + (size_t)j * n] = (i == j ? 1.0 : 0.0) + q[i + (size_t)j * n] / om;
+    c.reset(make_chain(parity_tips ? V_LOGLIK_PARITY : V_LOGLIK, x, 1, n, q.data(), pid, b.data(), om, nullptr, 0, 0, opt, nullptr, true));
+  }
+};
+
+// pm_expected_sumstats over sites [s0, s0 + count) of x (write: per branch and per node too).
+void expected_block(const pm_tree* x, int n, const double* Q, const double* pid, int parity_tips, const pm_options* opt, long long s0,
+                    long long count, bool write, double* stats, long long ld, double* ll, double* branch_stats, double* node_marginals) {
+  pm_tree t = *x;
+  t.n_sites = count;
+  if (x->states_u8) t.states_u8 = x->states_u8 + s0 * (long long)x->n_tips;
+  if (x->states) t.states = x->states + s0 * (long long)x->n_tips;
+  LoglikChain(&t, n, Q, pid, parity_tips, opt).c->expected(write, stats, ld, ll, branch_stats, node_marginals);
+}
+
 }  // namespace
 
 // ----------------------------------------------------------------------------------------------------------------
@@ -1944,15 +2031,70 @@ int pm_loglik(const pm_tree* x, int32_t n, const double* Q, const double* pid, i
     if (!x || !Q || !pid || !out) fail(PM_ERR_ARG, "null argument");
     if (n < 2 || n > PM_DIC_NMAX) fail(PM_ERR_ARG, "number of states must be in 2..%d", PM_DIC_NMAX);
     if (parity_tips && (n & 1)) fail(PM_ERR_ARG, "parity tip partials need an even number of states");
-    // the chain machinery wants a uniformization pair (Omega, B) although the likelihood does not use it
-    std::vector<double> q(Q, Q + (size_t)n * n), b((size_t)n * n, 0.0);
-    double om = 0;
-    for (int i = 0; i < n; i++) om = std::max(om, 2 * std::fabs(q[i + (size_t)i * n]));
-    if (!(om > 0)) om = 1;
-    for (int i = 0; i < n; i++) for (int j = 0; j < n; j++) b[i + (size_t)j * n] = (i == j ? 1.0 : 0.0) + q[i + (size_t)j * n] / om;
-    std::unique_ptr<pm_chain> c(make_chain(parity_tips ? V_LOGLIK_PARITY : V_LOGLIK, x, 1, n, q.data(), pid, b.data(), om, nullptr, 0, 0,
-                                           opt, nullptr, true));
-    *out = c->loglik();
+    *out = LoglikChain(x, n, Q, pid, parity_tips, opt).c->loglik();
+  });
+}
+
+int pm_expected_sumstats(const pm_tree* x, int32_t n, const double* Q, const double* pid, int32_t parity_tips, const int64_t* sites,
+                         int64_t nsel, const pm_options* opt, double* stats, double* loglik, double* branch_stats, double* node_marginals,
+                         char* err, size_t errlen) {
+  return guarded(err, errlen, [&] {
+    if (!x || !Q || !pid) fail(PM_ERR_ARG, "null argument");
+    if (n < 2 || n > PM_DIC_NMAX) fail(PM_ERR_ARG, "number of states must be in 2..%d", PM_DIC_NMAX);
+    if (parity_tips && (n & 1)) fail(PM_ERR_ARG, "parity tip partials need an even number of states");
+    if (x->n_sites < 1) fail(PM_ERR_ARG, "n_sites must be >= 1");
+    if (!x->states && !x->states_u8) fail(PM_ERR_ARG, "states missing");
+    if (nsel < 0 || (nsel > 0 && !sites)) fail(PM_ERR_ARG, "bad site selection");
+    for (int64_t i = 0; i < nsel; i++)
+      if (sites[i] < 0 || sites[i] >= x->n_sites) fail(PM_ERR_ARG, "site %lld out of range (%lld sites)", (long long)sites[i], (long long)x->n_sites);
+    pm_options def;
+    if (!opt) { pm_default_options(&def); opt = &def; }
+    const long long S = x->n_sites, T = x->n_tips, E = x->n_edges, NK = (long long)n * n;
+    const bool main_pass = stats || loglik, sel_pass = nsel > 0 && (branch_stats || node_marginals);
+    if (!main_pass && !sel_pass) return;
+    // Sites run in tiles whose per-site device state (partials, tip codes, node states, outputs) takes at most half of the
+    // free memory beside the per-branch matrices.  A site's result does not depend on its tile.
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) fail(PM_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
+    CK(cudaSetDevice(opt->device));
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const long long rsz = opt->precision == PM_F32 ? 4 : 8;
+    const long long fixed = E * (NK * NK + NK) * rsz, avail = (long long)(free_b / 2) - fixed;
+    const long long env_tile = read_switches().site_tile;
+    const auto tile_of = [&](long long per_site, long long count) {
+      long long ts = std::max<long long>(32, avail / per_site);
+      if (env_tile > 0) ts = std::min(ts, env_tile);
+      return std::min(ts, count);
+    };
+    const long long base = (T - 1) * n * rsz + (2 * T - 1) + T + (NK + 1) * 8;
+    if (main_pass) {
+      const long long ts = tile_of(base, S);
+      for (long long s0 = 0; s0 < S; s0 += ts)
+        expected_block(x, n, Q, pid, parity_tips, opt, s0, std::min(ts, S - s0), false, stats ? stats + s0 : nullptr, S,
+                       loglik ? loglik + s0 : nullptr, nullptr, nullptr);
+    }
+    if (sel_pass) {
+      // the selected sites as a problem of their own: their tip rows gathered in the order of `sites`
+      const bool u8 = x->states_u8 != nullptr;
+      std::vector<uint8_t> g8(u8 ? (size_t)nsel * T : 0);
+      std::vector<int32_t> g32(u8 ? 0 : (size_t)nsel * T);
+      for (int64_t i = 0; i < nsel; i++) {
+        if (u8) std::copy(x->states_u8 + sites[i] * T, x->states_u8 + (sites[i] + 1) * T, g8.begin() + i * T);
+        else std::copy(x->states + sites[i] * T, x->states + (sites[i] + 1) * T, g32.begin() + i * T);
+      }
+      pm_tree xs = *x;
+      xs.n_sites = nsel;
+      xs.states_u8 = u8 ? g8.data() : nullptr;
+      xs.states = u8 ? nullptr : g32.data();
+      const long long ts = tile_of(base + (E * NK + (2 * T - 1) * n) * 8, nsel);
+      for (long long s0 = 0; s0 < nsel; s0 += ts) {
+        const long long cnt = std::min(ts, nsel - s0);
+        // (outputs the caller did not ask for still have a device buffer: the kernel writes both)
+        expected_block(&xs, n, Q, pid, parity_tips, opt, s0, cnt, true, nullptr, cnt, nullptr,
+                       branch_stats ? branch_stats + s0 * E * NK : nullptr, node_marginals ? node_marginals + s0 * (2 * T - 1) * n : nullptr);
+      }
+    }
   });
 }
 
